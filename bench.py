@@ -3,6 +3,13 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: under torchrun, one rank per GPU)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR
+
+`--steps K` is the number of timed steps of every timed loop (the top-level record, `e2e`, each of `configs` and
+`strong_scaling`).  `--dump-outputs DIR` writes what the top-level record's last timed step computed, the verdict of
+every tuple (rank 0's shard when N > 1), to DIR/verify_ok.npy (float32, 1.0 = the signature verifies); the inputs are
+seeded, so two builds run with the same arguments can be compared output for output.  bench.py writes nothing into
+the source tree, which may be read-only.
 
 TOP-LEVEL RECORD (the driver's contract; config.workload): single-key `PublicKey::verify`
 (/root/reference/src/keys/public.rs:121-130) over 2^22 (message, key, signature) tuples PER GPU (weak scaling:
@@ -43,6 +50,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # no __pycache__ in the source tree
 
 LOG2_BATCH = 22
 METRIC = "verifies_per_s"
@@ -67,6 +75,22 @@ def make_inputs(n, seed):
 
 def corrupt_mask(n):
     return (np.arange(n, dtype=np.int64) * 2654435761 % 10) == 0  # deterministic ~10 %
+
+
+DUMP_BYTES = 64 * 10**6  # --dump-outputs writes at most this much in all
+DUMP_SAMPLE, DUMP_SAMPLE_SEED = 1 << 22, 0xD0  # 2^22 x (float32 value + float64 index) = 50 MB
+
+
+def dump_outputs(out_dir, name, values):
+    """values (one per tuple) -> out_dir/<name>.npy as float32.  A batch too large for DUMP_BYTES is replaced by a fixed,
+    seeded sample of DUMP_SAMPLE tuples, whose indices go to out_dir/<name>_index.npy (float64, exact below 2^53)."""
+    os.makedirs(out_dir, exist_ok=True)
+    values = np.asarray(values, dtype=np.float32)
+    if values.nbytes > DUMP_BYTES:
+        idx = np.sort(np.random.RandomState(DUMP_SAMPLE_SEED).choice(len(values), DUMP_SAMPLE, replace=False))
+        np.save(os.path.join(out_dir, name + "_index.npy"), idx.astype(np.float64))
+        values = values[idx]
+    np.save(os.path.join(out_dir, name + ".npy"), values)
 
 
 # ---- rand 0.8 StdRng (ChaCha12) over whole blocks, vectorised: block i of the stream = the 64 bytes that the i-th
@@ -249,7 +273,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="top-level record only (no `configs`, typed, strong scaling)")
     ap.add_argument("--only", default="", help="comma-separated config names to run (development aid)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the top-level record's per-tuple verdicts of its last timed step to DIR/verify_ok.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
     if args.impl == "reference":
         return cpu_reference_arm(args)
@@ -348,6 +376,8 @@ def main():
     sampler.stop_flag = True
     verdict = unpack(d_bm, n)
     assert (verdict == ~bad).all(), "GPU verdicts wrong: valid signatures must verify, corrupted ones must not"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, "verify_ok", verdict)
     value = world * n / (ms_step * 1e-3)
     e2e_s = time_host(lambda: eng.call("verify", n, POINTS_AFFINE, P(h_pk), P(h_u), P(h_R), P(h_msg), P(h_bm), None),
                       args.steps, min(args.warmup, 2))
@@ -370,7 +400,7 @@ def main():
     configs = {}
     only = set(x for x in args.only.split(",") if x)
     want = lambda name: not args.no_extras and (not only or name in only)
-    ksteps, kwarm = max(2, min(args.steps, 5)), max(1, min(args.warmup, 2))
+    ksteps, kwarm = args.steps, max(1, min(args.warmup, 2))
 
     def record(name, workload, cnt, unit, op_key, dev_call, host_call, h2d_b, d2h_b, check, cpu_fn=None, traffic_key=None):
         ms, _ = time_device(dev_call, ksteps, kwarm)

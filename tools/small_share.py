@@ -1,5 +1,5 @@
 import os, sys, time, json
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 from schnorr_b200 import POINTS_AFFINE, Engine, PinnedBuffer
 lg = int(sys.argv[1]) if len(sys.argv) > 1 else 19
