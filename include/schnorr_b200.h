@@ -249,7 +249,9 @@ int sb200_dbg_hades(sb200_ctx* ctx, int64_t n, int dense, uint32_t* states);  /*
 int sb200_dbg_scalar_mul(sb200_ctx* ctx, int64_t n, uint32_t flags, int base, const uint32_t* points,
                          const uint32_t* k, uint32_t* out);
 /* the curve half of sb200_verify alone, with caller-supplied challenges c (n x 8 u32, any integer < 2^252): verdict
- * i = (u G + c PK == R).  Lets a test drive the half-size-scalar path and its full-size fallback with chosen c. */
+ * i = (u G + c PK == R).  Runs the curve kernel sb200_verify runs for a batch of this size (the persistent form above one
+ * wave of resident CTAs, or as SB200_CURVE_PERSISTENT forces it).  Lets a test drive the half-size-scalar path and its
+ * full-size fallback with chosen c. */
 int sb200_dbg_verify_ec(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* pk, const uint32_t* sig_u,
                         const uint32_t* sig_R, const uint32_t* c, uint32_t* verdicts);
 /* the Hades tables the context derived from its parameters (rc 335, mds 25, pre 5, sparse 649, post 25 field

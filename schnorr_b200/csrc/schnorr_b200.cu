@@ -185,15 +185,6 @@ __global__ void __launch_bounds__(TPB, min_ctas(OP)) k_run(const KArgs a) {
     if ((threadIdx.x & 31) == 0 && active) a.bitmap[i >> 5] = a.inv_mask ? word & ~a.inv_mask[i >> 5] : word;
     return;
   }
-  if (OP == OP_DBG_VERIFY_EC) {  // in: pk, u, R, c -> bitmap
-    uint32_t u[8];
-    ldg_scalar(a.in[1] + i * 8, u);
-    ldg_scalar(a.in[3] + i * 8, c);
-    bool ok = verify_ec(ldg_point(a.in[0], i, aff), u, ldg_point(a.in[2], i, aff), c, a.combG);
-    unsigned word = __ballot_sync(0xffffffffu, ok && active);
-    if ((threadIdx.x & 31) == 0 && active) a.bitmap[i >> 5] = word;
-    return;
-  }
   if (OP == OP_POINTS_CHECK) {  // in: points -> bitmap
     bool ok = point_well_formed(ldg_point(a.in[0], i, aff));
     unsigned word = __ballot_sync(0xffffffffu, ok && active);
@@ -999,6 +990,21 @@ int launch(sb200_ctx* ctx, Op op, const KArgs& a, cudaStream_t st) {
     CU(cudaGetLastError());
     return SB200_OK;
   }
+  if (op == OP_DBG_VERIFY_EC) {  // in: pk, u, R, c -> bitmap: the production curve kernel, in the form the batch size picks,
+                                 // fed the caller's challenges where the challenge kernel would have written them
+    KArgs v = a;
+    v.out[0] = const_cast<uint32_t*>(a.in[3]);
+    v.in[3] = nullptr;
+#if SB_EC_GLOBAL_TABLES
+    CU(cudaMemsetAsync(&a.ws->tile, 0, sizeof(unsigned), st));  // the persistent form's work counter
+    launch_curve_p<0>(v, grid, st);
+#else
+    k_run<OP_VERIFY_EC><<<grid, TPB, 0, st>>>(v);
+#endif
+    ctx->launches.fetch_add(1, std::memory_order_relaxed);
+    CU(cudaGetLastError());
+    return SB200_OK;
+  }
 #if SB_VERIFY_SPLIT
   if (op == OP_VERIFY) {  // a.out[0] is always set here: the caller's c_out or scratch
     k_run<OP_CHALLENGE><<<grid, TPB, 0, st>>>(a);
@@ -1066,7 +1072,7 @@ int launch(sb200_ctx* ctx, Op op, const KArgs& a, cudaStream_t st) {
     CASE(OP_KEYGEN_VARGEN) CASE(OP_DBG_FQ) CASE(OP_DBG_FR_MUL) CASE(OP_DBG_HADES)
     CASE(OP_DBG_SMUL) CASE(OP_DECOMPRESS) CASE(OP_COMPRESS) CASE(OP_FROM_WIDE)
     CASE(OP_SIGN_DOUBLE_BYTES) CASE(OP_SIGN_VARGEN_BYTES)
-    CASE(OP_POINTS_CHECK) CASE(OP_DBG_VERIFY_EC) CASE(OP_WITNESS) CASE(OP_DBG_LAT3)
+    CASE(OP_POINTS_CHECK) CASE(OP_WITNESS) CASE(OP_DBG_LAT3)
 #undef CASE
     default: return SB200_ERR_ARG;
   }

@@ -144,11 +144,13 @@ def test_config1_single_verify_2_16_vs_cpu_restatement(engine):
     bad[::10, 0] ^= 1
     ok_a, c_a = engine.verify(pk, bad, R_, msg)
     assert (c_a == c).all() and not ok_a[::10].any() and ok_a[1::10].all()
-    okc, cc = ref_cpu.verify(pk[:4096], u[:4096], R_[:4096], msg[:4096])
-    assert okc.all() and (cc == c[:4096]).all()
-    uc, Rc, _ = ref_cpu.sign(sk[:2048], msg[:2048], nonce[:2048])
-    assert (uc == u[:2048]).all() and (Rc == R_[:2048]).all()
-    assert (ref_cpu.keygen(sk[:2048]) == pk[:2048]).all()
+    s = np.arange(0, n, n // 4096)  # strided over the whole batch: every pipeline chunk and late work items
+    okc, cc = ref_cpu.verify(pk[s], bad[s], R_[s], msg[s])
+    assert (okc == ok_a[s]).all() and okc.any() and not okc.all() and (cc == c[s]).all()
+    s2 = s[::2]
+    uc, Rc, _ = ref_cpu.sign(sk[s2], msg[s2], nonce[s2])
+    assert (uc == u[s2]).all() and (Rc == R_[s2]).all()
+    assert (ref_cpu.keygen(sk[s2]) == pk[s2]).all()
 
 
 def test_ragged_batch_across_pipeline_chunks(engine):
@@ -194,8 +196,9 @@ def test_config2_double_verify_2_20_properties(engine):
     u2 = u.copy(); u2[bad, 1] ^= 4
     ok, c2 = engine.verify_double(pk, pkp, u2, R_, Rp, msg)
     assert (ok == ~bad).all() and (c2 == c).all()
-    okc, _ = ref_cpu.verify_double(pk[:1024], pkp[:1024], u2[:1024], R_[:1024], Rp[:1024], msg[:1024])
-    assert (okc == ok[:1024]).all()
+    s = np.arange(0, n, n // 1024)  # strided over the whole batch: every pipeline chunk and late work items
+    okc, _ = ref_cpu.verify_double(pk[s], pkp[s], u2[s], R_[s], Rp[s], msg[s])
+    assert (okc == ok[s]).all()
     # swapping the two halves of the key breaks exactly the valid ones
     ok, _ = engine.verify_double(pkp[:4096], pk[:4096], u[:4096], R_[:4096], Rp[:4096], msg[:4096])
     assert not ok.any()
@@ -239,9 +242,10 @@ def test_config4_vargen_verify_2_22_ten_percent_corrupted(engine):
     ok, _ = engine.verify_vargen(pk2, gen2, u2, R_, msg2)
     assert (ok == ~bad).all()
     assert 0.09 < bad.mean() < 0.11
-    s = slice(0, 1024)
+    s = np.arange(0, n, 4093)  # strided over the whole batch (every chunk, late work items); odd: all four corruption kinds
     okc, _ = ref_cpu.verify_vargen(pk2[s], gen2[s], u2[s], R_[s], msg2[s])
     assert (okc == ok[s]).all()
+    assert all((bad[s] & (mode[s] == k)).any() for k in range(4))
 
 
 def test_multi_device_context_shards_without_collective():

@@ -138,3 +138,111 @@ def test_c_restatement_matches_python_oracle():
     pkv = ref_cpu.keygen(V.scalars(sk), gen=V.points(gens))
     ok, _ = ref_cpu.verify_vargen(pkv, V.points(gens), u, Rr, V.fqs(m))
     assert ok.all()
+
+
+def _whole_curve_cases(rnd, n):
+    """points the scale tests hand to ref_cpu: prime-order multiples, whole-curve points, sk G + torsion, the
+    small-order points and the identity"""
+    tors = V.torsion_points()
+    out = []
+    for i in range(n):
+        k = i % 4
+        if k == 0:
+            out.append(V.mul(o.G, rnd.randrange(R)))
+        elif k == 1:
+            out.append(V.rand_curve_point(rnd))
+        elif k == 2:
+            out.append(o.pt_add(V.mul(o.G, rnd.randrange(R)), tors[i % len(tors)]))
+        else:
+            out.append(tors[(i // 4) % len(tors)])
+    return out
+
+
+def _maybe_proj(rnd, pts, proj):
+    return V.points(pts, [rnd.randrange(1, Q) for _ in pts] if proj else None)
+
+
+@pytest.mark.parametrize("proj", [False, True], ids=["affine", "projective"])
+def test_c_restatement_on_the_whole_curve(proj):
+    """ref_cpu is the reference the large GPU batches are judged by: pin its verdicts and challenges against the Python
+    oracle on keys, nonce points and generators off the prime-order subgroup, small-order keys, the identity, (U : V : Z)
+    inputs with random Z, and variable-generator tuples with u = r - 1"""
+    rnd = random.Random(6 + proj)
+    n = 144
+    tors = V.torsion_points()
+    # single-key: valid by construction on the prime-order part, so keys with a torsion part pass iff c T = O
+    sk = [rnd.randrange(R) for _ in range(n)]
+    nonce = [rnd.randrange(R) for _ in range(n)]
+    m = [rnd.randrange(Q) for _ in range(n)]
+    pk, u, Rr = [], [], []
+    for i in range(n):
+        a, b, mm = sk[i], nonce[i], m[i]
+        ui, Ri, _ = o.sign(a, b, mm, mul=V.mul)
+        P = V.mul(o.G, a)
+        k = i % 6
+        if k == 1:
+            P = o.pt_add(P, tors[i % len(tors)])
+        elif k == 2:
+            P, ui, Ri = tors[i % len(tors)], b, V.mul(o.G, b)  # small-order key with R = u G
+        elif k == 3:
+            Ri = o.pt_add(Ri, tors[(i + 3) % len(tors)])
+        elif k == 4:
+            P = V.rand_curve_point(rnd)
+        elif k == 5:
+            ui = (ui + 1) % R
+        pk.append(P); u.append(ui); Rr.append(Ri)
+    want = [o.verify(*t, mul=V.mul) for t in zip(pk, u, Rr, m)]
+    ok, c = ref_cpu.verify(_maybe_proj(rnd, pk, proj), V.scalars(u), _maybe_proj(rnd, Rr, proj), V.fqs(m), affine=not proj)
+    assert ok.tolist() == want and any(want[1::6]) and not all(want[1::6]) and any(want[2::6]) and not all(want[2::6])
+    assert V.ints_out(c) == [o.challenge_hash(r_, mm) for r_, mm in zip(Rr, m)]
+    # double-key over whole-curve points in every position
+    P1, P2, R1, R2 = (_whole_curve_cases(rnd, n) for _ in range(4))
+    for i in range(0, n, 3):  # a third valid by construction, some with a torsion part on one key only
+        ui, R1[i], R2[i], _ = o.sign_double(sk[i], nonce[i], m[i], mul=V.mul)
+        P1[i], P2[i], u[i] = V.mul(o.G, sk[i]), V.mul(o.G_NUMS, sk[i]), ui
+        if i % 2:
+            P2[i] = o.pt_add(P2[i], tors[i % len(tors)])
+    want = [o.verify_double(*t, mul=V.mul) for t in zip(P1, P2, u, R1, R2, m)]
+    ok, c = ref_cpu.verify_double(*(_maybe_proj(rnd, x, proj) for x in (P1, P2)), V.scalars(u),
+                                  *(_maybe_proj(rnd, x, proj) for x in (R1, R2)), V.fqs(m), affine=not proj)
+    assert ok.tolist() == want and any(want) and not all(want)
+    assert V.ints_out(c) == [o.challenge_hash_double(a, b, mm) for a, b, mm in zip(R1, R2, m)]
+    # variable generator: whole-curve generators and keys, and the forced-fallback lanes u = r - 1 (valid by construction)
+    gens, pkv, Rv = (_whole_curve_cases(rnd, n) for _ in range(3))
+    uv = [rnd.randrange(R) for _ in range(n)]
+    for i in range(n):
+        g = gens[i]
+        if i % 3 == 0:
+            uv[i], Rv[i], _ = o.sign_vargen(sk[i], g, nonce[i], m[i], mul=V.mul)
+            pkv[i] = V.mul(g, sk[i])
+        elif i % 3 == 1 and g != o.IDENTITY:
+            k = rnd.randrange(1, R)
+            Rv[i] = V.mul(g, k)
+            c_ = o.challenge_hash(Rv[i], m[i])
+            uv[i], pkv[i] = R - 1, V.mul(g, (k - (R - 1)) * pow(c_, -1, R) % R)
+    want = [o.verify_vargen(*t, mul=V.mul) for t in zip(pkv, gens, uv, Rv, m)]
+    ok, c = ref_cpu.verify_vargen(*(_maybe_proj(rnd, x, proj) for x in (pkv, gens)), V.scalars(uv), _maybe_proj(rnd, Rv, proj),
+                                  V.fqs(m), affine=not proj)
+    assert ok.tolist() == want and any(want) and not all(want)
+    assert V.ints_out(c) == [o.challenge_hash(r_, mm) for r_, mm in zip(Rv, m)]
+
+
+def test_c_restatement_reads_only_252_scalar_bits():
+    """ref_cpu's multiplication walks bits 251..0 of u, as the reference's does, so it cannot judge a non-canonical u:
+    its verdict on u >= r is the verdict on u mod 2^252.  The product rejects u >= r (JubJubScalar::from_bytes), so a
+    GPU verdict is compared with ref_cpu's verdict AND u < r."""
+    rnd = random.Random(9)
+    n = 64
+    sk, nonce, m = [rnd.randrange(R) for _ in range(n)], [rnd.randrange(R) for _ in range(n)], [rnd.randrange(Q) for _ in range(n)]
+    for i in range(1, n, 8):  # u = nonce below 2^252 - r: u + r still fits the 252 bits
+        sk[i], nonce[i] = 0, rnd.randrange((1 << 252) - R)
+    sigs = [o.sign(a, b, mm, mul=V.mul) for a, b, mm in zip(sk, nonce, m)]
+    pk = [V.mul(o.G, a) for a in sk]
+    # u + r: bit 252 set or clear depending on u; u + r - 2^252 when set; the largest 256-bit values
+    big = [s[0] + R for s in sigs]
+    big[::8] = [(s[0] % (1 << 252)) | (0xF << 252) for s in sigs[::8]]  # same low 252 bits as a valid u
+    ok, _ = ref_cpu.verify(V.points(pk), V.scalars(big), V.points([s[1] for s in sigs]), V.fqs(m))
+    want = [o.verify(pk[i], big[i] % (1 << 252), sigs[i][1], m[i], mul=V.mul) for i in range(n)]
+    assert ok.tolist() == want
+    assert all(ok[::8]) and all(ok[1::8]) and not all(ok)  # so `& (u < r)` is what makes the expected verdict false
+    assert all(b < (1 << 252) for b in big[1::8])
