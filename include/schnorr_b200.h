@@ -244,7 +244,7 @@ int sb200_dbg_lattice3(sb200_ctx* ctx, int64_t n, const uint32_t* c, const uint3
 int sb200_dbg_fr_mul(sb200_ctx* ctx, int64_t n, const uint32_t* a, const uint32_t* b, uint32_t* out);
 /* Hades252 permutation of n states (5 field elements each, in place); dense != 0 runs the
  * reference-shaped dense partial rounds instead of the sparse factorisation. */
-int sb200_dbg_hades(sb200_ctx* ctx, int64_t n, int dense, uint32_t* states);  /* dense: 0 = sparse IMAD, 1 = dense IMAD (reference-shaped), 2 = FP64 pipe */
+int sb200_dbg_hades(sb200_ctx* ctx, int64_t n, int dense, uint32_t* states);  /* dense: 0 = production form (small-integer layers when the MDS qualifies, else sparse rounds), 1 = dense (reference-shaped), 2 = FP64 pipe */
 /* out[i] = k[i] * P[i] (affine); base: 0 = fixed G, 1 = fixed G', 2 = variable (points given) */
 int sb200_dbg_scalar_mul(sb200_ctx* ctx, int64_t n, uint32_t flags, int base, const uint32_t* points,
                          const uint32_t* k, uint32_t* out);

@@ -4,10 +4,18 @@
 //
 // One permutation per thread, state in registers (5 x 8 limbs), constants broadcast from
 // __constant__ memory (every lane reads the same address in lock-step).
-// The 59 partial rounds run in the sparse factorisation derived at context creation (params_host.cuh;
-// 9 products per round instead of 25; algebraically identical, hence bit-exact); the dense form is
-// kept as hades_perm_dense for the parity tests and the self-check of the derivation.
+// When the MDS matrix is L^-1 times a matrix C of small integers (the default Cauchy matrix 1/(i+j+5): L = 360360,
+// entries of C at most 72072), every round runs dense with C s in place of M s: 200 exact DFMAs and one reduction per
+// word instead of five Montgomery dot products (hades_perm_int).  Any other MDS runs the 59 partial rounds in the
+// sparse factorisation derived at context creation (params_host.cuh; 9 products per round instead of 25).  Both are
+// algebraically identical to the dense rounds, hence bit-exact; the dense form is kept as hades_perm_dense for the
+// parity tests and the self-check of the derivation.
 #pragma once
+#include <cstddef>
+#include <cstring>
+#if !defined(__CUDA_ARCH__)
+#include <cmath>
+#endif
 #include "fq.cuh"
 
 namespace sb200 {
@@ -22,7 +30,17 @@ struct HadesTables {
   uint32_t pre[5][8];          // sparse form: added to the state before the partial rounds
   uint32_t sparse[59 * 11][8]; // per partial round: key (1), row (5), column (5; entry 4 unused)
   uint32_t post[25][8];        // dense matrix applied once after the partial rounds
+  // Small-integer form (params_host.cuh derive_int_tables), valid when `int_layers` != 0: MDS = C / L with C a matrix
+  // of small integers, the state kept at a known per-round scale tau (Montgomery limbs of tau * x).
+  double cmat[25];             // C = L * MDS, row-major, exact small integers
+  uint32_t src[335][8];        // round constants times the scale of their round
+  uint32_t fix[59][8];         // per partial round: tau^-4 (brings the S-box word from tau^5 back to tau)
+  uint32_t unscale[8];         // tau^-1 of the scale after the last layer
+  uint32_t int_layers;         // 1: hades_perm runs the small-integer layers
 };
+// What sb200_params_check / sb200_dbg_hades_tables hand out (include/schnorr_b200.h: 1039 x 8 words)
+constexpr size_t HADES_ABI_BYTES = 1039 * 32;
+static_assert(offsetof(HadesTables, cmat) == HADES_ABI_BYTES, "the public table views keep their offsets");
 #if defined(__CUDACC__)
 __constant__ HadesTables d_hades;
 #endif
@@ -95,8 +113,129 @@ SB_HD void hades_perm_dense(fq* s) {
   for (int r = 0; r < 4; r++, rc += 5) hades_full_round<false>(s, rc);
 }
 
-// Production permutation: sparse partial rounds.
+// ---- small-integer layers on the FP64 pipe -------------------------------------------------------------------------
+// A limb times an entry of C is below 2^32 * 2^20 / 5, so a five-term column plus the carry of the previous column
+// stays below 2^52: a DFMA chain seeded with 2^52 holds it exactly, the integer in the low mantissa bits.  Every DFMA
+// here is exact, so the host build (std::fma on the same doubles) computes the same bits.
+constexpr uint32_t HI_2P52 = 0x43300000u;  // high word of 2^52
+constexpr double RECIP_Q224 = 0x1.1aa84a76ff6f1p-31;  // largest double <= 2^224 / q
+
+SB_HD double hl_fma(double a, double b, double c) {
+#if defined(__CUDA_ARCH__)
+  return __fma_rn(a, b, c);
+#else
+  SB_COUNT(dfma, 1);
+  return std::fma(a, b, c);
+#endif
+}
+SB_HD double hl_pair(uint32_t hi, uint32_t lo) {  // the double with these bits
+#if defined(__CUDA_ARCH__)
+  return __hiloint2double((int)hi, (int)lo);
+#else
+  uint64_t b = (uint64_t)hi << 32 | lo;
+  double d;
+  memcpy(&d, &b, 8);
+  return d;
+#endif
+}
+SB_HD uint64_t hl_bits(double d) {
+#if defined(__CUDA_ARCH__)
+  return (uint64_t)__double_as_longlong(d);
+#else
+  uint64_t b;
+  memcpy(&b, &d, 8);
+  return b;
+#endif
+}
+SB_HD double hl_sub52(double d) {  // d - 2^52, exact for d in [2^52, 2^53)
+#if defined(__CUDA_ARCH__)
+  return __dsub_rn(d, 0x1p+52);
+#else
+  return d - 0x1p+52;
+#endif
+}
+
+// r <- (top * 2^256 + r) mod q, canonical, for a value below 2^20 q (a layer row is below 5 * max C * q).
+// Q = floor(T * RECIP_Q224) with T = top * 2^32 + r[7] is the quotient or one less (T * 2^224 <= value, and the error of
+// the estimate is below 2^-30), so value - Q q is in [0, 2q).  Q < 2^20 and every limb of q is below 2^32, so each
+// Q q_i is one exact DFMA.
+SB_HD void hl_reduce(fq& r, uint32_t top) {
+  const double T = hl_sub52(hl_pair(HI_2P52 | top, r.v[7]));
+#if defined(__CUDA_ARCH__)
+  const double h = __fma_rz(T, RECIP_Q224, 0x1p+52);  // 2^52 + floor(T * RECIP_Q224)
+#else
+  SB_COUNT(dfma, 1);  // the same floor, from the 53-bit significand of RECIP_Q224 (= m * 2^-83)
+  const uint64_t Ti = (uint64_t)top << 32 | r.v[7];
+  const double h = 0x1p+52 + (double)(uint64_t)(((unsigned __int128)Ti * 0x11aa84a76ff6f1ull) >> 83);
+#endif
+  const double Qd = hl_sub52(h);
+  uint32_t lo[8], hi[8];
+  lo[0] = (uint32_t)hl_bits(h);  // q_0 = 1
+  hi[0] = 0;
+#pragma unroll
+  for (int i = 1; i < 8; i++) {
+    const uint64_t b = hl_bits(hl_fma(Qd, (double)FqP::p(i), 0x1p+52));
+    lo[i] = (uint32_t)b;
+    hi[i] = (uint32_t)(b >> 32) & 0xfffffu;
+  }
+  uint32_t qq[8], sh[8];  // Q q mod 2^256 = lo + hi * 2^32; the difference is below 2q < 2^256
+  sh[0] = 0;
+#pragma unroll
+  for (int i = 1; i < 8; i++) sh[i] = hi[i - 1];
+  add8(qq, lo, sh);
+  sub8(r.v, r.v, qq);
+  cond_sub_p<FqP>(r.v);
+}
+
+// s <- C s mod q, in place.  Columns in increasing limb order; each output limb overwrites the input limb of the same
+// column, whose five readers have all run, and the column's carry seeds the next column's chain.
+SB_HD void hades_int_layer(fq* s) {
+  uint32_t c[5];
+#pragma unroll
+  for (int i = 0; i < 8; i++) {
+    double x[5];
+#pragma unroll
+    for (int j = 0; j < 5; j++) x[j] = hl_sub52(hl_pair(HI_2P52, s[j].v[i]));
+#pragma unroll
+    for (int k = 0; k < 5; k++) {
+      double acc = hl_pair(HI_2P52, i ? c[k] : 0u);
+#pragma unroll
+      for (int j = 0; j < 5; j++) acc = hl_fma(SB_HADES(cmat)[k * 5 + j], x[j], acc);
+      const uint64_t b = hl_bits(acc);
+      s[k].v[i] = (uint32_t)b;
+      c[k] = (uint32_t)(b >> 32) & 0xfffffu;
+    }
+  }
+#pragma unroll
+  for (int k = 0; k < 5; k++) hl_reduce(s[k], c[k]);
+}
+
+// All 67 rounds dense, with M s computed as C s and the factor L tracked in the scale: round constants are pre-scaled,
+// a full S-box raises the scale to its fifth power, and in a partial round one product by tau^-4 returns the S-box
+// word to the scale of the others.  Exact arithmetic in F_q, so the result equals hades_perm_dense bit for bit.
+SB_HD void hades_perm_int(fq* s) {
+#pragma unroll 1
+  for (int r = 0; r < 67; r++) {
+#pragma unroll
+    for (int k = 0; k < 5; k++) s[k] = fq_add(s[k], ld8(SB_HADES(src)[r * 5 + k]));
+    if (r < 4 || r >= 63) {
+#pragma unroll
+      for (int k = 0; k < 5; k++) s[k] = fq_pow5(s[k]);
+    } else {
+      s[4] = fq_mul(fq_pow5(s[4]), ld8(SB_HADES(fix)[r - 4]));
+    }
+    hades_int_layer(s);
+  }
+#pragma unroll
+  for (int k = 0; k < 5; k++) s[k] = fq_mul(s[k], ld8(SB_HADES(unscale)));
+}
+
+// Production permutation: the small-integer layers when the context's MDS qualifies, else sparse partial rounds.
 SB_HD void hades_perm(fq* s) {
+  if (SB_HADES(int_layers)) {
+    hades_perm_int(s);
+    return;
+  }
   int rc = 0;
 #pragma unroll 1
   for (int r = 0; r < 4; r++, rc += 5) hades_full_round(s, rc);

@@ -9,7 +9,8 @@
 // This file: (1) the published recipes for the defaults (SHA-512 chain for the round constants in both recalled forms,
 // Cauchy MDS), (2) validation of supplied parameters, (3) the exact sparse factorisation of the 59 partial rounds that
 // the kernels run (same algebra as tools/gen_constants.py build_sparse_partial, re-derived here at init because the
-// inputs are only known then), (4) a dense-vs-sparse self-check.  Host code only; runs once per context.
+// inputs are only known then), (4) the small-integer form of the rounds when the MDS qualifies (derive_int_tables),
+// (5) a self-check of the production form against the dense permutation.  Host code only; runs once per context.
 #pragma once
 #include <cstring>
 
@@ -169,6 +170,51 @@ inline bool mat_inv(const Mat4& m, Mat4& out) {  // Gauss-Jordan; false if singu
   return true;
 }
 
+// Small-integer form of the rounds (hades.cuh hades_perm_int).  The MDS qualifies when every entry is 1/d for an integer
+// d and, with L = lcm of the d, the matrix C = L * MDS (C[k][j] = L / d[k][j]) keeps a five-term column of the layer
+// exact in a double: 5 * max C * 2^32 < 2^52.  The state then runs at a scale tau (the kernels hold tau * x):
+//   round r adds tau_r * rc[r];  a full S-box makes the scale tau_r^5;  in a partial round the S-box word is brought back
+//   from tau_r^5 to tau_r by fix = tau_r^-4;  the layer C multiplies the scale by L;  at the end, unscale = tau_67^-1.
+// Sets T.int_layers = 0 and leaves the other new fields zero when the MDS does not qualify.
+constexpr uint32_t INT_LAYER_CMAX_BOUND = (1u << 20) / 5;  // max C < this  <=>  5 * max C * 2^32 < 2^52
+
+inline void derive_int_tables(HadesTables& T) {
+  constexpr int W = 5, NP = 59, NF = 4;
+  memset(T.cmat, 0, sizeof(T.cmat));
+  memset(T.src, 0, sizeof(T.src));
+  memset(T.fix, 0, sizeof(T.fix));
+  memset(T.unscale, 0, sizeof(T.unscale));
+  T.int_layers = 0;
+  uint64_t d[25], L = 1, cmax = 0;
+  for (int e = 0; e < 25; e++) {
+    const fq iv = fq_from_mont(fq_inv(ld(T.mds[e])));
+    for (int i = 1; i < 8; i++)
+      if (iv.v[i]) return;
+    if (iv.v[0] == 0 || iv.v[0] >= INT_LAYER_CMAX_BOUND) return;
+    d[e] = iv.v[0];
+    uint64_t a = L, b = d[e];
+    while (b) { uint64_t t = a % b; a = b; b = t; }
+    L = L / a * d[e];
+    if (L >= (1ull << 32)) return;
+  }
+  for (int e = 0; e < 25; e++) cmax = L / d[e] > cmax ? L / d[e] : cmax;
+  if (cmax >= INT_LAYER_CMAX_BOUND) return;
+  for (int e = 0; e < 25; e++) T.cmat[e] = (double)(L / d[e]);
+  const fq Lf = fq_small((uint32_t)L);
+  fq tau = fq_one();
+  for (int r = 0; r < 2 * NF + NP; r++) {
+    for (int k = 0; k < W; k++) st(T.src[r * W + k], fq_mul(ld(T.rc[r * W + k]), tau));
+    if (r < NF || r >= NF + NP) {
+      tau = fq_mul(fq_sqr(fq_sqr(tau)), tau);
+    } else {
+      st(T.fix[r - NF], fq_inv(fq_sqr(fq_sqr(tau))));
+    }
+    tau = fq_mul(tau, Lf);
+  }
+  st(T.unscale, fq_inv(tau));
+  T.int_layers = 1;
+}
+
 // Sparse factorisation of the 59 partial rounds (S-box on the LAST word, index P = 4).
 // Partial round t:  x <- M * S_P(x + c_t).  With x = (B_t y_o ; y_P) (B_0 = I) and the MDS split into blocks
 // M = [[Moo, Mop], [Mpo, Mpp]] over (others, P):
@@ -231,6 +277,7 @@ inline bool derive_hades_tables(const uint32_t (*rc)[8], const uint32_t (*mds)[5
       fq v = (i < 4 && j < 4) ? B.a[i][j] : (i == P && j == P ? fq_one() : fq_zero());
       st(T.post[i * W + j], v);
     }
+  derive_int_tables(T);
   return true;
 }
 

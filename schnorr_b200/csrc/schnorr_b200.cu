@@ -1354,7 +1354,8 @@ int prepare_params(const sb200_params* p, HadesTables& T) {
   if (!params::on_curve(gu, gv) || !params::on_curve(hu, hv)) return SB200_ERR_PARAMS;
   if (!params::prime_order(gu, gv) || !params::prime_order(hu, hv)) return SB200_ERR_PARAMS;
   if (!params::derive_hades_tables(p->round_constants, p->mds, T)) return SB200_ERR_PARAMS;
-  // self-check: the sparse form must reproduce the reference-shaped dense permutation (host build of the same code)
+  // self-check: the production form (small-integer layers or sparse rounds) must reproduce the reference-shaped dense
+  // permutation (host build of the same code)
   h_hades = T;
   uint64_t s = 0x9e3779b97f4a7c15ull;
   for (int trial = 0; trial < 3; trial++) {
@@ -1490,7 +1491,7 @@ void sb200_destroy(sb200_ctx* ctx) {
 int sb200_params_check(const sb200_params* params_in, uint32_t* tables_out) {
   HadesTables* T = new HadesTables();
   int rc = prepare_params(params_in, *T);
-  if (!rc && tables_out) memcpy(tables_out, T, sizeof(HadesTables));
+  if (!rc && tables_out) memcpy(tables_out, T, HADES_ABI_BYTES);
   delete T;
   return rc;
 }
@@ -1501,7 +1502,7 @@ int sb200_get_params(const sb200_ctx* ctx, sb200_params* out) {
 }
 int sb200_dbg_hades_tables(const sb200_ctx* ctx, uint32_t* out) {
   if (!ctx || !out) return SB200_ERR_ARG;
-  memcpy(out, &ctx->tables, sizeof(HadesTables));
+  memcpy(out, &ctx->tables, HADES_ABI_BYTES);
   return SB200_OK;
 }
 

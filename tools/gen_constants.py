@@ -8,8 +8,9 @@ What is baked: the two field moduli and their Montgomery constants, the curve co
 tables, and the DEFAULT coordinates of the two generators.  What is NOT baked any more: the Hades round
 constants, the MDS matrix and the sparse factorisation of the partial rounds -- those are inputs of
 `sb200_init_ex` (include/schnorr_b200.h `sb200_params`) and are derived at context creation by
-csrc/params_host.cuh.  This file keeps the Python twin of that derivation (`hades_tables(rule)`), which
-tests/test_params.py compares bit-for-bit with what the library derives, and emits the tables of the
+csrc/params_host.cuh.  This file keeps the Python twin of that derivation (`hades_tables(rule)`, and
+`int_layer_tables` for the small-integer layers), which tests/test_params.py and tests/test_hades_cauchy.py compare
+bit-for-bit with what the library derives, and emits the tables of the
 compiled-out FP64 experiment (csrc/experimental/constants_fd_gen.cuh).
 
 Round-constant rule (`--ark`, SURVEY.md 8(c) recall-risk item 1; both recalled from dusk-hades assets/HOWTO.md):
@@ -252,6 +253,66 @@ def hades_tables(rule=DEFAULT_ARK):
     return {k: [mont(x) for x in v] for k, v in out.items()}
 
 
+INT_LAYER_CMAX_BOUND = (1 << 20) // 5  # max C below this <=> 5 * max C * 2^32 < 2^52 (a layer column fits a double)
+
+
+def int_layer_matrix(mds):
+    """(L, C) with C = L * mds a matrix of small integers, if mds qualifies for the small-integer layers, else None
+    (twin of csrc/params_host.cuh derive_int_tables)."""
+    import math
+    d = []
+    for row in mds:
+        for x in row:
+            v = inv(x) if x % Q else 0
+            if not 0 < v < INT_LAYER_CMAX_BOUND:
+                return None
+            d.append(v)
+    L = 1
+    for v in d:
+        L = math.lcm(L, v)
+        if L >= 1 << 32:
+            return None
+    C = [[L // d[k * WIDTH + j] for j in range(WIDTH)] for k in range(WIDTH)]
+    if max(max(r) for r in C) >= INT_LAYER_CMAX_BOUND:
+        return None
+    return L, C
+
+
+def int_layer_tables(rc=None, mds=None):
+    """The small-integer tables (cmat, src, fix, unscale) for the given round constants / MDS (plain integers),
+    scaled values as Montgomery integers; None when the MDS does not qualify."""
+    rc, mds = (RC if rc is None else rc), (MDS if mds is None else mds)
+    lc = int_layer_matrix(mds)
+    if lc is None:
+        return None
+    L, C = lc
+    tau, src, fix = 1, [], []
+    for rnd in range(FULL + PARTIAL):
+        src += [tau * rc[rnd * WIDTH + k] % Q for k in range(WIDTH)]
+        if rnd < FULL // 2 or rnd >= FULL // 2 + PARTIAL:
+            tau = pow(tau, 5, Q)
+        else:
+            fix.append(inv(pow(tau, 4, Q)))
+        tau = tau * L % Q
+    return {"cmat": [C[k][j] for k in range(WIDTH) for j in range(WIDTH)], "src": [mont(x) for x in src],
+            "fix": [mont(x) for x in fix], "unscale": [mont(inv(tau))]}
+
+
+def hades_int(state, tabs):
+    """The permutation as hades.cuh hades_perm_int runs it (plain integers in and out)."""
+    C = [tabs["cmat"][k * WIDTH:(k + 1) * WIDTH] for k in range(WIDTH)]
+    unm = lambda x: x * pow(RADIX, -1, Q) % Q
+    s = list(state)
+    for rnd in range(FULL + PARTIAL):
+        s = [(x + unm(tabs["src"][rnd * WIDTH + k])) % Q for k, x in enumerate(s)]
+        if rnd < FULL // 2 or rnd >= FULL // 2 + PARTIAL:
+            s = [pow(x, 5, Q) for x in s]
+        else:
+            s[P] = pow(s[P], 5, Q) * unm(tabs["fix"][rnd - FULL // 2]) % Q
+        s = [sum(C[k][j] * s[j] for j in range(WIDTH)) % Q for k in range(WIDTH)]
+    return [x * unm(tabs["unscale"][0]) % Q for x in s]
+
+
 def main():
     import argparse
     import random
@@ -265,6 +326,9 @@ def main():
         st = [rnd.randrange(Q) for _ in range(WIDTH)]
         assert hades_dense(st) == hades_sparse(st, sp), "sparse Hades factorisation is not exact"
     assert hades_dense([0] * 5) == hades_sparse([0] * 5, sp)
+    it = int_layer_tables()
+    assert it is not None and all(hades_dense(s) == hades_int(s, it) for s in ([0] * 5, [Q - 1] * 5, list(range(5)))), \
+        "small-integer Hades form is not exact"
     pre_add, ks, rows, cols, post = sp
 
     D = (-10240 * inv(10241)) % Q

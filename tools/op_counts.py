@@ -44,8 +44,8 @@ buf = np.zeros(8, np.uint32)
 
 def measure(fn):
     lib.h_counts_reset(); fn(); lib.h_counts_get(H.ptr(cnt))
-    w, mul, sqr, addsub, frm, dot5 = (int(x) for x in cnt[:6])
-    return {"imad_wide_per_tuple": w, "fq_mul": mul, "fq_sqr": sqr, "fq_dot5": dot5, "fq_addsub": addsub, "fr_mont_mul": frm}
+    w, mul, sqr, addsub, frm, dot5, dfma = (int(x) for x in cnt[:7])
+    return {"imad_wide_per_tuple": w, "fq_mul": mul, "fq_sqr": sqr, "fq_dot5": dot5, "fq_addsub": addsub, "fr_mont_mul": frm, "dfma": dfma}
 
 out = {}
 z1, z2 = rnd.randrange(1, o.Q), rnd.randrange(1, o.Q)
@@ -76,15 +76,15 @@ sb["fq_sqr"] = out["sign"]["fq_sqr"] - (K - 1) * out["fq_inv_euclid"]["fq_sqr"] 
 sb["note"] = "executed count of k_fixed_batch<OP_SIGN>: one shared inversion per 4 signatures (the one-tuple body is `sign`)"
 out["sign_batch4"] = sb
 # byte-level verify = two decompressions (decode kernel) + the limb-level verification; canonical -> Montgomery of the message: 1 product
-vb = {k: out["verify_affine"][k] + 2 * out["decompress"][k] for k in ("imad_wide_per_tuple", "fq_mul", "fq_sqr", "fq_dot5", "fq_addsub", "fr_mont_mul")}
+vb = {k: out["verify_affine"][k] + 2 * out["decompress"][k] for k in ("imad_wide_per_tuple", "fq_mul", "fq_sqr", "fq_dot5", "fq_addsub", "fr_mont_mul", "dfma")}
 vb["imad_wide_per_tuple"] += 120
 vb["fq_mul"] += 1
 vb["note"] = "decode kernel (2 point decompressions + message to Montgomery form) + challenge kernel + curve kernel"
 out["verify_bytes"] = vb
 st = np.concatenate([H.mont(x) for x in range(5)])
-out["hades_perm_sparse"] = measure(lambda: lib.h_hades(H.ptr(st), 0))
+out["hades_perm_sparse"] = measure(lambda: lib.h_hades(H.ptr(st), 0))  # the production form: small-integer layers for the default MDS
 out["hades_perm_dense"] = measure(lambda: lib.h_hades(H.ptr(st), 1))
-out["_note"] = "counted by the instrumented host build of schnorr_b200/csrc (same per-tuple code as the kernels, 16-bit comb); 1 fq_mul = 120 IMAD.WIDE, 1 fq_sqr = 84, 1 fq_dot5 (5 products, 1 reduction) = 368, 1 fr_mont_mul = 128; single-key verify also counts the 13 limb products of every step of the half-size-scalar Euclid (hgcd.cuh)"
+out["_note"] = "counted by the instrumented host build of schnorr_b200/csrc (same per-tuple code as the kernels, 16-bit comb); 1 fq_mul = 120 IMAD.WIDE, 1 fq_sqr = 84, 1 fq_dot5 (5 products, 1 reduction) = 368, 1 fr_mont_mul = 128; dfma = FP64 fused multiply-adds of the small-integer Hades layers (hades.cuh, 1 per limb product of C s, plus the reductions); single-key verify also counts the 13 limb products of every step of the half-size-scalar Euclid (hgcd.cuh)"
 if "--check" not in sys.argv:
     path = os.path.join(ROOT, "profiles", "op_counts.json")
     old = json.load(open(path)) if os.path.exists(path) else {}
