@@ -29,8 +29,10 @@
  *   verdicts = bitmap, bit (i & 31) of word (i >> 5) is tuple i's `verify` result; ceil(n/32) words.
  *
  * Nonces are an INPUT (`nonce[i]` is the one `JubJubScalar::random(rng)` draw of signature i,
- * /root/reference/src/keys/secret.rs:155): the RNG stays on the host; the library never generates
- * randomness.
+ * /root/reference/src/keys/secret.rs:155): the RNG state stays with the caller.  The library generates no
+ * randomness of its own; sb200_stdrng_random and sb200_sign_stdrng expand a caller-owned StdRng position
+ * (seed + keystream word) deterministically on the device into exactly the draws the caller's generator would
+ * have made, and hand back the advanced position.
  *
  * Threading: one batch in flight per context (calls on one context are serialised by an internal
  * mutex); distinct contexts are independent.  Calls block until the outputs are in host memory,
@@ -183,6 +185,28 @@ int sb200_points_compress(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint3
 /* Field::random's from_bytes_wide on n 64-byte draws: field 0 -> JubJubScalar (canonical limbs),
  * field 1 -> BlsScalar (Montgomery limbs).  /root/reference/src/keys/secret.rs:83,155 */
 int sb200_scalars_from_wide(sb200_ctx* ctx, int64_t n, uint32_t flags, int field, const uint8_t* wide64, uint32_t* out);
+/* Position in a rand 0.8 StdRng (ChaCha12, stream 0): the 32-byte seed as 8 LE words, and the index of the next
+ * unread 32-bit word of the keystream (16 x block counter + word within the block).  rand_core hands the keystream out
+ * in whole words, so this is the generator's complete state.  The key determines every nonce drawn from it: it reaches
+ * the device only as a kernel parameter, is never written to device memory and never appears in sb200_last_error. */
+typedef struct sb200_stdrng {
+  uint32_t key[8];
+  uint64_t word_pos;
+} sb200_stdrng;
+/* n consecutive Field::random draws: out[i] = from_bytes_wide(the 16 words at word_pos + 16 i);
+ * field 0 -> JubJubScalar (canonical), 1 -> BlsScalar (Montgomery).  flags: SB200_DEVICE_PTRS only.
+ * On SB200_OK rng->word_pos has advanced by 16 n; on any error it is unchanged.  SB200_ERR_ARG also for a null rng
+ * and for word_pos + 16 n overflowing 2^64.  Draw i belongs to tuple i however the batch is chunked or split over
+ * devices.  /root/reference/src/keys/secret.rs:83,155 */
+int sb200_stdrng_random(sb200_ctx* ctx, int64_t n, uint32_t flags, int field, sb200_stdrng* rng, uint32_t* out);
+/* sb200_sign / _sign_double / _sign_vargen (scheme 0 / 1 / 2) with nonce i = JubJubScalar::random draw i of *rng.
+ * Same outputs, bit for bit, as drawing the nonces on the host and calling the scheme's sign entry point.  flags:
+ * SB200_DEVICE_PTRS, SB200_SIGN_OBLIVIOUS, and for scheme 2 SB200_POINTS_AFFINE (the layout of `generator`, which
+ * only scheme 2 reads).  R_prime_out only for scheme 1.  rng->word_pos advances by 16 n on SB200_OK only.
+ * Two launches: the draws into a device-only row, then the scheme's sign kernel reading its nonces from there. */
+int sb200_sign_stdrng(sb200_ctx* ctx, int64_t n, uint32_t flags, int scheme, const uint32_t* sk, const uint32_t* msg,
+                      const uint32_t* generator, sb200_stdrng* rng, uint32_t* u_out, uint32_t* R_out,
+                      uint32_t* R_prime_out, uint32_t* c_out);
 /* canonical <-> Montgomery limbs of n field elements (BlsScalar::from_bytes / to_bytes minus the range check) */
 int sb200_fq_to_mont(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* in, uint32_t* out);
 int sb200_fq_from_mont(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* in, uint32_t* out);

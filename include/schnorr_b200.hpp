@@ -3,8 +3,9 @@
 // The reference is compiled code (Rust); its toolchain is not in this image, so the reference-facing host
 // layer is written in C++ with the reference's type names, method names, argument meaning and error
 // behaviour.  Header-only; link with -lschnorr_b200.  Everything arithmetic happens on the GPU through
-// include/schnorr_b200.h (single calls are batches of one); the host only moves bytes and runs the RNG,
-// exactly the split the reference has between `dusk-schnorr` and its arithmetic crates.
+// include/schnorr_b200.h (single calls are batches of one); the host only moves bytes and keeps the RNG state,
+// exactly the split the reference has between `dusk-schnorr` and its arithmetic crates.  The batch signers hand the
+// RNG's position to the device, which draws the nonces (sb200_sign_stdrng) and returns the advanced position.
 //
 //   SecretKey        /root/reference/src/keys/secret.rs:56-263      random, sign, sign_double, with_variable_generator, to/from_bytes
 //   SecretKeyVarGen  /root/reference/src/keys/secret.rs:307-451     new, random, sign, to/from_bytes
@@ -173,6 +174,27 @@ class StdRng {
     std::memcpy(&v, b, 8);
     return v;
   }
+  // Position of the next unread 32-bit keystream word (16 x block + word within the block), rand_chacha's get_word_pos.
+  // Meaningful on a word boundary only: every draw of this API is 8 or 64 bytes, so only a caller's own fill_bytes
+  // of a length that is not a multiple of 4 leaves the stream inside a word.
+  bool on_word_boundary() const { return pos_ % 4 == 0; }
+  uint64_t word_pos() const { return 16 * block_ - (64 - pos_) / 4; }
+  // continue the stream at keystream word `w` (rand_chacha's set_word_pos)
+  void seek(uint64_t w) {
+    block_ = w / 16;
+    pos_ = 64;
+    if (w % 16) {
+      refill();
+      pos_ = 4 * (size_t)(w % 16);
+    }
+  }
+  // the device-side generator's view of this stream: seed and current word position
+  sb200_stdrng position() const {
+    sb200_stdrng p;
+    std::memcpy(p.key, key_, 32);
+    p.word_pos = word_pos();
+    return p;
+  }
 
  private:
   static uint32_t rotl(uint32_t v, int n) { return (v << n) | (v >> (32 - n)); }
@@ -205,6 +227,18 @@ class StdRng {
 };
 
 namespace detail {
+// nonce i of a batch signer = the i-th JubJubScalar::random draw of rng.  On a word boundary the device draws them
+// from the stream's position (sb200_sign_stdrng), and the stream is moved to where the host draws would have left it;
+// otherwise the host draws them.  Returns false when the caller must sign with host-drawn nonces.
+inline bool sign_stdrng(StdRng& rng, int scheme, size_t n, uint32_t flags, const uint32_t* sk, const uint32_t* msg,
+                        const uint32_t* gen, uint32_t* u, uint32_t* R, uint32_t* Rp) {
+  if (!rng.on_word_boundary()) return false;
+  sb200_stdrng pos = rng.position();
+  Context& c = Context::global();
+  c.check(sb200_sign_stdrng(c.raw(), (int64_t)n, flags, scheme, sk, msg, gen, &pos, u, R, Rp, nullptr), "sign_stdrng");
+  rng.seek(pos.word_pos);
+  return true;
+}
 inline void wide_draws(StdRng& rng, size_t n, int field, uint32_t* out /* n x 8 */) {
   avec<uint8_t> w(64 * n);
   rng.fill_bytes(w.data(), 64 * n);
@@ -389,13 +423,16 @@ class SecretKey {  // /root/reference/src/keys/secret.rs:56-263
   // batch: signature i consumes the rng's i-th JubJubScalar::random draw, in order (secret.rs:155)
   static std::vector<Signature> sign_batch(const std::vector<SecretKey>& sks, StdRng& rng, const std::vector<BlsScalar>& msgs) {
     size_t n = sks.size();
-    avec<uint32_t> sk(8 * n), m(8 * n), nonce(8 * n), u(8 * n), R(16 * n);
+    avec<uint32_t> sk(8 * n), m(8 * n), u(8 * n), R(16 * n);
     detail::parallel_for(n, [&](size_t lo, size_t hi) {
       for (size_t i = lo; i < hi; i++) { std::memcpy(&sk[8 * i], sks[i].s_.l, 32); std::memcpy(&m[8 * i], msgs[i].l, 32); }
     });
-    detail::wide_draws(rng, n, 0, nonce.data());
-    Context& c = Context::global();
-    c.check(sb200_sign(c.raw(), (int64_t)n, 0, sk.data(), m.data(), nonce.data(), u.data(), R.data(), nullptr), "sign");
+    if (!detail::sign_stdrng(rng, 0, n, 0, sk.data(), m.data(), nullptr, u.data(), R.data(), nullptr)) {
+      avec<uint32_t> nonce(8 * n);
+      detail::wide_draws(rng, n, 0, nonce.data());
+      Context& c = Context::global();
+      c.check(sb200_sign(c.raw(), (int64_t)n, 0, sk.data(), m.data(), nonce.data(), u.data(), R.data(), nullptr), "sign");
+    }
     std::vector<Signature> out(n);
     detail::parallel_for(n, [&](size_t lo, size_t hi) {
       for (size_t i = lo; i < hi; i++) { std::memcpy(out[i].u_.l, &u[8 * i], 32); out[i].R_ = JubJubExtended::from_affine_limbs(&R[16 * i]); }
@@ -404,11 +441,14 @@ class SecretKey {  // /root/reference/src/keys/secret.rs:56-263
   }
   static std::vector<SignatureDouble> sign_double_batch(const std::vector<SecretKey>& sks, StdRng& rng, const std::vector<BlsScalar>& msgs) {
     size_t n = sks.size();
-    avec<uint32_t> sk(8 * n), m(8 * n), nonce(8 * n), u(8 * n), R(16 * n), Rp(16 * n);
+    avec<uint32_t> sk(8 * n), m(8 * n), u(8 * n), R(16 * n), Rp(16 * n);
     for (size_t i = 0; i < n; i++) { std::memcpy(&sk[8 * i], sks[i].s_.l, 32); std::memcpy(&m[8 * i], msgs[i].l, 32); }
-    detail::wide_draws(rng, n, 0, nonce.data());
-    Context& c = Context::global();
-    c.check(sb200_sign_double(c.raw(), (int64_t)n, 0, sk.data(), m.data(), nonce.data(), u.data(), R.data(), Rp.data(), nullptr), "sign_double");
+    if (!detail::sign_stdrng(rng, 1, n, 0, sk.data(), m.data(), nullptr, u.data(), R.data(), Rp.data())) {
+      avec<uint32_t> nonce(8 * n);
+      detail::wide_draws(rng, n, 0, nonce.data());
+      Context& c = Context::global();
+      c.check(sb200_sign_double(c.raw(), (int64_t)n, 0, sk.data(), m.data(), nonce.data(), u.data(), R.data(), Rp.data(), nullptr), "sign_double");
+    }
     std::vector<SignatureDouble> out(n);
     for (size_t i = 0; i < n; i++) {
       std::memcpy(out[i].u_.l, &u[8 * i], 32);
@@ -453,11 +493,14 @@ class SecretKeyVarGen {  // /root/reference/src/keys/secret.rs:307-451
   }
   bool operator==(const SecretKeyVarGen& o) const { return sk_ == o.sk_ && generator_ == o.generator_; }
   SignatureVarGen sign(StdRng& rng, const BlsScalar& msg) const {
-    avec<uint32_t> sk(8), g(24), m(8), nonce(8), u(8), R(16);
+    avec<uint32_t> sk(8), g(24), m(8), u(8), R(16);
     std::memcpy(sk.data(), sk_.l, 32); std::memcpy(g.data(), generator_.l, 96); std::memcpy(m.data(), msg.l, 32);
-    detail::wide_draws(rng, 1, 0, nonce.data());
-    Context& c = Context::global();
-    c.check(sb200_sign_vargen(c.raw(), 1, SB200_POINTS_PROJECTIVE, sk.data(), g.data(), m.data(), nonce.data(), u.data(), R.data(), nullptr), "sign_vargen");
+    if (!detail::sign_stdrng(rng, 2, 1, SB200_POINTS_PROJECTIVE, sk.data(), m.data(), g.data(), u.data(), R.data(), nullptr)) {
+      avec<uint32_t> nonce(8);
+      detail::wide_draws(rng, 1, 0, nonce.data());
+      Context& c = Context::global();
+      c.check(sb200_sign_vargen(c.raw(), 1, SB200_POINTS_PROJECTIVE, sk.data(), g.data(), m.data(), nonce.data(), u.data(), R.data(), nullptr), "sign_vargen");
+    }
     SignatureVarGen s;
     std::memcpy(s.u_.l, u.data(), 32);
     s.R_ = JubJubExtended::from_affine_limbs(R.data());

@@ -100,6 +100,14 @@ impl Sb200Params {
     }
 }
 
+/// `sb200_stdrng`: a rand 0.8 `StdRng` (= `rand_chacha::ChaCha12Rng`, stream 0) as its seed (8 little-endian words)
+/// and the index of the next unread 32-bit keystream word.
+#[repr(C)]
+struct Sb200StdRng {
+    key: [u32; 8],
+    word_pos: u64,
+}
+
 #[link(name = "schnorr_b200")]
 extern "C" {
     fn sb200_init(devices: *const c_int, n_devices: c_int, out: *mut *mut Sb200Ctx) -> c_int;
@@ -142,6 +150,10 @@ extern "C" {
     fn sb200_points_compress(ctx: *mut Sb200Ctx, n: i64, flags: u32, points: *const u32, bytes32_out: *mut u8) -> c_int;
     fn sb200_scalars_from_wide(ctx: *mut Sb200Ctx, n: i64, flags: u32, field: c_int, wide64: *const u8,
                                out: *mut u32) -> c_int;
+    fn sb200_stdrng_random(ctx: *mut Sb200Ctx, n: i64, flags: u32, field: c_int, rng: *mut Sb200StdRng, out: *mut u32) -> c_int;
+    fn sb200_sign_stdrng(ctx: *mut Sb200Ctx, n: i64, flags: u32, scheme: c_int, sk: *const u32, msg: *const u32,
+                         generator: *const u32, rng: *mut Sb200StdRng, u_out: *mut u32, R_out: *mut u32,
+                         R_prime_out: *mut u32, c_out: *mut u32) -> c_int;
     fn sb200_fq_to_mont(ctx: *mut Sb200Ctx, n: i64, flags: u32, input: *const u32, out: *mut u32) -> c_int;
     fn sb200_fq_from_mont(ctx: *mut Sb200Ctx, n: i64, flags: u32, input: *const u32, out: *mut u32) -> c_int;
     fn sb200_verify_bytes(ctx: *mut Sb200Ctx, n: i64, flags: u32, pk32: *const u8, sig64: *const u8, msg32: *const u8,
@@ -354,6 +366,41 @@ impl SecretKey {
             sb200_sign(ctx.raw, n as i64, 0, sk.as_ptr(), m.as_ptr(), nonce.as_ptr(), u.as_mut_ptr(), r.as_mut_ptr(),
                        core::ptr::null_mut())
         })?;
+        Ok((0..n).map(|i| Signature::new(scalar_at(&u, i), point_at(&r, i))).collect())
+    }
+
+    /// `sign_batch` over the generator rand 0.8's `StdRng` wraps (`rand_chacha::ChaCha12Rng`): the nonces are drawn on the
+    /// device from the generator's seed and word position (`sb200_sign_stdrng`) instead of on the host, and the generator
+    /// is moved past them -- it ends exactly where n `JubJubScalar::random` draws would have left it, and the signatures
+    /// are the same.  A generic `RngCore` exposes no position; it keeps `sign_batch`, and so does a `ChaCha12Rng` on a
+    /// stream other than 0 or past 2^64 words (the library's positions are 64-bit).  Uncompiled, like the rest of this
+    /// file: the four `ChaCha12Rng` methods are rand_chacha 0.3's as recalled.
+    pub fn sign_batch_chacha12(ctx: &CudaCtx, sks: &[SecretKey], rng: &mut rand_chacha::ChaCha12Rng, msgs: &[BlsScalar])
+                               -> Result<Vec<Signature>, CudaError> {
+        let n = sks.len();
+        assert!(msgs.len() == n);
+        // the library expands stream 0 at 64-bit word positions; any other generator state keeps the host draw
+        let word_pos = match u64::try_from(rng.get_word_pos()) {
+            Ok(w) if rng.get_stream() == 0 => w,
+            _ => return Self::sign_batch(ctx, sks, rng, msgs),
+        };
+        let seed = rng.get_seed();
+        let mut pos = Sb200StdRng { key: [0u32; 8], word_pos: 0 };
+        for i in 0..8 {
+            pos.key[i] = u32::from_le_bytes([seed[4 * i], seed[4 * i + 1], seed[4 * i + 2], seed[4 * i + 3]]);
+        }
+        pos.word_pos = word_pos;
+        let (mut sk, mut m) = (Vec32::with_capacity(8 * n), Vec32::with_capacity(8 * n));
+        for i in 0..n {
+            push_scalar(&mut sk, sks[i].as_ref());
+            push_fq(&mut m, &msgs[i]);
+        }
+        let (mut u, mut r) = (Vec32::zeroed(8 * n), Vec32::zeroed(16 * n));
+        ctx.check(unsafe {
+            sb200_sign_stdrng(ctx.raw, n as i64, 0, 0, sk.as_ptr(), m.as_ptr(), core::ptr::null(), &mut pos, u.as_mut_ptr(),
+                              r.as_mut_ptr(), core::ptr::null_mut(), core::ptr::null_mut())
+        })?;
+        rng.set_word_pos(pos.word_pos as u128);
         Ok((0..n).map(|i| Signature::new(scalar_at(&u, i), point_at(&r, i))).collect())
     }
 

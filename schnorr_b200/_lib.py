@@ -47,6 +47,17 @@ def default_params(ark: int = ARK_ENV) -> Params:
     return p
 
 
+class StdRngPos(ctypes.Structure):
+    """`sb200_stdrng`: a rand 0.8 StdRng (ChaCha12, stream 0) as its 32-byte seed (8 little-endian words) and the index
+    of the next unread 32-bit keystream word (16 x block + word within the block)."""
+    _fields_ = [("key", ctypes.c_uint32 * 8), ("word_pos", ctypes.c_uint64)]
+
+    @classmethod
+    def of(cls, key, word_pos: int) -> "StdRngPos":
+        k = np.asarray(key, dtype=np.uint32).reshape(8)
+        return cls((ctypes.c_uint32 * 8)(*[int(x) for x in k]), int(word_pos))
+
+
 def _split_tables(out: np.ndarray) -> dict:
     cut = np.cumsum([0, 335, 25, 5, 649, 25])
     return {k: out[cut[i]:cut[i + 1]].copy() for i, k in enumerate(("rc", "mds", "pre", "sparse", "post"))}
@@ -111,6 +122,8 @@ def load_library() -> ctypes.CDLL:
         "sb200_points_decompress": (ci, [vp, i64, u32] + [u32p] * 3),
         "sb200_points_compress": (ci, [vp, i64, u32] + [u32p] * 2),
         "sb200_scalars_from_wide": (ci, [vp, i64, u32, ci] + [u32p] * 2),
+        "sb200_stdrng_random": (ci, [vp, i64, u32, ci, vp, u32p]),
+        "sb200_sign_stdrng": (ci, [vp, i64, u32, ci] + [u32p] * 3 + [vp] + [u32p] * 4),
         "sb200_fq_to_mont": (ci, [vp, i64, u32] + [u32p] * 2),
         "sb200_fq_from_mont": (ci, [vp, i64, u32] + [u32p] * 2),
         "sb200_verify_bytes": (ci, [vp, i64, u32] + [u32p] * 5),
@@ -139,7 +152,7 @@ EXPORTED_SYMBOLS = [
     "sb200_launch_count", "sb200_host_alloc", "sb200_host_free", "sb200_verify", "sb200_verify_double",
     "sb200_verify_vargen", "sb200_sign", "sb200_sign_double", "sb200_sign_vargen", "sb200_keygen",
     "sb200_keygen_double", "sb200_keygen_vargen", "sb200_points_decompress", "sb200_points_compress",
-    "sb200_scalars_from_wide", "sb200_fq_to_mont", "sb200_fq_from_mont", "sb200_verify_bytes", "sb200_sign_bytes",
+    "sb200_scalars_from_wide", "sb200_stdrng_random", "sb200_sign_stdrng", "sb200_fq_to_mont", "sb200_fq_from_mont", "sb200_verify_bytes", "sb200_sign_bytes",
     "sb200_verify_double_bytes", "sb200_verify_vargen_bytes", "sb200_sign_double_bytes", "sb200_sign_vargen_bytes", "sb200_dbg_fq", "sb200_dbg_fr_mul", "sb200_dbg_lattice3", "sb200_dbg_hades",
     "sb200_dbg_scalar_mul",
 ]
@@ -360,6 +373,36 @@ class Engine:
         rc = self._lib.sb200_scalars_from_wide(self._h, n, 0, field, b.ctypes.data, out.ctypes.data)
         self._check(rc, "scalars_from_wide")
         return out
+
+    def stdrng_random(self, key, word_pos: int, n: int, field: int, flags: int = 0, out=None):
+        """n consecutive Field::random draws of the StdRng at (key, word_pos), computed on the device: [n, 8] limbs
+        (field 0 = JubJubScalar canonical, 1 = BlsScalar Montgomery) and the advanced word position (word_pos + 16 n).
+        With flags = DEVICE_PTRS, `out` is a device pointer and nothing is returned but the position."""
+        pos = StdRngPos.of(key, word_pos)
+        res = aligned_empty((n, 8)) if out is None else None
+        rc = self._lib.sb200_stdrng_random(self._h, n, flags, field, ctypes.byref(pos), res.ctypes.data if res is not None else out)
+        self._check(rc, "stdrng_random")
+        return (res, pos.word_pos) if res is not None else pos.word_pos
+
+    def sign_stdrng(self, scheme: int, sk, msg, key, word_pos: int, gen=None, affine=True, oblivious=False):
+        """sign (scheme 0), sign_double (1) or sign_vargen (2) with nonce i = the i-th JubJubScalar::random draw of the
+        StdRng at (key, word_pos), drawn on the device.  Returns the scheme's sign outputs (u, R[, R'], c) followed by
+        the advanced word position."""
+        n = np.asarray(sk).size // 8
+        sk, msg = _arr(sk, 8, n, "sk"), _arr(msg, 8, n, "msg")
+        fl = SIGN_OBLIVIOUS if oblivious else 0
+        g = None
+        if scheme == 2:
+            fl |= POINTS_AFFINE if affine else POINTS_PROJECTIVE
+            g = _arr(gen, self._pw(affine), n, "gen")
+        u, R, c = aligned_empty((n, 8)), aligned_empty((n, 16)), aligned_empty((n, 8))
+        Rp = aligned_empty((n, 16)) if scheme == 1 else None
+        pos = StdRngPos.of(key, word_pos)
+        rc = self._lib.sb200_sign_stdrng(self._h, n, fl, scheme, sk.ctypes.data, msg.ctypes.data,
+                                         g.ctypes.data if g is not None else None, ctypes.byref(pos), u.ctypes.data,
+                                         R.ctypes.data, Rp.ctypes.data if Rp is not None else None, c.ctypes.data)
+        self._check(rc, "sign_stdrng")
+        return ((u, R, Rp, c) if scheme == 1 else (u, R, c)) + (int(pos.word_pos),)
 
     def fq_to_mont(self, a):
         n = np.asarray(a).size // 8

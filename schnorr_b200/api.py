@@ -15,7 +15,8 @@ is written here in Python with the SAME names, argument meaning and error behavi
 
 Every scalar multiplication, hash and comparison runs on the GPU through the C ABI (single calls are
 batches of one); only representation work stays on the host, as in the reference: byte
-(de)serialisation, canonical<->Montgomery conversion and the RNG.  There is no CPU fallback for the
+(de)serialisation, canonical<->Montgomery conversion and the RNG state.  The batch signers hand the RNG's
+position to the device, which draws the nonces the host would have drawn and returns the advanced position.  There is no CPU fallback for the
 arithmetic: without the CUDA library / a B200 the first call raises.
 
 New relative to the reference: the `*_batch` class methods (what north_star calls the batch entry
@@ -225,12 +226,29 @@ class StdRng:
             x += st
         return np.ascontiguousarray(x.T)
 
+    @property
+    def word_pos(self) -> int:
+        """index of the next unread 32-bit keystream word (rand_chacha's `get_word_pos`); None when a byte draw of a
+        length that is not a multiple of 4 left the stream inside a word"""
+        return None if len(self.buf) % 4 else 16 * self.block - len(self.buf) // 4
+
+    def seek(self, word_pos: int) -> None:
+        """continue the stream at keystream word `word_pos` (rand_chacha's `set_word_pos`)"""
+        self.block, off = divmod(int(word_pos), 16)
+        self.buf = b""
+        if off:
+            self.buf = self.blocks(self.block, 1).tobytes()[4 * off:]
+            self.block += 1
+
     def fill_bytes(self, n: int) -> bytes:
         while len(self.buf) < n:
             self.buf += self.blocks(self.block, 4).tobytes()
             self.block += 4
         out, self.buf = self.buf[:n], self.buf[n:]
         return out
+
+    def next_u64(self) -> int:
+        return int.from_bytes(self.fill_bytes(8), "little")
 
     def random_scalar(self) -> int:
         return int.from_bytes(self.fill_bytes(64), "little") % R
@@ -337,17 +355,26 @@ class SecretKey:
     def with_variable_generator(self, generator: JubJubExtended) -> "SecretKeyVarGen":
         return SecretKeyVarGen(self._s, generator)
 
-    # batch entry points: signature i consumes the rng's i-th JubJubScalar::random draw, in order
+    # batch entry points: signature i consumes the rng's i-th JubJubScalar::random draw, in order.  On a word boundary
+    # (always, unless a byte draw of odd length came before) the device draws the nonces from the rng's position.
     @staticmethod
     def sign_batch(sks: Sequence["SecretKey"], rng: StdRng, msgs: Sequence[int]) -> List[Signature]:
-        nonces = rng.random_scalars(len(sks))
-        u, Rr, _ = get_engine().sign(_scalars([k._s for k in sks]), _fqs(msgs), _scalars(nonces))
+        sk, m = _scalars([k._s for k in sks]), _fqs(msgs)
+        if rng.word_pos is not None:
+            u, Rr, _, pos = get_engine().sign_stdrng(0, sk, m, rng.key, rng.word_pos)
+            rng.seek(pos)
+        else:
+            u, Rr, _ = get_engine().sign(sk, m, _scalars(rng.random_scalars(len(sks))))
         return [Signature(_int(u[i]), p) for i, p in enumerate(_points_out(Rr))]
 
     @staticmethod
     def sign_double_batch(sks: Sequence["SecretKey"], rng: StdRng, msgs: Sequence[int]) -> List[SignatureDouble]:
-        nonces = rng.random_scalars(len(sks))
-        u, Rr, Rp, _ = get_engine().sign_double(_scalars([k._s for k in sks]), _fqs(msgs), _scalars(nonces))
+        sk, m = _scalars([k._s for k in sks]), _fqs(msgs)
+        if rng.word_pos is not None:
+            u, Rr, Rp, _, pos = get_engine().sign_stdrng(1, sk, m, rng.key, rng.word_pos)
+            rng.seek(pos)
+        else:
+            u, Rr, Rp, _ = get_engine().sign_double(sk, m, _scalars(rng.random_scalars(len(sks))))
         return [SignatureDouble(_int(u[i]), a, b) for i, (a, b) in enumerate(zip(_points_out(Rr), _points_out(Rp)))]
 
 
@@ -392,9 +419,12 @@ class SecretKeyVarGen:
 
     @staticmethod
     def sign_batch(sks: Sequence["SecretKeyVarGen"], rng: StdRng, msgs: Sequence[int]) -> List[SignatureVarGen]:
-        nonces = rng.random_scalars(len(sks))
-        u, Rr, _ = get_engine().sign_vargen(_scalars([k._s for k in sks]), _points([k._g for k in sks]), _fqs(msgs),
-                                            _scalars(nonces), affine=False)
+        sk, gen, m = _scalars([k._s for k in sks]), _points([k._g for k in sks]), _fqs(msgs)
+        if rng.word_pos is not None:
+            u, Rr, _, pos = get_engine().sign_stdrng(2, sk, m, rng.key, rng.word_pos, gen=gen, affine=False)
+            rng.seek(pos)
+        else:
+            u, Rr, _ = get_engine().sign_vargen(sk, gen, m, _scalars(rng.random_scalars(len(sks))), affine=False)
         return [SignatureVarGen(_int(u[i]), p) for i, p in enumerate(_points_out(Rr))]
 
 

@@ -21,6 +21,7 @@
 
 #include "../../include/schnorr_b200.h"
 #include "wire.cuh"
+#include "rng.cuh"
 #include "params_host.cuh"
 
 using namespace sb200;
@@ -62,7 +63,8 @@ enum Op : int {
   OP_DECOMPRESS, OP_COMPRESS, OP_FROM_WIDE, OP_VERIFY_BYTES, OP_SIGN_BYTES, OP_CHALLENGE, OP_VERIFY_EC,
   OP_VERIFY_DOUBLE_BYTES, OP_VERIFY_VARGEN_BYTES, OP_SIGN_DOUBLE_BYTES, OP_SIGN_VARGEN_BYTES,
   OP_CHALLENGE_DOUBLE, OP_VERIFY_DOUBLE_EC, OP_CHALLENGE_VARGEN, OP_VERIFY_VARGEN_EC, OP_POINTS_CHECK, OP_DBG_VERIFY_EC,
-  OP_DECODE_VERIFY, OP_WITNESS, OP_DBG_LAT3
+  OP_DECODE_VERIFY, OP_WITNESS, OP_DBG_LAT3,
+  OP_STDRNG, OP_SIGN_STDRNG, OP_SIGN_DOUBLE_STDRNG, OP_SIGN_VARGEN_STDRNG
 };
 
 struct KArgs {
@@ -83,6 +85,8 @@ struct KArgs {
   uint8_t* scratch;          // device-only rows between the kernels of one call (challenges, decoded byte-level inputs)
   const uint32_t* inv_mask;  // curve kernels: verdict word &= ~inv_mask word (tuples whose from_bytes failed)
   uint32_t* dec[MAX_IN];     // decode kernel: where the decoded arrays of the byte-level verify calls go
+  uint32_t rng_key[8];       // OP_STDRNG: the StdRng seed (secret: it reaches the device only as this kernel parameter)
+  uint64_t rng_word;         // OP_STDRNG: keystream word position of tuple 0 of this launch
 };
 
 // scheduling state of one warp-specialised launch (k_verify_ws): the next-tile counter, reset before every launch,
@@ -431,6 +435,12 @@ __global__ void __launch_bounds__(TPB, min_ctas(OP)) k_run(const KArgs a) {
 #pragma unroll
       for (int k = 0; k < 8; k++) r[k] = x.v[k];
     }
+    if (active) stg8(a.out[0] + i * 8, r);
+    return;
+  }
+  if (OP == OP_STDRNG) {  // -> out0: Field::random draw i at word rng_word + 16 i (aux 0: mod r canonical, aux 1: mod q Montgomery)
+    uint32_t r[8];
+    stdrng_random(a.rng_key, a.rng_word + 16u * (uint64_t)i, a.aux, r);
     if (active) stg8(a.out[0] + i * 8, r);
     return;
   }
@@ -879,6 +889,7 @@ struct Desc {
   uint32_t* out[MAX_OUT] = {};
   int out_words[MAX_OUT] = {};
   uint32_t* bitmap = nullptr;
+  const sb200_stdrng* rng = nullptr;  // OP_STDRNG and the seeded signers: key and word position of tuple 0
 };
 
 // Hades tables live in each device's constant memory: one parameter set per process and device.
@@ -1042,6 +1053,22 @@ int launch(sb200_ctx* ctx, Op op, const KArgs& a, cudaStream_t st) {
     return SB200_OK;
   }
 #endif
+  if (op == OP_SIGN_STDRNG || op == OP_SIGN_DOUBLE_STDRNG || op == OP_SIGN_VARGEN_STDRNG) {
+    // the chunk's nonces into a.scratch, then the unchanged sign kernel reads them from there as its nonce input
+    const Op sop = op == OP_SIGN_STDRNG ? OP_SIGN : op == OP_SIGN_DOUBLE_STDRNG ? OP_SIGN_DOUBLE : OP_SIGN_VARGEN;
+    KArgs g{};
+    g.n = a.n; g.aux = 0;
+    g.out[0] = (uint32_t*)a.scratch;
+    memcpy(g.rng_key, a.rng_key, sizeof(g.rng_key));
+    g.rng_word = a.rng_word;
+    k_run<OP_STDRNG><<<grid, TPB, 0, st>>>(g);
+    ctx->launches.fetch_add(1, std::memory_order_relaxed);
+    CU(cudaGetLastError());
+    KArgs s = a;
+    memset(s.rng_key, 0, sizeof(s.rng_key));
+    s.in[sop == OP_SIGN_VARGEN ? 3 : 2] = (const uint32_t*)a.scratch;
+    return launch(ctx, sop, s, st);
+  }
   if (a.flags & SB200_SIGN_OBLIVIOUS) {
     const size_t one = (size_t)CT_TABLE_WORDS * 4;
     switch (op) {
@@ -1072,7 +1099,7 @@ int launch(sb200_ctx* ctx, Op op, const KArgs& a, cudaStream_t st) {
     CASE(OP_KEYGEN_VARGEN) CASE(OP_DBG_FQ) CASE(OP_DBG_FR_MUL) CASE(OP_DBG_HADES)
     CASE(OP_DBG_SMUL) CASE(OP_DECOMPRESS) CASE(OP_COMPRESS) CASE(OP_FROM_WIDE)
     CASE(OP_SIGN_DOUBLE_BYTES) CASE(OP_SIGN_VARGEN_BYTES)
-    CASE(OP_POINTS_CHECK) CASE(OP_WITNESS) CASE(OP_DBG_LAT3)
+    CASE(OP_POINTS_CHECK) CASE(OP_WITNESS) CASE(OP_DBG_LAT3) CASE(OP_STDRNG)
 #undef CASE
     default: return SB200_ERR_ARG;
   }
@@ -1087,7 +1114,7 @@ bool splits_with_scratch(const Desc& d) {  // hash and curve kernels hand c over
 }
 
 // device-only bytes between the kernels of one call over n tuples: challenges (split verification without c_out),
-// plus the decoded rows and the invalid bitmap of the byte-level verify calls
+// the decoded rows and the invalid bitmap of the byte-level verify calls, the nonces of the seeded signers
 size_t scratch_bytes(const Desc& d, int64_t n) {
   size_t per = 0;
   int arrays = 0;
@@ -1095,6 +1122,7 @@ size_t scratch_bytes(const Desc& d, int64_t n) {
     case OP_VERIFY_BYTES: per = 32 + (16 + 8 + 16 + 8) * 4; arrays = 6; break;
     case OP_VERIFY_DOUBLE_BYTES: per = 32 + (16 * 4 + 8 + 8) * 4; arrays = 8; break;
     case OP_VERIFY_VARGEN_BYTES: per = 32 + (16 * 3 + 8 + 8) * 4; arrays = 7; break;
+    case OP_SIGN_STDRNG: case OP_SIGN_DOUBLE_STDRNG: case OP_SIGN_VARGEN_STDRNG: per = 32; arrays = 1; break;
     default: per = splits_with_scratch(d) ? 32 : 0; arrays = per ? 1 : 0; break;
   }
   if (!per) return 0;
@@ -1166,6 +1194,10 @@ int run_device(sb200_ctx* ctx, DevCtx& dc, const Desc& d, int64_t lo, int64_t hi
     a.n = cn; a.flags = d.flags; a.aux = d.aux; a.combG = dc.combG; a.combGp = dc.combGp;
     a.comb4G = dc.comb4; a.comb4Gp = dc.comb4 + CT_TABLE_WORDS;
     a.ws = dc.ws[slot]; a.nsm = dc.nsm; a.ec_scratch = dc.ec_scratch[slot]; a.persist = ctx->persist;
+    if (d.rng) {  // draw i belongs to tuple i: the chunk starts c0 draws into the stream
+      memcpy(a.rng_key, d.rng->key, sizeof(a.rng_key));
+      a.rng_word = d.rng->word_pos + 16u * (uint64_t)c0;
+    }
     for (int k = 0; k < d.nin; k++) {
       if (!d.in_words[k]) continue;
       size_t bytes = (size_t)cn * d.in_words[k] * 4;
@@ -1233,7 +1265,7 @@ int run(sb200_ctx* ctx, int64_t n, const Desc& d) {
   if (d.op == OP_VERIFY && SB_VERIFY_WS) allowed |= SB200_VERIFY_DUAL_PIPE;
   if (d.op == OP_VERIFY || d.op == OP_VERIFY_DOUBLE || d.op == OP_VERIFY_VARGEN) allowed |= SB200_CHECK_POINTS;
   if (d.op == OP_SIGN || d.op == OP_SIGN_DOUBLE || d.op == OP_SIGN_VARGEN || d.op == OP_KEYGEN || d.op == OP_KEYGEN_DOUBLE ||
-      d.op == OP_KEYGEN_VARGEN)
+      d.op == OP_KEYGEN_VARGEN || d.op == OP_SIGN_STDRNG || d.op == OP_SIGN_DOUBLE_STDRNG || d.op == OP_SIGN_VARGEN_STDRNG)
     allowed |= SB200_SIGN_OBLIVIOUS;
   if (d.flags & ~allowed) return SB200_ERR_ARG;
   for (int k = 0; k < d.nin; k++)
@@ -1256,6 +1288,10 @@ int run(sb200_ctx* ctx, int64_t n, const Desc& d) {
     a.n = n; a.flags = d.flags; a.aux = d.aux; a.combG = dc.combG; a.combGp = dc.combGp; a.bitmap = d.bitmap;
     a.comb4G = dc.comb4; a.comb4Gp = dc.comb4 + CT_TABLE_WORDS;
     a.ws = dc.ws[2]; a.nsm = dc.nsm; a.ec_scratch = dc.ec_scratch[2]; a.persist = ctx->persist;
+    if (d.rng) {
+      memcpy(a.rng_key, d.rng->key, sizeof(a.rng_key));
+      a.rng_word = d.rng->word_pos;
+    }
     for (int k = 0; k < d.nin; k++) a.in[k] = d.in[k];
     for (int k = 0; k < d.nout; k++) a.out[k] = d.out[k];
     if (const size_t need = scratch_bytes(d, n)) {
@@ -1614,6 +1650,33 @@ int sb200_scalars_from_wide(sb200_ctx* ctx, int64_t n, uint32_t flags, int field
   Desc d; d.op = OP_FROM_WIDE; d.flags = flags; d.aux = field; d.nin = 1; d.nout = 1;
   IN(0, (const uint32_t*)wide, 16); OUT(0, out, 8);
   return run(ctx, n, d);
+}
+// the position advances only when the call succeeds (as `&mut rng` would)
+int sb200_stdrng_random(sb200_ctx* ctx, int64_t n, uint32_t flags, int field, sb200_stdrng* rng, uint32_t* out) {
+  if (stdrng_random_args(n, flags, field, rng, out) != SB200_OK) return SB200_ERR_ARG;
+  Desc d; d.op = OP_STDRNG; d.flags = flags; d.aux = field; d.nin = 0; d.nout = 1; d.rng = rng;
+  OUT(0, out, 8);
+  const int rc = run(ctx, n, d);
+  if (rc == SB200_OK) rng->word_pos += 16u * (uint64_t)n;
+  return rc;
+}
+int sb200_sign_stdrng(sb200_ctx* ctx, int64_t n, uint32_t flags, int scheme, const uint32_t* sk, const uint32_t* msg,
+                      const uint32_t* gen, sb200_stdrng* rng, uint32_t* u_out, uint32_t* R_out, uint32_t* Rp_out, uint32_t* c_out) {
+  if (sign_stdrng_args(n, flags, scheme, sk, msg, gen, rng, u_out, R_out, Rp_out) != SB200_OK) return SB200_ERR_ARG;
+  static const Op ops[3] = {OP_SIGN_STDRNG, OP_SIGN_DOUBLE_STDRNG, OP_SIGN_VARGEN_STDRNG};
+  Desc d; d.op = ops[scheme]; d.flags = flags; d.nout = 4; d.rng = rng;
+  IN(0, sk, 8);
+  if (scheme == 2) {  // the inputs of sb200_sign_vargen (sk, gen, msg, nonce) without the nonce
+    d.nin = 4;
+    IN(1, gen, pt_words(flags)); IN(2, msg, 8); IN(3, nullptr, 0);
+  } else {  // those of sb200_sign / _double (sk, msg, nonce)
+    d.nin = 3;
+    IN(1, msg, 8); IN(2, nullptr, 0);
+  }
+  OUT(0, u_out, 8); OUT(1, R_out, 16); OUT(2, scheme == 1 ? Rp_out : nullptr, 16); OUT(3, c_out, 8);
+  const int rc = run(ctx, n, d);
+  if (rc == SB200_OK) rng->word_pos += 16u * (uint64_t)n;
+  return rc;
 }
 int sb200_fq_to_mont(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* in, uint32_t* out) {
   if (!out || (flags & SB200_POINTS_AFFINE)) return SB200_ERR_ARG;
