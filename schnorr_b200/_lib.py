@@ -74,6 +74,57 @@ def params_check(p: Params):
 def ark_rule(name: Optional[str]) -> int:
     return {None: ARK_ENV, "env": ARK_ENV, "cumsum": ARK_CUMSUM, "plain": ARK_PLAIN}[name]
 
+
+vp, u32p, i64, u32, ci = ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_uint32, ctypes.c_int
+_PROTOTYPES = {  # every symbol of include/schnorr_b200.h: (restype, argtypes)
+    "sb200_init": (ci, [ctypes.POINTER(ci), ci, ctypes.POINTER(vp)]),
+    "sb200_init_ex": (ci, [vp, ctypes.POINTER(ci), ci, ctypes.POINTER(vp)]),
+    "sb200_default_params": (ci, [ci, vp]),
+    "sb200_get_params": (ci, [vp, vp]),
+    "sb200_params_check": (ci, [vp, u32p]),
+    "sb200_points_check": (ci, [vp, i64, u32] + [u32p] * 2),
+    "sb200_sign_witness": (ci, [vp, i64, u32, ci] + [u32p] * 5),
+    "sb200_dbg_verify_ec": (ci, [vp, i64, u32] + [u32p] * 5),
+    "sb200_dbg_hades_tables": (ci, [vp, u32p]),
+    "sb200_destroy": (None, [vp]),
+    "sb200_strerror": (ctypes.c_char_p, [ci]),
+    "sb200_last_error": (ctypes.c_char_p, [vp]),
+    "sb200_device_count": (ci, [vp]),
+    "sb200_set_stream": (ci, [vp, vp]),
+    "sb200_launch_count": (ctypes.c_uint64, [vp]),
+    "sb200_host_alloc": (ci, [ctypes.c_size_t, ctypes.POINTER(vp)]),
+    "sb200_host_free": (None, [vp]),
+    "sb200_verify": (ci, [vp, i64, u32] + [u32p] * 6),
+    "sb200_verify_double": (ci, [vp, i64, u32] + [u32p] * 8),
+    "sb200_verify_vargen": (ci, [vp, i64, u32] + [u32p] * 7),
+    "sb200_sign": (ci, [vp, i64, u32] + [u32p] * 6),
+    "sb200_sign_double": (ci, [vp, i64, u32] + [u32p] * 7),
+    "sb200_sign_vargen": (ci, [vp, i64, u32] + [u32p] * 7),
+    "sb200_keygen": (ci, [vp, i64, u32] + [u32p] * 2),
+    "sb200_keygen_double": (ci, [vp, i64, u32] + [u32p] * 3),
+    "sb200_keygen_vargen": (ci, [vp, i64, u32] + [u32p] * 3),
+    "sb200_points_decompress": (ci, [vp, i64, u32] + [u32p] * 3),
+    "sb200_points_compress": (ci, [vp, i64, u32] + [u32p] * 2),
+    "sb200_scalars_from_wide": (ci, [vp, i64, u32, ci] + [u32p] * 2),
+    "sb200_stdrng_random": (ci, [vp, i64, u32, ci, vp, u32p]),
+    "sb200_sign_stdrng": (ci, [vp, i64, u32, ci] + [u32p] * 3 + [vp] + [u32p] * 4),
+    "sb200_fq_to_mont": (ci, [vp, i64, u32] + [u32p] * 2),
+    "sb200_fq_from_mont": (ci, [vp, i64, u32] + [u32p] * 2),
+    "sb200_verify_bytes": (ci, [vp, i64, u32] + [u32p] * 5),
+    "sb200_sign_bytes": (ci, [vp, i64, u32] + [u32p] * 5),
+    "sb200_verify_double_bytes": (ci, [vp, i64, u32] + [u32p] * 5),
+    "sb200_verify_vargen_bytes": (ci, [vp, i64, u32] + [u32p] * 5),
+    "sb200_sign_double_bytes": (ci, [vp, i64, u32] + [u32p] * 5),
+    "sb200_sign_vargen_bytes": (ci, [vp, i64, u32] + [u32p] * 5),
+    "sb200_dbg_fq": (ci, [vp, i64, ci] + [u32p] * 3),
+    "sb200_dbg_fr_mul": (ci, [vp, i64] + [u32p] * 3),
+    "sb200_dbg_lattice3": (ci, [vp, i64] + [u32p] * 3),
+    "sb200_dbg_hades": (ci, [vp, i64, ci, u32p]),
+    "sb200_dbg_scalar_mul": (ci, [vp, i64, u32, ci] + [u32p] * 3),
+}
+del vp, u32p, i64, u32, ci
+EXPORTED_SYMBOLS = list(_PROTOTYPES)
+
 _lib = None
 
 
@@ -91,71 +142,11 @@ def load_library() -> ctypes.CDLL:
             f"{LIB_PATH} not found: build it with `python -c 'import __graft_entry__ as g; g.build()'` "
             "(nvcc, sm_100a). There is no CPU fallback.")
     lib = ctypes.CDLL(LIB_PATH)
-    vp, u32p, i64, u32, ci = ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int64, ctypes.c_uint32, ctypes.c_int
-    sig = {
-        "sb200_init": (ci, [ctypes.POINTER(ci), ci, ctypes.POINTER(vp)]),
-        "sb200_init_ex": (ci, [vp, ctypes.POINTER(ci), ci, ctypes.POINTER(vp)]),
-        "sb200_default_params": (ci, [ci, vp]),
-        "sb200_get_params": (ci, [vp, vp]),
-        "sb200_params_check": (ci, [vp, u32p]),
-        "sb200_points_check": (ci, [vp, i64, u32] + [u32p] * 2),
-        "sb200_sign_witness": (ci, [vp, i64, u32, ci] + [u32p] * 5),
-        "sb200_dbg_verify_ec": (ci, [vp, i64, u32] + [u32p] * 5),
-        "sb200_dbg_hades_tables": (ci, [vp, u32p]),
-        "sb200_destroy": (None, [vp]),
-        "sb200_strerror": (ctypes.c_char_p, [ci]),
-        "sb200_last_error": (ctypes.c_char_p, [vp]),
-        "sb200_device_count": (ci, [vp]),
-        "sb200_set_stream": (ci, [vp, vp]),
-        "sb200_launch_count": (ctypes.c_uint64, [vp]),
-        "sb200_host_alloc": (ci, [ctypes.c_size_t, ctypes.POINTER(vp)]),
-        "sb200_host_free": (None, [vp]),
-        "sb200_verify": (ci, [vp, i64, u32] + [u32p] * 6),
-        "sb200_verify_double": (ci, [vp, i64, u32] + [u32p] * 8),
-        "sb200_verify_vargen": (ci, [vp, i64, u32] + [u32p] * 7),
-        "sb200_sign": (ci, [vp, i64, u32] + [u32p] * 6),
-        "sb200_sign_double": (ci, [vp, i64, u32] + [u32p] * 7),
-        "sb200_sign_vargen": (ci, [vp, i64, u32] + [u32p] * 7),
-        "sb200_keygen": (ci, [vp, i64, u32] + [u32p] * 2),
-        "sb200_keygen_double": (ci, [vp, i64, u32] + [u32p] * 3),
-        "sb200_keygen_vargen": (ci, [vp, i64, u32] + [u32p] * 3),
-        "sb200_points_decompress": (ci, [vp, i64, u32] + [u32p] * 3),
-        "sb200_points_compress": (ci, [vp, i64, u32] + [u32p] * 2),
-        "sb200_scalars_from_wide": (ci, [vp, i64, u32, ci] + [u32p] * 2),
-        "sb200_stdrng_random": (ci, [vp, i64, u32, ci, vp, u32p]),
-        "sb200_sign_stdrng": (ci, [vp, i64, u32, ci] + [u32p] * 3 + [vp] + [u32p] * 4),
-        "sb200_fq_to_mont": (ci, [vp, i64, u32] + [u32p] * 2),
-        "sb200_fq_from_mont": (ci, [vp, i64, u32] + [u32p] * 2),
-        "sb200_verify_bytes": (ci, [vp, i64, u32] + [u32p] * 5),
-        "sb200_sign_bytes": (ci, [vp, i64, u32] + [u32p] * 5),
-        "sb200_verify_double_bytes": (ci, [vp, i64, u32] + [u32p] * 5),
-        "sb200_verify_vargen_bytes": (ci, [vp, i64, u32] + [u32p] * 5),
-        "sb200_sign_double_bytes": (ci, [vp, i64, u32] + [u32p] * 5),
-        "sb200_sign_vargen_bytes": (ci, [vp, i64, u32] + [u32p] * 5),
-        "sb200_dbg_fq": (ci, [vp, i64, ci] + [u32p] * 3),
-        "sb200_dbg_fr_mul": (ci, [vp, i64] + [u32p] * 3),
-        "sb200_dbg_lattice3": (ci, [vp, i64] + [u32p] * 3),
-        "sb200_dbg_hades": (ci, [vp, i64, ci, u32p]),
-        "sb200_dbg_scalar_mul": (ci, [vp, i64, u32, ci] + [u32p] * 3),
-    }
-    for name, (res, args) in sig.items():
+    for name, (res, args) in _PROTOTYPES.items():
         fn = getattr(lib, name)  # AttributeError if the library does not export a declared symbol
         fn.restype, fn.argtypes = res, args
     _lib = lib
     return lib
-
-
-EXPORTED_SYMBOLS = [
-    "sb200_sign_witness", "sb200_init_ex", "sb200_default_params", "sb200_get_params", "sb200_params_check", "sb200_points_check", "sb200_dbg_verify_ec",
-    "sb200_dbg_hades_tables",
-    "sb200_init", "sb200_destroy", "sb200_strerror", "sb200_last_error", "sb200_device_count", "sb200_set_stream",
-    "sb200_launch_count", "sb200_host_alloc", "sb200_host_free", "sb200_verify", "sb200_verify_double",
-    "sb200_verify_vargen", "sb200_sign", "sb200_sign_double", "sb200_sign_vargen", "sb200_keygen",
-    "sb200_keygen_double", "sb200_keygen_vargen", "sb200_points_decompress", "sb200_points_compress",
-    "sb200_scalars_from_wide", "sb200_stdrng_random", "sb200_sign_stdrng", "sb200_fq_to_mont", "sb200_fq_from_mont", "sb200_verify_bytes", "sb200_sign_bytes",
-    "sb200_verify_double_bytes", "sb200_verify_vargen_bytes", "sb200_sign_double_bytes", "sb200_sign_vargen_bytes", "sb200_dbg_fq", "sb200_dbg_fr_mul", "sb200_dbg_lattice3", "sb200_dbg_hades",
-    "sb200_dbg_scalar_mul",
-]
 
 
 def aligned_empty(shape, dtype=np.uint32, align=64) -> np.ndarray:

@@ -644,19 +644,6 @@ __global__ void __launch_bounds__(TPB, ec_p_ctas(SCHEME)) k_curve_p(const KArgs 
     if ((threadIdx.x & 31) == 0 && active) a.bitmap[i >> 5] = a.inv_mask ? word & ~a.inv_mask[i >> 5] : word;
   }
 }
-// A batch that fits one wave of resident CTAs gains nothing from the persistent form (no slot is reused, the scratch region is
-// cold in L2): it runs the local-memory kernel (measured at 2^16 tuples: 16.4 vs 15.0 M verifies/s).
-template <int SCHEME>
-inline void launch_curve_p(const KArgs& a, unsigned grid, cudaStream_t st) {
-  if (a.persist == 2 || (a.persist == 0 && grid <= (unsigned)(ec_p_ctas(SCHEME) * a.nsm))) {
-    if (SCHEME == 0) k_run<OP_VERIFY_EC><<<grid, TPB, 0, st>>>(a);
-    else if (SCHEME == 1) k_run<OP_VERIFY_DOUBLE_EC><<<grid, TPB, 0, st>>>(a);
-    else k_run<OP_VERIFY_VARGEN_EC><<<grid, TPB, 0, st>>>(a);
-    return;
-  }
-  k_curve_p<SCHEME><<<std::min<unsigned>(grid, (unsigned)(ec_p_ctas(SCHEME) * a.nsm)), TPB, ec_p_smem(SCHEME), st>>>(a, a.ec_scratch);
-}
-
 #endif  // SB_EC_GLOBAL_TABLES
 
 // Fixed-base signing / key generation with several tuples per thread: the scalar multiples of G (and G') are
@@ -890,6 +877,7 @@ struct Desc {
   int out_words[MAX_OUT] = {};
   uint32_t* bitmap = nullptr;
   const sb200_stdrng* rng = nullptr;  // OP_STDRNG and the seeded signers: key and word position of tuple 0
+  unsigned need = 0;  // outputs that may not be null: bit k for out[k], bit MAX_OUT for the bitmap
 };
 
 // Hades tables live in each device's constant memory: one parameter set per process and device.
@@ -941,192 +929,216 @@ namespace {
     }                                                                                         \
   } while (0)
 
+// ---- what the library knows about each operation: one row per Op, in Op order ------------------------------------------
+// How an op launches.  INTERNAL: a stage of other ops, never called by itself.  ONE: `kernel`, one tuple per thread.
+// FIXED: the k_fixed_batch `kernel` (or its SB200_SIGN_OBLIVIOUS form `ct`), fixed_k(op) tuples per thread.  VERIFY:
+// challenge kernel, then curve kernel, the challenges through c_out or scratch.  VERIFY_BYTES: decode kernel, then VERIFY
+// on the decoded rows.  SIGN_STDRNG: the nonces drawn into scratch, then the scheme's sign op.  DBG_VERIFY_EC: the curve
+// kernel alone, on the caller's challenges.
+enum Form : uint8_t { INTERNAL, ONE, FIXED, VERIFY, VERIFY_BYTES, SIGN_STDRNG, DBG_VERIFY_EC };
+using KFn = void (*)(KArgs);
+struct OpInfo {
+  Form form;
+  uint32_t flags;       // the SB200_* flags the op accepts: any other one is SB200_ERR_ARG
+  int scheme;           // VERIFY*, SIGN_STDRNG, FIXED: 0 single-key, 1 double-key (two combs), 2 variable generator
+  KFn kernel, ct;
+  size_t ct_smem;       // shared memory of `ct`: one or two 4-bit combs
+  uint32_t forced;      // flags the op always runs with: the byte-level verifications hand affine points between kernels
+  unsigned scratch;     // device-only bytes per tuple between the kernels of one call, in `scratch_arrays` arrays: the
+  int scratch_arrays;   // challenges or nonces, and the decoded rows (points 64 B, u and m 32 B) and invalid bitmap
+};
+constexpr OpInfo row(Form form, uint32_t flags = 0, int scheme = 0, KFn kernel = nullptr, KFn ct = nullptr) {
+  const unsigned points = scheme == 0 ? 2 : scheme == 1 ? 4 : 3, rows = form == VERIFY_BYTES ? 64 * points + 64 : 0;
+  const bool handover = form == VERIFY || form == VERIFY_BYTES || form == SIGN_STDRNG;
+  return {form, flags, scheme, kernel, ct, ct ? (size_t)(scheme == 1 ? 2 : 1) * CT_TABLE_WORDS * 4 : 0,
+          form == VERIFY_BYTES ? (uint32_t)SB200_POINTS_AFFINE : 0u, handover ? 32 + rows : 0u,
+          handover ? (rows ? (int)points + 4 : 1) : 0};
+}
+constexpr uint32_t D = SB200_DEVICE_PTRS, AD = SB200_POINTS_AFFINE | D, CHK = AD | SB200_CHECK_POINTS;
+constexpr uint32_t OBL = AD | SB200_SIGN_OBLIVIOUS, DUAL = SB_VERIFY_WS ? SB200_VERIFY_DUAL_PIPE : 0;
+constexpr OpInfo OPS[] = {
+#if SB_VERIFY_SPLIT
+    row(VERIFY, CHK | DUAL, 0),  // OP_VERIFY
+    row(VERIFY, CHK, 1),         // OP_VERIFY_DOUBLE
+#else  // the fused one-launch verification kernels are only built when the split form is switched off
+    row(ONE, CHK | DUAL, 0, k_run<OP_VERIFY>),
+    row(ONE, CHK, 1, k_run<OP_VERIFY_DOUBLE>),
+#endif
+#if SB_VERIFY_SPLIT && SB_VARGEN_SPLIT
+    row(VERIFY, CHK, 2),  // OP_VERIFY_VARGEN
+#else
+    row(ONE, CHK, 2, k_run<OP_VERIFY_VARGEN>),
+#endif
+    row(FIXED, OBL, 0, k_fixed_batch<OP_SIGN>, k_fixed_batch<OP_SIGN, true>),
+    row(FIXED, OBL, 1, k_fixed_batch<OP_SIGN_DOUBLE>, k_fixed_batch<OP_SIGN_DOUBLE, true>),
+    row(ONE, OBL, 0, k_run<OP_SIGN_VARGEN>),
+    row(FIXED, OBL, 0, k_fixed_batch<OP_KEYGEN>, k_fixed_batch<OP_KEYGEN, true>),
+    row(FIXED, OBL, 1, k_fixed_batch<OP_KEYGEN_DOUBLE>, k_fixed_batch<OP_KEYGEN_DOUBLE, true>),
+    row(ONE, OBL, 0, k_run<OP_KEYGEN_VARGEN>),
+    row(ONE, D, 0, k_run<OP_DBG_FQ>),
+    row(ONE, AD, 0, k_run<OP_DBG_FR_MUL>),
+    row(ONE, AD, 0, k_run<OP_DBG_HADES>),
+    row(ONE, AD, 0, k_run<OP_DBG_SMUL>),
+    row(ONE, D, 0, k_run<OP_DECOMPRESS>),
+    row(ONE, AD, 0, k_run<OP_COMPRESS>),
+    row(ONE, D, 0, k_run<OP_FROM_WIDE>),
+    row(VERIFY_BYTES, D, 0),  // OP_VERIFY_BYTES
+    row(FIXED, D, 0, k_fixed_batch<OP_SIGN_BYTES>),
+    row(INTERNAL),  // OP_CHALLENGE
+    row(INTERNAL),  // OP_VERIFY_EC
+    row(VERIFY_BYTES, D, 1),  // OP_VERIFY_DOUBLE_BYTES
+    row(VERIFY_BYTES, D, 2),  // OP_VERIFY_VARGEN_BYTES
+    row(ONE, D, 0, k_run<OP_SIGN_DOUBLE_BYTES>),
+    row(ONE, D, 0, k_run<OP_SIGN_VARGEN_BYTES>),
+    row(INTERNAL),  // OP_CHALLENGE_DOUBLE
+    row(INTERNAL),  // OP_VERIFY_DOUBLE_EC
+    row(INTERNAL),  // OP_CHALLENGE_VARGEN
+    row(INTERNAL),  // OP_VERIFY_VARGEN_EC
+    row(ONE, AD, 0, k_run<OP_POINTS_CHECK>),
+    row(DBG_VERIFY_EC, AD, 0),  // OP_DBG_VERIFY_EC
+    row(INTERNAL),  // OP_DECODE_VERIFY
+    row(ONE, AD, 0, k_run<OP_WITNESS>),
+    row(ONE, AD, 0, k_run<OP_DBG_LAT3>),
+    row(ONE, D, 0, k_run<OP_STDRNG>),
+    row(SIGN_STDRNG, D | SB200_SIGN_OBLIVIOUS, 0),  // OP_SIGN_STDRNG
+    row(SIGN_STDRNG, D | SB200_SIGN_OBLIVIOUS, 1),  // OP_SIGN_DOUBLE_STDRNG
+    row(SIGN_STDRNG, OBL, 2),                       // OP_SIGN_VARGEN_STDRNG
+};
+static_assert(sizeof(OPS) / sizeof(OPS[0]) == OP_SIGN_VARGEN_STDRNG + 1, "one row per Op");
+
+// ---- launches ---------------------------------------------------------------------------------------------------------
+struct Launcher {  // issues kernels on one stream and counts them (sb200_launch_count)
+  sb200_ctx* ctx;
+  cudaStream_t st;
+  template <class... P, class... A>
+  void operator()(void (*k)(P...), unsigned grid, unsigned block, size_t smem, const A&... args) const {
+    k<<<grid, block, smem, st>>>(args...);
+    ctx->launches.fetch_add(1, std::memory_order_relaxed);
+  }
+};
+
+// The curve half of a verification.  With SB_EC_GLOBAL_TABLES a batch above one wave of resident CTAs runs the persistent
+// form, which takes its tuples from the counter a.ws->tile: the challenge kernel before it resets the counter, without one
+// (reset_tile) it is cleared here.  A batch that fits one wave gains nothing from the persistent form (no slot is reused,
+// the scratch region is cold in L2): it runs the local-memory kernel (measured at 2^16 tuples: 16.4 vs 15.0 M verifies/s).
+int launch_curve(const Launcher& go, int scheme, const KArgs& a, unsigned grid, bool reset_tile = false) {
+  static const KFn one_shot[3] = {k_run<OP_VERIFY_EC>, k_run<OP_VERIFY_DOUBLE_EC>, k_run<OP_VERIFY_VARGEN_EC>};
+#if SB_EC_GLOBAL_TABLES
+  static void (*const persistent[3])(KArgs, pniels*) = {k_curve_p<0>, k_curve_p<1>, k_curve_p<2>};
+  sb200_ctx* ctx = go.ctx;
+  if (reset_tile) CU(cudaMemsetAsync(&a.ws->tile, 0, sizeof(unsigned), go.st));
+  const unsigned wave = (unsigned)(ec_p_ctas(scheme) * a.nsm);
+  if (a.persist == 1 || (a.persist == 0 && grid > wave)) {
+    go(persistent[scheme], std::min(grid, wave), TPB, ec_p_smem(scheme), a, a.ec_scratch);
+    return SB200_OK;
+  }
+#endif
+  go(one_shot[scheme], grid, TPB, 0, a);
+  return SB200_OK;
+}
+
+int launch_verify(const Launcher& go, int scheme, const KArgs& a, unsigned grid) {  // a.out[0]: where the challenges go
+  static const KFn challenge[3] = {k_run<OP_CHALLENGE>, k_run<OP_CHALLENGE_DOUBLE>, k_run<OP_CHALLENGE_VARGEN>};
+  go(challenge[scheme], grid, TPB, 0, a);
+  return launch_curve(go, scheme, a, grid);
+}
+
 int launch(sb200_ctx* ctx, Op op, const KArgs& a, cudaStream_t st) {
   if (a.n <= 0) return SB200_OK;
-  unsigned grid = (unsigned)((a.n + TPB - 1) / TPB);
-  auto gridk = [&](int op_) { return (unsigned)((a.n + TPB * fixed_k(op_) - 1) / (TPB * fixed_k(op_))); };
+  const OpInfo& o = OPS[op];
+  const Launcher go{ctx, st};
+  const unsigned grid = (unsigned)((a.n + TPB - 1) / TPB);
+  int rc = SB200_OK;
 #if SB_VERIFY_WS
   if (op == OP_VERIFY && (a.flags & SB200_VERIFY_DUAL_PIPE)) {  // persistent warp-specialised kernel, one CTA per SM
     CU(cudaMemsetAsync(&a.ws->tile, 0, sizeof(unsigned), st));
-    unsigned ntiles = (unsigned)((a.n + WS_TILE - 1) / WS_TILE);
-    unsigned g = std::min<unsigned>(ntiles, (unsigned)a.nsm);
-    k_verify_ws<<<g, WS_THREADS, WS_SMEM, st>>>(a);
-    ctx->launches.fetch_add(1, std::memory_order_relaxed);
+    go(k_verify_ws, std::min<unsigned>((unsigned)((a.n + WS_TILE - 1) / WS_TILE), (unsigned)a.nsm), WS_THREADS, WS_SMEM, a);
     CU(cudaGetLastError());
     return SB200_OK;
   }
 #endif
-  if (op == OP_VERIFY_BYTES || op == OP_VERIFY_DOUBLE_BYTES || op == OP_VERIFY_VARGEN_BYTES) {
-    // decode kernel -> challenge kernel -> curve kernel, the decoded rows and the challenges in a.scratch
-    const int scheme = op == OP_VERIFY_BYTES ? 0 : op == OP_VERIFY_DOUBLE_BYTES ? 1 : 2;
-    const int npk = scheme == 0 ? 1 : 2, nr = scheme == 1 ? 2 : 1, narr = npk + 1 + nr + 1;
-    uint8_t* p = a.scratch;
-    auto carve = [&](size_t bytes) { uint8_t* r = p; p += (bytes + 63) & ~(size_t)63; return (uint32_t*)r; };
-    KArgs dk = a, v = a;
-    dk.aux = scheme;
-    v.flags = (a.flags & SB200_DEVICE_PTRS) | SB200_POINTS_AFFINE;
-    v.out[0] = carve((size_t)a.n * 32);
-    for (int k = 0; k < narr; k++) {
-      const bool is_scalar = (k == npk) || (k == narr - 1);  // u and m are 8 words, points 16
-      dk.dec[k] = carve((size_t)a.n * (is_scalar ? 32 : 64));
-      v.in[k] = dk.dec[k];
+  switch (o.form) {
+    case ONE:
+    case FIXED: {
+      const bool ct = o.ct && (a.flags & SB200_SIGN_OBLIVIOUS);
+      const int64_t per_cta = TPB * (o.form == FIXED ? fixed_k(op) : 1);
+      go(ct ? o.ct : o.kernel, (unsigned)((a.n + per_cta - 1) / per_cta), TPB, ct ? o.ct_smem : 0, a);
+      break;
     }
-    dk.bitmap = a.out[0] ? a.out[0] : carve((size_t)((a.n + 31) / 32) * 4);  // the caller's `invalid` or scratch
-    v.inv_mask = dk.bitmap;
-    for (int k = 1; k < MAX_OUT; k++) v.out[k] = nullptr;
-    k_run<OP_DECODE_VERIFY><<<grid, TPB, 0, st>>>(dk);
-    if (scheme == 0) {
-      k_run<OP_CHALLENGE><<<grid, TPB, 0, st>>>(v);
-#if SB_EC_GLOBAL_TABLES
-      launch_curve_p<0>(v, grid, st);
-#else
-      k_run<OP_VERIFY_EC><<<grid, TPB, 0, st>>>(v);
-#endif
-    } else if (scheme == 1) {
-      k_run<OP_CHALLENGE_DOUBLE><<<grid, TPB, 0, st>>>(v);
-#if SB_EC_GLOBAL_TABLES
-      launch_curve_p<1>(v, grid, st);
-#else
-      k_run<OP_VERIFY_DOUBLE_EC><<<grid, TPB, 0, st>>>(v);
-#endif
-    } else {
-      k_run<OP_CHALLENGE_VARGEN><<<grid, TPB, 0, st>>>(v);
-#if SB_EC_GLOBAL_TABLES
-      launch_curve_p<2>(v, grid, st);
-#else
-      k_run<OP_VERIFY_VARGEN_EC><<<grid, TPB, 0, st>>>(v);
-#endif
+    case VERIFY:  // a.out[0] is always set here: the caller's c_out or scratch
+      rc = launch_verify(go, o.scheme, a, grid);
+      break;
+    case VERIFY_BYTES: {  // decode kernel -> challenge kernel -> curve kernel, the decoded rows and the challenges in a.scratch
+      const int npk = o.scheme == 0 ? 1 : 2, nr = o.scheme == 1 ? 2 : 1, narr = npk + 1 + nr + 1;
+      uint8_t* p = a.scratch;
+      auto carve = [&](size_t bytes) { uint8_t* r = p; p += (bytes + 63) & ~(size_t)63; return (uint32_t*)r; };
+      KArgs dk = a, v = a;
+      dk.aux = o.scheme;
+      v.out[0] = carve((size_t)a.n * 32);
+      for (int k = 0; k < narr; k++) {
+        const bool is_scalar = (k == npk) || (k == narr - 1);  // u and m are 8 words, points 16
+        dk.dec[k] = carve((size_t)a.n * (is_scalar ? 32 : 64));
+        v.in[k] = dk.dec[k];
+      }
+      dk.bitmap = a.out[0] ? a.out[0] : carve((size_t)((a.n + 31) / 32) * 4);  // the caller's `invalid` or scratch
+      v.inv_mask = dk.bitmap;
+      for (int k = 1; k < MAX_OUT; k++) v.out[k] = nullptr;
+      go(k_run<OP_DECODE_VERIFY>, grid, TPB, 0, dk);
+      rc = launch_verify(go, o.scheme, v, grid);
+      break;
     }
-    ctx->launches.fetch_add(3, std::memory_order_relaxed);
-    CU(cudaGetLastError());
-    return SB200_OK;
-  }
-  if (op == OP_DBG_VERIFY_EC) {  // in: pk, u, R, c -> bitmap: the production curve kernel, in the form the batch size picks,
-                                 // fed the caller's challenges where the challenge kernel would have written them
-    KArgs v = a;
-    v.out[0] = const_cast<uint32_t*>(a.in[3]);
-    v.in[3] = nullptr;
-#if SB_EC_GLOBAL_TABLES
-    CU(cudaMemsetAsync(&a.ws->tile, 0, sizeof(unsigned), st));  // the persistent form's work counter
-    launch_curve_p<0>(v, grid, st);
-#else
-    k_run<OP_VERIFY_EC><<<grid, TPB, 0, st>>>(v);
-#endif
-    ctx->launches.fetch_add(1, std::memory_order_relaxed);
-    CU(cudaGetLastError());
-    return SB200_OK;
-  }
-#if SB_VERIFY_SPLIT
-  if (op == OP_VERIFY) {  // a.out[0] is always set here: the caller's c_out or scratch
-    k_run<OP_CHALLENGE><<<grid, TPB, 0, st>>>(a);
-#if SB_EC_GLOBAL_TABLES
-    launch_curve_p<0>(a, grid, st);
-#else
-    k_run<OP_VERIFY_EC><<<grid, TPB, 0, st>>>(a);
-#endif
-    ctx->launches.fetch_add(2, std::memory_order_relaxed);
-    CU(cudaGetLastError());
-    return SB200_OK;
-  }
-#if SB_VARGEN_SPLIT
-  if (op == OP_VERIFY_VARGEN) {
-    k_run<OP_CHALLENGE_VARGEN><<<grid, TPB, 0, st>>>(a);
-#if SB_EC_GLOBAL_TABLES
-    launch_curve_p<2>(a, grid, st);
-#else
-    k_run<OP_VERIFY_VARGEN_EC><<<grid, TPB, 0, st>>>(a);
-#endif
-    ctx->launches.fetch_add(2, std::memory_order_relaxed);
-    CU(cudaGetLastError());
-    return SB200_OK;
-  }
-#endif
-  if (op == OP_VERIFY_DOUBLE) {
-    k_run<OP_CHALLENGE_DOUBLE><<<grid, TPB, 0, st>>>(a);
-#if SB_EC_GLOBAL_TABLES
-    launch_curve_p<1>(a, grid, st);
-#else
-    k_run<OP_VERIFY_DOUBLE_EC><<<grid, TPB, 0, st>>>(a);
-#endif
-    ctx->launches.fetch_add(2, std::memory_order_relaxed);
-    CU(cudaGetLastError());
-    return SB200_OK;
-  }
-#endif
-  if (op == OP_SIGN_STDRNG || op == OP_SIGN_DOUBLE_STDRNG || op == OP_SIGN_VARGEN_STDRNG) {
-    // the chunk's nonces into a.scratch, then the unchanged sign kernel reads them from there as its nonce input
-    const Op sop = op == OP_SIGN_STDRNG ? OP_SIGN : op == OP_SIGN_DOUBLE_STDRNG ? OP_SIGN_DOUBLE : OP_SIGN_VARGEN;
-    KArgs g{};
-    g.n = a.n; g.aux = 0;
-    g.out[0] = (uint32_t*)a.scratch;
-    memcpy(g.rng_key, a.rng_key, sizeof(g.rng_key));
-    g.rng_word = a.rng_word;
-    k_run<OP_STDRNG><<<grid, TPB, 0, st>>>(g);
-    ctx->launches.fetch_add(1, std::memory_order_relaxed);
-    CU(cudaGetLastError());
-    KArgs s = a;
-    memset(s.rng_key, 0, sizeof(s.rng_key));
-    s.in[sop == OP_SIGN_VARGEN ? 3 : 2] = (const uint32_t*)a.scratch;
-    return launch(ctx, sop, s, st);
-  }
-  if (a.flags & SB200_SIGN_OBLIVIOUS) {
-    const size_t one = (size_t)CT_TABLE_WORDS * 4;
-    switch (op) {
-      case OP_SIGN: k_fixed_batch<OP_SIGN, true><<<gridk(OP_SIGN), TPB, one, st>>>(a); break;
-      case OP_SIGN_DOUBLE: k_fixed_batch<OP_SIGN_DOUBLE, true><<<gridk(OP_SIGN_DOUBLE), TPB, 2 * one, st>>>(a); break;
-      case OP_KEYGEN: k_fixed_batch<OP_KEYGEN, true><<<gridk(OP_KEYGEN), TPB, one, st>>>(a); break;
-      case OP_KEYGEN_DOUBLE: k_fixed_batch<OP_KEYGEN_DOUBLE, true><<<gridk(OP_KEYGEN_DOUBLE), TPB, 2 * one, st>>>(a); break;
-      case OP_SIGN_VARGEN: k_run<OP_SIGN_VARGEN><<<grid, TPB, 0, st>>>(a); break;
-      case OP_KEYGEN_VARGEN: k_run<OP_KEYGEN_VARGEN><<<grid, TPB, 0, st>>>(a); break;
-      default: return SB200_ERR_ARG;
+    case DBG_VERIFY_EC: {  // in: pk, u, R, c -> bitmap: the production curve kernel, in the form the batch size picks,
+                           // fed the caller's challenges where the challenge kernel would have written them
+      KArgs v = a;
+      v.out[0] = const_cast<uint32_t*>(a.in[3]);
+      v.in[3] = nullptr;
+      rc = launch_curve(go, 0, v, grid, true);
+      break;
     }
-    ctx->launches.fetch_add(1, std::memory_order_relaxed);
-    CU(cudaGetLastError());
-    return SB200_OK;
+    case SIGN_STDRNG: {  // the chunk's nonces into a.scratch, then the unchanged sign kernel reads them from there as its nonce input
+      KArgs g{};
+      g.n = a.n;
+      g.out[0] = (uint32_t*)a.scratch;
+      memcpy(g.rng_key, a.rng_key, sizeof(g.rng_key));
+      g.rng_word = a.rng_word;
+      go(k_run<OP_STDRNG>, grid, TPB, 0, g);
+      CU(cudaGetLastError());  // no signature from a failed draw: the scratch row would still hold an earlier call's nonces
+      KArgs s = a;
+      memset(s.rng_key, 0, sizeof(s.rng_key));
+      s.in[o.scheme == 2 ? 3 : 2] = (const uint32_t*)a.scratch;
+      static const Op sign_op[3] = {OP_SIGN, OP_SIGN_DOUBLE, OP_SIGN_VARGEN};
+      return launch(ctx, sign_op[o.scheme], s, st);
+    }
+    default:
+      return SB200_ERR_ARG;
   }
-  switch (op) {
-#define CASEK(O) case O: k_fixed_batch<O><<<gridk(O), TPB, 0, st>>>(a); break;
-    CASEK(OP_SIGN) CASEK(OP_SIGN_DOUBLE) CASEK(OP_KEYGEN) CASEK(OP_KEYGEN_DOUBLE) CASEK(OP_SIGN_BYTES)
-#undef CASEK
-#define CASE(O) case O: k_run<O><<<grid, TPB, 0, st>>>(a); break;
-#if !SB_VERIFY_SPLIT  // the fused one-launch verification kernels: only built when the split form is switched off
-    CASE(OP_VERIFY) CASE(OP_VERIFY_DOUBLE)
-#endif
-#if !(SB_VERIFY_SPLIT && SB_VARGEN_SPLIT)
-    CASE(OP_VERIFY_VARGEN)
-#endif
-    CASE(OP_SIGN_VARGEN)
-    CASE(OP_KEYGEN_VARGEN) CASE(OP_DBG_FQ) CASE(OP_DBG_FR_MUL) CASE(OP_DBG_HADES)
-    CASE(OP_DBG_SMUL) CASE(OP_DECOMPRESS) CASE(OP_COMPRESS) CASE(OP_FROM_WIDE)
-    CASE(OP_SIGN_DOUBLE_BYTES) CASE(OP_SIGN_VARGEN_BYTES)
-    CASE(OP_POINTS_CHECK) CASE(OP_WITNESS) CASE(OP_DBG_LAT3) CASE(OP_STDRNG)
-#undef CASE
-    default: return SB200_ERR_ARG;
-  }
-  ctx->launches.fetch_add(1, std::memory_order_relaxed);
+  if (rc) return rc;
   CU(cudaGetLastError());
   return SB200_OK;
 }
 
 bool splits_with_scratch(const Desc& d) {  // hash and curve kernels hand c over in memory
-  return SB_VERIFY_SPLIT && ((d.op == OP_VERIFY && !(d.flags & SB200_VERIFY_DUAL_PIPE)) || d.op == OP_VERIFY_DOUBLE ||
-                             (SB_VARGEN_SPLIT && d.op == OP_VERIFY_VARGEN)) && !d.out[0];
+  return OPS[d.op].form == VERIFY && !(d.flags & SB200_VERIFY_DUAL_PIPE) && !d.out[0];
 }
 
-// device-only bytes between the kernels of one call over n tuples: challenges (split verification without c_out),
-// the decoded rows and the invalid bitmap of the byte-level verify calls, the nonces of the seeded signers
+// device-only bytes between the kernels of one call over n tuples
 size_t scratch_bytes(const Desc& d, int64_t n) {
-  size_t per = 0;
-  int arrays = 0;
-  switch (d.op) {
-    case OP_VERIFY_BYTES: per = 32 + (16 + 8 + 16 + 8) * 4; arrays = 6; break;
-    case OP_VERIFY_DOUBLE_BYTES: per = 32 + (16 * 4 + 8 + 8) * 4; arrays = 8; break;
-    case OP_VERIFY_VARGEN_BYTES: per = 32 + (16 * 3 + 8 + 8) * 4; arrays = 7; break;
-    case OP_SIGN_STDRNG: case OP_SIGN_DOUBLE_STDRNG: case OP_SIGN_VARGEN_STDRNG: per = 32; arrays = 1; break;
-    default: per = splits_with_scratch(d) ? 32 : 0; arrays = per ? 1 : 0; break;
+  const OpInfo& o = OPS[d.op];
+  if (!o.scratch || (o.form == VERIFY && !splits_with_scratch(d))) return 0;
+  return (size_t)n * o.scratch + (size_t)((n + 31) / 32) * 4 + 64 * (o.scratch_arrays + 1);
+}
+
+// the kernel arguments every launch of a call shares; `first`: index of the launch's tuple 0 in the call
+KArgs kargs(const sb200_ctx* ctx, const DevCtx& dc, int slot, const Desc& d, int64_t n, int64_t first) {
+  KArgs a{};
+  a.n = n; a.flags = d.flags; a.aux = d.aux; a.combG = dc.combG; a.combGp = dc.combGp;
+  a.comb4G = dc.comb4; a.comb4Gp = dc.comb4 + CT_TABLE_WORDS;
+  a.ws = dc.ws[slot]; a.nsm = dc.nsm; a.ec_scratch = dc.ec_scratch[slot]; a.persist = ctx->persist;
+  if (d.rng) {  // draw i belongs to tuple i: tuple `first` is that many draws into the stream
+    memcpy(a.rng_key, d.rng->key, sizeof(a.rng_key));
+    a.rng_word = d.rng->word_pos + 16u * (uint64_t)first;
   }
-  if (!per) return 0;
-  return (size_t)n * per + (size_t)((n + 31) / 32) * 4 + 64 * (arrays + 1);
+  return a;
 }
 
 bool host_pinned(const void* p) {
@@ -1190,14 +1202,7 @@ int run_device(sb200_ctx* ctx, DevCtx& dc, const Desc& d, int64_t lo, int64_t hi
     cudaStream_t st = dc.stream[slot];
     uint8_t *p = dc.arena[slot], *hi_p = dc.hin[slot].p, *ho_p = dc.hout[slot].p;
     auto carve = [](uint8_t*& q, size_t bytes) { uint8_t* r = q; q += (bytes + 63) & ~(size_t)63; return r; };
-    KArgs a{};
-    a.n = cn; a.flags = d.flags; a.aux = d.aux; a.combG = dc.combG; a.combGp = dc.combGp;
-    a.comb4G = dc.comb4; a.comb4Gp = dc.comb4 + CT_TABLE_WORDS;
-    a.ws = dc.ws[slot]; a.nsm = dc.nsm; a.ec_scratch = dc.ec_scratch[slot]; a.persist = ctx->persist;
-    if (d.rng) {  // draw i belongs to tuple i: the chunk starts c0 draws into the stream
-      memcpy(a.rng_key, d.rng->key, sizeof(a.rng_key));
-      a.rng_word = d.rng->word_pos + 16u * (uint64_t)c0;
-    }
+    KArgs a = kargs(ctx, dc, slot, d, cn, c0);
     for (int k = 0; k < d.nin; k++) {
       if (!d.in_words[k]) continue;
       size_t bytes = (size_t)cn * d.in_words[k] * 4;
@@ -1259,19 +1264,14 @@ void quiesce(DevCtx& dc) {
   cudaGetLastError();
 }
 
-int run(sb200_ctx* ctx, int64_t n, const Desc& d) {
-  if (!ctx || n < 0) return SB200_ERR_ARG;
-  uint32_t allowed = SB200_POINTS_AFFINE | SB200_DEVICE_PTRS;
-  if (d.op == OP_VERIFY && SB_VERIFY_WS) allowed |= SB200_VERIFY_DUAL_PIPE;
-  if (d.op == OP_VERIFY || d.op == OP_VERIFY_DOUBLE || d.op == OP_VERIFY_VARGEN) allowed |= SB200_CHECK_POINTS;
-  if (d.op == OP_SIGN || d.op == OP_SIGN_DOUBLE || d.op == OP_SIGN_VARGEN || d.op == OP_KEYGEN || d.op == OP_KEYGEN_DOUBLE ||
-      d.op == OP_KEYGEN_VARGEN || d.op == OP_SIGN_STDRNG || d.op == OP_SIGN_DOUBLE_STDRNG || d.op == OP_SIGN_VARGEN_STDRNG)
-    allowed |= SB200_SIGN_OBLIVIOUS;
-  if (d.flags & ~allowed) return SB200_ERR_ARG;
+int run(sb200_ctx* ctx, int64_t n, Desc d) {
+  if (!ctx || n < 0 || (d.flags & ~OPS[d.op].flags)) return SB200_ERR_ARG;
+  d.flags |= OPS[d.op].forced;
   for (int k = 0; k < d.nin; k++)
     if (d.in_words[k] && (!d.in[k] || ((uintptr_t)d.in[k] & 15))) return SB200_ERR_ARG;
   for (int k = 0; k < d.nout; k++)
-    if (d.out[k] && ((uintptr_t)d.out[k] & 15)) return SB200_ERR_ARG;
+    if (d.out[k] ? ((uintptr_t)d.out[k] & 15) : (d.need >> k & 1)) return SB200_ERR_ARG;
+  if (!d.bitmap && (d.need >> MAX_OUT & 1)) return SB200_ERR_ARG;
   if (n == 0) return SB200_OK;
   std::lock_guard<std::mutex> lock(ctx->mu);
   ctx->set_err("");
@@ -1284,14 +1284,8 @@ int run(sb200_ctx* ctx, int64_t n, const Desc& d) {
     cudaStream_t st = ctx->user_stream;
     // the scratch buffers below are shared by all SB200_DEVICE_PTRS calls of this context: order a stream switch
     if (dc.user_ev_valid && dc.last_user_stream != st) CU(cudaStreamWaitEvent(st, dc.user_ev, 0));
-    KArgs a{};
-    a.n = n; a.flags = d.flags; a.aux = d.aux; a.combG = dc.combG; a.combGp = dc.combGp; a.bitmap = d.bitmap;
-    a.comb4G = dc.comb4; a.comb4Gp = dc.comb4 + CT_TABLE_WORDS;
-    a.ws = dc.ws[2]; a.nsm = dc.nsm; a.ec_scratch = dc.ec_scratch[2]; a.persist = ctx->persist;
-    if (d.rng) {
-      memcpy(a.rng_key, d.rng->key, sizeof(a.rng_key));
-      a.rng_word = d.rng->word_pos;
-    }
+    KArgs a = kargs(ctx, dc, 2, d, n, 0);
+    a.bitmap = d.bitmap;
     for (int k = 0; k < d.nin; k++) a.in[k] = d.in[k];
     for (int k = 0; k < d.nout; k++) a.out[k] = d.out[k];
     if (const size_t need = scratch_bytes(d, n)) {
@@ -1483,11 +1477,9 @@ int sb200_init_ex(const sb200_params* params_in, const int* devices, int n_devic
     size_t tb = (size_t)COMB_WINDOWS * COMB_ENTRIES * 24 * 4;
     if (cudaMalloc(&dc.combG, tb) != cudaSuccess || cudaMalloc(&dc.combGp, tb) != cudaSuccess) return fail(SB200_ERR_NOMEM);
     if (cudaMalloc(&dc.comb4, (size_t)2 * CT_TABLE_WORDS * 4) != cudaSuccess) return fail(SB200_ERR_NOMEM);
-    if (cudaFuncSetAttribute(k_fixed_batch<OP_SIGN_DOUBLE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * CT_TABLE_WORDS * 4) != cudaSuccess ||
-        cudaFuncSetAttribute(k_fixed_batch<OP_KEYGEN_DOUBLE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * CT_TABLE_WORDS * 4) != cudaSuccess ||
-        cudaFuncSetAttribute(k_fixed_batch<OP_SIGN, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, CT_TABLE_WORDS * 4) != cudaSuccess ||
-        cudaFuncSetAttribute(k_fixed_batch<OP_KEYGEN, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, CT_TABLE_WORDS * 4) != cudaSuccess)
-      return fail(SB200_ERR_CUDA);
+    for (const OpInfo& o : OPS)
+      if (o.ct && cudaFuncSetAttribute(o.ct, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)o.ct_smem) != cudaSuccess)
+        return fail(SB200_ERR_CUDA);
     dc.nsm = prop.multiProcessorCount;
 #if SB_VERIFY_WS
     if (cudaFuncSetAttribute(k_verify_ws, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WS_SMEM) != cudaSuccess) return fail(SB200_ERR_CUDA);
@@ -1569,176 +1561,147 @@ int sb200_host_alloc(size_t bytes, void** out) {
 void sb200_host_free(void* p) { if (p) cudaFreeHost(p); }
 
 #define IN(k, ptr, words) d.in[k] = (ptr); d.in_words[k] = (words)
-#define OUT(k, ptr, words) d.out[k] = (ptr); d.out_words[k] = (words)
+#define OPT_OUT(k, ptr, words) d.out[k] = (ptr); d.out_words[k] = (words)
+#define OUT(k, ptr, words) OPT_OUT(k, ptr, words); d.need |= 1u << (k)
+#define BITMAP(ptr) d.bitmap = (ptr); d.need |= 1u << MAX_OUT
 
 int sb200_verify(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* pk, const uint32_t* sig_u, const uint32_t* sig_R,
                  const uint32_t* msg, uint32_t* verdicts, uint32_t* c_out) {
-  if (!verdicts) return SB200_ERR_ARG;
-  Desc d; d.op = OP_VERIFY; d.flags = flags; d.nin = 4; d.nout = 1; d.bitmap = verdicts;
-  IN(0, pk, pt_words(flags)); IN(1, sig_u, 8); IN(2, sig_R, pt_words(flags)); IN(3, msg, 8); OUT(0, c_out, 8);
+  Desc d; d.op = OP_VERIFY; d.flags = flags; d.nin = 4; d.nout = 1; BITMAP(verdicts);
+  IN(0, pk, pt_words(flags)); IN(1, sig_u, 8); IN(2, sig_R, pt_words(flags)); IN(3, msg, 8); OPT_OUT(0, c_out, 8);
   return run(ctx, n, d);
 }
 int sb200_verify_double(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* pk, const uint32_t* pkp, const uint32_t* sig_u,
                         const uint32_t* sig_R, const uint32_t* sig_Rp, const uint32_t* msg, uint32_t* verdicts, uint32_t* c_out) {
-  if (!verdicts) return SB200_ERR_ARG;
-  Desc d; d.op = OP_VERIFY_DOUBLE; d.flags = flags; d.nin = 6; d.nout = 1; d.bitmap = verdicts;
+  Desc d; d.op = OP_VERIFY_DOUBLE; d.flags = flags; d.nin = 6; d.nout = 1; BITMAP(verdicts);
   int pw = pt_words(flags);
-  IN(0, pk, pw); IN(1, pkp, pw); IN(2, sig_u, 8); IN(3, sig_R, pw); IN(4, sig_Rp, pw); IN(5, msg, 8); OUT(0, c_out, 8);
+  IN(0, pk, pw); IN(1, pkp, pw); IN(2, sig_u, 8); IN(3, sig_R, pw); IN(4, sig_Rp, pw); IN(5, msg, 8); OPT_OUT(0, c_out, 8);
   return run(ctx, n, d);
 }
 int sb200_verify_vargen(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* pk, const uint32_t* gen, const uint32_t* sig_u,
                         const uint32_t* sig_R, const uint32_t* msg, uint32_t* verdicts, uint32_t* c_out) {
-  if (!verdicts) return SB200_ERR_ARG;
-  Desc d; d.op = OP_VERIFY_VARGEN; d.flags = flags; d.nin = 5; d.nout = 1; d.bitmap = verdicts;
+  Desc d; d.op = OP_VERIFY_VARGEN; d.flags = flags; d.nin = 5; d.nout = 1; BITMAP(verdicts);
   int pw = pt_words(flags);
-  IN(0, pk, pw); IN(1, gen, pw); IN(2, sig_u, 8); IN(3, sig_R, pw); IN(4, msg, 8); OUT(0, c_out, 8);
+  IN(0, pk, pw); IN(1, gen, pw); IN(2, sig_u, 8); IN(3, sig_R, pw); IN(4, msg, 8); OPT_OUT(0, c_out, 8);
   return run(ctx, n, d);
+}
+// the signers of one scheme: sk, (generator,) msg, nonce -> u, R, (R',) c; with `rng` the nonces are drawn on the device
+static int sign_call(sb200_ctx* ctx, int64_t n, uint32_t flags, int scheme, const uint32_t* sk, const uint32_t* gen, const uint32_t* msg,
+                     const uint32_t* nonce, sb200_stdrng* rng, uint32_t* u_out, uint32_t* R_out, uint32_t* Rp_out, uint32_t* c_out) {
+  static const Op ops[2][3] = {{OP_SIGN, OP_SIGN_DOUBLE, OP_SIGN_VARGEN}, {OP_SIGN_STDRNG, OP_SIGN_DOUBLE_STDRNG, OP_SIGN_VARGEN_STDRNG}};
+  const int g = scheme == 2;  // the generator comes second
+  Desc d; d.op = ops[rng != nullptr][scheme]; d.flags = flags; d.nin = 3 + g; d.nout = 4; d.rng = rng;
+  IN(0, sk, 8); IN(1, gen, g ? pt_words(flags) : 0); IN(1 + g, msg, 8); IN(2 + g, nonce, rng ? 0 : 8);
+  OUT(0, u_out, 8); OUT(1, R_out, 16); OPT_OUT(3, c_out, 8);
+  if (scheme == 1) { OUT(2, Rp_out, 16); }
+  const int rc = run(ctx, n, d);
+  if (rc == SB200_OK && rng) rng->word_pos += 16u * (uint64_t)n;  // only on success, as `&mut rng` would
+  return rc;
 }
 int sb200_sign(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* sk, const uint32_t* msg, const uint32_t* nonce,
                uint32_t* u_out, uint32_t* R_out, uint32_t* c_out) {
-  if (!u_out || !R_out) return SB200_ERR_ARG;
-  Desc d; d.op = OP_SIGN; d.flags = flags; d.nin = 3; d.nout = 4;
-  IN(0, sk, 8); IN(1, msg, 8); IN(2, nonce, 8); OUT(0, u_out, 8); OUT(1, R_out, 16); OUT(3, c_out, 8);
-  return run(ctx, n, d);
+  return sign_call(ctx, n, flags, 0, sk, nullptr, msg, nonce, nullptr, u_out, R_out, nullptr, c_out);
 }
 int sb200_sign_double(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* sk, const uint32_t* msg, const uint32_t* nonce,
                       uint32_t* u_out, uint32_t* R_out, uint32_t* Rp_out, uint32_t* c_out) {
-  if (!u_out || !R_out || !Rp_out) return SB200_ERR_ARG;
-  Desc d; d.op = OP_SIGN_DOUBLE; d.flags = flags; d.nin = 3; d.nout = 4;
-  IN(0, sk, 8); IN(1, msg, 8); IN(2, nonce, 8); OUT(0, u_out, 8); OUT(1, R_out, 16); OUT(2, Rp_out, 16); OUT(3, c_out, 8);
-  return run(ctx, n, d);
+  return sign_call(ctx, n, flags, 1, sk, nullptr, msg, nonce, nullptr, u_out, R_out, Rp_out, c_out);
 }
 int sb200_sign_vargen(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* sk, const uint32_t* gen, const uint32_t* msg,
                       const uint32_t* nonce, uint32_t* u_out, uint32_t* R_out, uint32_t* c_out) {
-  if (!u_out || !R_out) return SB200_ERR_ARG;
-  Desc d; d.op = OP_SIGN_VARGEN; d.flags = flags; d.nin = 4; d.nout = 4;
-  IN(0, sk, 8); IN(1, gen, pt_words(flags)); IN(2, msg, 8); IN(3, nonce, 8); OUT(0, u_out, 8); OUT(1, R_out, 16); OUT(3, c_out, 8);
-  return run(ctx, n, d);
+  return sign_call(ctx, n, flags, 2, sk, gen, msg, nonce, nullptr, u_out, R_out, nullptr, c_out);
+}
+int sb200_sign_stdrng(sb200_ctx* ctx, int64_t n, uint32_t flags, int scheme, const uint32_t* sk, const uint32_t* msg,
+                      const uint32_t* gen, sb200_stdrng* rng, uint32_t* u_out, uint32_t* R_out, uint32_t* Rp_out, uint32_t* c_out) {
+  if (sign_stdrng_args(n, flags, scheme, sk, msg, gen, rng, u_out, R_out, Rp_out) != SB200_OK) return SB200_ERR_ARG;
+  return sign_call(ctx, n, flags, scheme, sk, gen, msg, nullptr, rng, u_out, R_out, Rp_out, c_out);
 }
 int sb200_keygen(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* sk, uint32_t* pk_out) {
-  if (!pk_out) return SB200_ERR_ARG;
   Desc d; d.op = OP_KEYGEN; d.flags = flags; d.nin = 1; d.nout = 1;
   IN(0, sk, 8); OUT(0, pk_out, 16);
   return run(ctx, n, d);
 }
 int sb200_keygen_double(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* sk, uint32_t* pk_out, uint32_t* pkp_out) {
-  if (!pk_out || !pkp_out) return SB200_ERR_ARG;
   Desc d; d.op = OP_KEYGEN_DOUBLE; d.flags = flags; d.nin = 1; d.nout = 2;
   IN(0, sk, 8); OUT(0, pk_out, 16); OUT(1, pkp_out, 16);
   return run(ctx, n, d);
 }
 int sb200_keygen_vargen(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* sk, const uint32_t* gen, uint32_t* pk_out) {
-  if (!pk_out) return SB200_ERR_ARG;
   Desc d; d.op = OP_KEYGEN_VARGEN; d.flags = flags; d.nin = 2; d.nout = 1;
   IN(0, sk, 8); IN(1, gen, pt_words(flags)); OUT(0, pk_out, 16);
   return run(ctx, n, d);
 }
 int sb200_points_decompress(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint8_t* bytes, uint32_t* points_out, uint32_t* ok_bitmap) {
-  if (!points_out || !ok_bitmap || (flags & SB200_POINTS_AFFINE)) return SB200_ERR_ARG;
-  Desc d; d.op = OP_DECOMPRESS; d.flags = flags; d.nin = 1; d.nout = 1; d.bitmap = ok_bitmap;
+  Desc d; d.op = OP_DECOMPRESS; d.flags = flags; d.nin = 1; d.nout = 1; BITMAP(ok_bitmap);
   IN(0, (const uint32_t*)bytes, 8); OUT(0, points_out, 16);
   return run(ctx, n, d);
 }
 int sb200_points_compress(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* points, uint8_t* bytes_out) {
-  if (!bytes_out) return SB200_ERR_ARG;
   Desc d; d.op = OP_COMPRESS; d.flags = flags; d.nin = 1; d.nout = 1;
   IN(0, points, pt_words(flags)); OUT(0, (uint32_t*)bytes_out, 8);
   return run(ctx, n, d);
 }
 int sb200_scalars_from_wide(sb200_ctx* ctx, int64_t n, uint32_t flags, int field, const uint8_t* wide, uint32_t* out) {
-  if (!out || field < 0 || field > 1 || (flags & SB200_POINTS_AFFINE)) return SB200_ERR_ARG;
+  if (field < 0 || field > 1) return SB200_ERR_ARG;
   Desc d; d.op = OP_FROM_WIDE; d.flags = flags; d.aux = field; d.nin = 1; d.nout = 1;
   IN(0, (const uint32_t*)wide, 16); OUT(0, out, 8);
   return run(ctx, n, d);
 }
-// the position advances only when the call succeeds (as `&mut rng` would)
 int sb200_stdrng_random(sb200_ctx* ctx, int64_t n, uint32_t flags, int field, sb200_stdrng* rng, uint32_t* out) {
   if (stdrng_random_args(n, flags, field, rng, out) != SB200_OK) return SB200_ERR_ARG;
   Desc d; d.op = OP_STDRNG; d.flags = flags; d.aux = field; d.nin = 0; d.nout = 1; d.rng = rng;
   OUT(0, out, 8);
   const int rc = run(ctx, n, d);
-  if (rc == SB200_OK) rng->word_pos += 16u * (uint64_t)n;
+  if (rc == SB200_OK) rng->word_pos += 16u * (uint64_t)n;  // only on success, as `&mut rng` would
   return rc;
 }
-int sb200_sign_stdrng(sb200_ctx* ctx, int64_t n, uint32_t flags, int scheme, const uint32_t* sk, const uint32_t* msg,
-                      const uint32_t* gen, sb200_stdrng* rng, uint32_t* u_out, uint32_t* R_out, uint32_t* Rp_out, uint32_t* c_out) {
-  if (sign_stdrng_args(n, flags, scheme, sk, msg, gen, rng, u_out, R_out, Rp_out) != SB200_OK) return SB200_ERR_ARG;
-  static const Op ops[3] = {OP_SIGN_STDRNG, OP_SIGN_DOUBLE_STDRNG, OP_SIGN_VARGEN_STDRNG};
-  Desc d; d.op = ops[scheme]; d.flags = flags; d.nout = 4; d.rng = rng;
-  IN(0, sk, 8);
-  if (scheme == 2) {  // the inputs of sb200_sign_vargen (sk, gen, msg, nonce) without the nonce
-    d.nin = 4;
-    IN(1, gen, pt_words(flags)); IN(2, msg, 8); IN(3, nullptr, 0);
-  } else {  // those of sb200_sign / _double (sk, msg, nonce)
-    d.nin = 3;
-    IN(1, msg, 8); IN(2, nullptr, 0);
-  }
-  OUT(0, u_out, 8); OUT(1, R_out, 16); OUT(2, scheme == 1 ? Rp_out : nullptr, 16); OUT(3, c_out, 8);
-  const int rc = run(ctx, n, d);
-  if (rc == SB200_OK) rng->word_pos += 16u * (uint64_t)n;
-  return rc;
-}
-int sb200_fq_to_mont(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* in, uint32_t* out) {
-  if (!out || (flags & SB200_POINTS_AFFINE)) return SB200_ERR_ARG;
-  Desc d; d.op = OP_DBG_FQ; d.flags = flags; d.aux = 5; d.nin = 2; d.nout = 1;
+static int fq_mont(sb200_ctx* ctx, int64_t n, uint32_t flags, int aux, const uint32_t* in, uint32_t* out) {
+  Desc d; d.op = OP_DBG_FQ; d.flags = flags; d.aux = aux; d.nin = 2; d.nout = 1;
   IN(0, in, 8); IN(1, nullptr, 0); OUT(0, out, 8);
   return run(ctx, n, d);
 }
-int sb200_fq_from_mont(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* in, uint32_t* out) {
-  if (!out || (flags & SB200_POINTS_AFFINE)) return SB200_ERR_ARG;
-  Desc d; d.op = OP_DBG_FQ; d.flags = flags; d.aux = 6; d.nin = 2; d.nout = 1;
-  IN(0, in, 8); IN(1, nullptr, 0); OUT(0, out, 8);
+int sb200_fq_to_mont(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* in, uint32_t* out) { return fq_mont(ctx, n, flags, 5, in, out); }
+int sb200_fq_from_mont(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* in, uint32_t* out) { return fq_mont(ctx, n, flags, 6, in, out); }
+// the byte-level calls of one scheme: pk_words / sk_words, sig_words and 8 words (msg, nonce) per tuple
+static int verify_bytes_call(sb200_ctx* ctx, int64_t n, uint32_t flags, Op op, int pk_words, int sig_words, const uint8_t* pk,
+                             const uint8_t* sig, const uint8_t* msg, uint32_t* verdicts, uint32_t* invalid) {
+  Desc d; d.op = op; d.flags = flags; d.nin = 3; d.nout = 1; BITMAP(verdicts);
+  IN(0, (const uint32_t*)pk, pk_words); IN(1, (const uint32_t*)sig, sig_words); IN(2, (const uint32_t*)msg, 8);
+  OPT_OUT(0, invalid, -1);  // bitmap-shaped output: one word per 32 tuples
+  return run(ctx, n, d);
+}
+static int sign_bytes_call(sb200_ctx* ctx, int64_t n, uint32_t flags, Op op, int sk_words, int sig_words, const uint8_t* sk,
+                           const uint8_t* msg, const uint8_t* nonce, uint8_t* sig_out, uint32_t* invalid) {
+  Desc d; d.op = op; d.flags = flags; d.nin = 3; d.nout = 1; d.bitmap = invalid;
+  IN(0, (const uint32_t*)sk, sk_words); IN(1, (const uint32_t*)msg, 8); IN(2, (const uint32_t*)nonce, 8); OUT(0, (uint32_t*)sig_out, sig_words);
   return run(ctx, n, d);
 }
 int sb200_verify_bytes(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint8_t* pk, const uint8_t* sig, const uint8_t* msg,
                        uint32_t* verdicts, uint32_t* invalid) {
-  if (!verdicts || (flags & SB200_POINTS_AFFINE)) return SB200_ERR_ARG;
-  Desc d; d.op = OP_VERIFY_BYTES; d.flags = flags | SB200_POINTS_AFFINE; d.nin = 3; d.nout = 1; d.bitmap = verdicts;
-  IN(0, (const uint32_t*)pk, 8); IN(1, (const uint32_t*)sig, 16); IN(2, (const uint32_t*)msg, 8);
-  d.out[0] = invalid; d.out_words[0] = -1;  // bitmap-shaped output: one word per 32 tuples
-  return run(ctx, n, d);
+  return verify_bytes_call(ctx, n, flags, OP_VERIFY_BYTES, 8, 16, pk, sig, msg, verdicts, invalid);
 }
 int sb200_sign_bytes(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint8_t* sk, const uint8_t* msg, const uint8_t* nonce,
                      uint8_t* sig_out, uint32_t* invalid) {
-  if (!sig_out || (flags & SB200_POINTS_AFFINE)) return SB200_ERR_ARG;
-  Desc d; d.op = OP_SIGN_BYTES; d.flags = flags; d.nin = 3; d.nout = 1; d.bitmap = invalid;
-  IN(0, (const uint32_t*)sk, 8); IN(1, (const uint32_t*)msg, 8); IN(2, (const uint32_t*)nonce, 8); OUT(0, (uint32_t*)sig_out, 16);
-  return run(ctx, n, d);
+  return sign_bytes_call(ctx, n, flags, OP_SIGN_BYTES, 8, 16, sk, msg, nonce, sig_out, invalid);
 }
 int sb200_verify_double_bytes(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint8_t* pk, const uint8_t* sig, const uint8_t* msg,
                               uint32_t* verdicts, uint32_t* invalid) {
-  if (!verdicts || (flags & SB200_POINTS_AFFINE)) return SB200_ERR_ARG;
-  Desc d; d.op = OP_VERIFY_DOUBLE_BYTES; d.flags = flags | SB200_POINTS_AFFINE; d.nin = 3; d.nout = 1; d.bitmap = verdicts;
-  IN(0, (const uint32_t*)pk, 16); IN(1, (const uint32_t*)sig, 24); IN(2, (const uint32_t*)msg, 8);
-  d.out[0] = invalid; d.out_words[0] = -1;
-  return run(ctx, n, d);
+  return verify_bytes_call(ctx, n, flags, OP_VERIFY_DOUBLE_BYTES, 16, 24, pk, sig, msg, verdicts, invalid);
 }
 int sb200_verify_vargen_bytes(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint8_t* pk, const uint8_t* sig, const uint8_t* msg,
                               uint32_t* verdicts, uint32_t* invalid) {
-  if (!verdicts || (flags & SB200_POINTS_AFFINE)) return SB200_ERR_ARG;
-  Desc d; d.op = OP_VERIFY_VARGEN_BYTES; d.flags = flags | SB200_POINTS_AFFINE; d.nin = 3; d.nout = 1; d.bitmap = verdicts;
-  IN(0, (const uint32_t*)pk, 16); IN(1, (const uint32_t*)sig, 16); IN(2, (const uint32_t*)msg, 8);
-  d.out[0] = invalid; d.out_words[0] = -1;
-  return run(ctx, n, d);
+  return verify_bytes_call(ctx, n, flags, OP_VERIFY_VARGEN_BYTES, 16, 16, pk, sig, msg, verdicts, invalid);
 }
 int sb200_sign_double_bytes(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint8_t* sk, const uint8_t* msg, const uint8_t* nonce,
                             uint8_t* sig_out, uint32_t* invalid) {
-  if (!sig_out || (flags & SB200_POINTS_AFFINE)) return SB200_ERR_ARG;
-  Desc d; d.op = OP_SIGN_DOUBLE_BYTES; d.flags = flags; d.nin = 3; d.nout = 1; d.bitmap = invalid;
-  IN(0, (const uint32_t*)sk, 8); IN(1, (const uint32_t*)msg, 8); IN(2, (const uint32_t*)nonce, 8); OUT(0, (uint32_t*)sig_out, 24);
-  return run(ctx, n, d);
+  return sign_bytes_call(ctx, n, flags, OP_SIGN_DOUBLE_BYTES, 8, 24, sk, msg, nonce, sig_out, invalid);
 }
 int sb200_sign_vargen_bytes(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint8_t* sk, const uint8_t* msg, const uint8_t* nonce,
                             uint8_t* sig_out, uint32_t* invalid) {
-  if (!sig_out || (flags & SB200_POINTS_AFFINE)) return SB200_ERR_ARG;
-  Desc d; d.op = OP_SIGN_VARGEN_BYTES; d.flags = flags | SB200_POINTS_AFFINE; d.nin = 3; d.nout = 1; d.bitmap = invalid;
-  IN(0, (const uint32_t*)sk, 16); IN(1, (const uint32_t*)msg, 8); IN(2, (const uint32_t*)nonce, 8); OUT(0, (uint32_t*)sig_out, 16);
-  return run(ctx, n, d);
+  return sign_bytes_call(ctx, n, flags, OP_SIGN_VARGEN_BYTES, 16, 16, sk, msg, nonce, sig_out, invalid);
 }
 int sb200_sign_witness(sb200_ctx* ctx, int64_t n, uint32_t flags, int scheme, const uint32_t* sk, const uint32_t* msg,
                        const uint32_t* nonce, const uint32_t* generator, uint32_t* rows_out) {
-  if (!rows_out || scheme < 0 || scheme > 2 || (scheme == 2 && !generator)) return SB200_ERR_ARG;
-  if (scheme != 2 && (flags & SB200_POINTS_AFFINE)) return SB200_ERR_ARG;
+  if (scheme < 0 || scheme > 2 || (scheme == 2 && !generator) || (scheme != 2 && (flags & SB200_POINTS_AFFINE))) return SB200_ERR_ARG;
   static const int width[3] = {11, 19, 13};
   Desc d; d.op = OP_WITNESS; d.flags = flags; d.aux = scheme; d.nin = 4; d.nout = 1;
   IN(0, sk, 8); IN(1, msg, 8); IN(2, nonce, 8); IN(3, scheme == 2 ? generator : nullptr, scheme == 2 ? pt_words(flags) : 0);
@@ -1746,44 +1709,40 @@ int sb200_sign_witness(sb200_ctx* ctx, int64_t n, uint32_t flags, int scheme, co
   return run(ctx, n, d);
 }
 int sb200_points_check(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* points, uint32_t* ok_bitmap) {
-  if (!ok_bitmap) return SB200_ERR_ARG;
-  Desc d; d.op = OP_POINTS_CHECK; d.flags = flags; d.nin = 1; d.nout = 0; d.bitmap = ok_bitmap;
+  Desc d; d.op = OP_POINTS_CHECK; d.flags = flags; d.nin = 1; d.nout = 0; BITMAP(ok_bitmap);
   IN(0, points, pt_words(flags));
   return run(ctx, n, d);
 }
 int sb200_dbg_verify_ec(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* pk, const uint32_t* sig_u, const uint32_t* sig_R,
                         const uint32_t* c, uint32_t* verdicts) {
-  if (!verdicts) return SB200_ERR_ARG;
-  Desc d; d.op = OP_DBG_VERIFY_EC; d.flags = flags; d.nin = 4; d.nout = 0; d.bitmap = verdicts;
+  Desc d; d.op = OP_DBG_VERIFY_EC; d.flags = flags; d.nin = 4; d.nout = 0; BITMAP(verdicts);
   IN(0, pk, pt_words(flags)); IN(1, sig_u, 8); IN(2, sig_R, pt_words(flags)); IN(3, c, 8);
   return run(ctx, n, d);
 }
 int sb200_dbg_fq(sb200_ctx* ctx, int64_t n, int op, const uint32_t* a, const uint32_t* b, uint32_t* out) {
-  if (!out || op < 0 || op > 7) return SB200_ERR_ARG;
+  if (op < 0 || op > 7) return SB200_ERR_ARG;
   Desc d; d.op = OP_DBG_FQ; d.flags = 0; d.aux = op; d.nin = 2; d.nout = 1;
   IN(0, a, 8); IN(1, b, b ? 8 : 0); OUT(0, out, 8);
   return run(ctx, n, d);
 }
 int sb200_dbg_lattice3(sb200_ctx* ctx, int64_t n, const uint32_t* c, const uint32_t* u, uint32_t* out) {
-  if (!out) return SB200_ERR_ARG;
   Desc d; d.op = OP_DBG_LAT3; d.flags = 0; d.nin = 2; d.nout = 1;
   IN(0, c, 8); IN(1, u, 8); OUT(0, out, 32);
   return run(ctx, n, d);
 }
 int sb200_dbg_fr_mul(sb200_ctx* ctx, int64_t n, const uint32_t* a, const uint32_t* b, uint32_t* out) {
-  if (!out) return SB200_ERR_ARG;
   Desc d; d.op = OP_DBG_FR_MUL; d.flags = 0; d.nin = 2; d.nout = 1;
   IN(0, a, 8); IN(1, b, 8); OUT(0, out, 8);
   return run(ctx, n, d);
 }
 int sb200_dbg_hades(sb200_ctx* ctx, int64_t n, int dense, uint32_t* states) {
-  if (!states || dense < 0 || dense > (SB_EXPERIMENTAL_FD ? 2 : 1)) return SB200_ERR_ARG;
+  if (dense < 0 || dense > (SB_EXPERIMENTAL_FD ? 2 : 1)) return SB200_ERR_ARG;
   Desc d; d.op = OP_DBG_HADES; d.flags = 0; d.aux = dense; d.nin = 1; d.nout = 1;
   IN(0, states, 40); OUT(0, states, 40);
   return run(ctx, n, d);
 }
 int sb200_dbg_scalar_mul(sb200_ctx* ctx, int64_t n, uint32_t flags, int base, const uint32_t* points, const uint32_t* k, uint32_t* out) {
-  if (!out || base < 0 || base > 2 || (base == 2 && !points)) return SB200_ERR_ARG;
+  if (base < 0 || base > 2 || (base == 2 && !points)) return SB200_ERR_ARG;
   Desc d; d.op = OP_DBG_SMUL; d.flags = flags; d.aux = base; d.nin = 2; d.nout = 1;
   IN(0, points, base == 2 ? pt_words(flags) : 0); IN(1, k, 8); OUT(0, out, 16);
   return run(ctx, n, d);
