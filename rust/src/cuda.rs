@@ -170,6 +170,13 @@ extern "C" {
                                nonce32: *const u8, sig96_out: *mut u8, invalid: *mut u32) -> c_int;
     fn sb200_sign_vargen_bytes(ctx: *mut Sb200Ctx, n: i64, flags: u32, sk64: *const u8, msg32: *const u8,
                                nonce32: *const u8, sig64_out: *mut u8, invalid: *mut u32) -> c_int;
+    // include/schnorr_b200_witness.h: witness rows of received signatures (pk2 = PK' | generator, sig_R_prime: double only)
+    fn sb200_verify_witness(ctx: *mut Sb200Ctx, n: i64, flags: u32, scheme: c_int, pk: *const u32, pk2: *const u32,
+                            sig_u: *const u32, sig_R: *const u32, sig_R_prime: *const u32, msg: *const u32,
+                            verdicts: *mut u32, rows_out: *mut u32) -> c_int;
+    fn sb200_verify_witness_bytes(ctx: *mut Sb200Ctx, n: i64, flags: u32, scheme: c_int, pk_bytes: *const u8,
+                                  sig_bytes: *const u8, msg32: *const u8, verdicts: *mut u32, rows_out: *mut u32,
+                                  invalid: *mut u32) -> c_int;
 }
 
 /// Owns one `sb200_ctx` (comb tables of G and G' resident on each listed device).  There is no CPU
@@ -304,6 +311,13 @@ fn scalar_at(a: &Vec32, i: usize) -> JubJubScalar {
 fn bits(words: &Vec32, n: usize) -> Vec<bool> {
     (0..n).map(|i| (words[i >> 5] >> (i & 31)) & 1 == 1).collect()
 }
+fn witness_rows<const W: usize>(rows: &Vec32, n: usize) -> Vec<[BlsScalar; W]> {
+    (0..n).map(|i| {
+        let mut w = [BlsScalar::zero(); W];
+        for (k, x) in w.iter_mut().enumerate() { *x = fq_at(rows, W * i + k); }
+        w
+    }).collect()
+}
 
 impl PublicKey {
     /// `out[i] == pks[i].verify(&sigs[i], msgs[i])` (src/keys/public.rs:121-130) for every i.
@@ -323,6 +337,30 @@ impl PublicKey {
                          words.as_mut_ptr(), core::ptr::null_mut())
         })?;
         Ok(bits(&words, n))
+    }
+
+    /// Verifier-side counterpart of `SecretKey::sign_batch_witness`: for signatures the caller received rather than made,
+    /// `verify_batch`'s verdicts together with the rows `u, R.u, R.v, PK.u, PK.v, m, c, SA.u, SA.v, SB.u, SB.v` that
+    /// `Signature::append` and `gadgets::verify_signature` allocate, SA = u G and SB = c PK computed on the device
+    /// (`sb200_verify_witness`).  A signature that fails keeps its true row; the row of a signature made by
+    /// `sign_batch_witness` equals the signer's.
+    pub fn verify_batch_witness(ctx: &CudaCtx, pks: &[PublicKey], sigs: &[Signature], msgs: &[BlsScalar])
+                                -> Result<(Vec<bool>, Vec<[BlsScalar; 11]>), CudaError> {
+        let n = pks.len();
+        assert!(sigs.len() == n && msgs.len() == n);
+        let (mut pk, mut u, mut r, mut m) = (Vec32::with_capacity(24 * n), Vec32::with_capacity(8 * n), Vec32::with_capacity(24 * n), Vec32::with_capacity(8 * n));
+        for i in 0..n {
+            push_point(&mut pk, pks[i].as_ref());
+            push_scalar(&mut u, sigs[i].u());
+            push_point(&mut r, sigs[i].R());
+            push_fq(&mut m, &msgs[i]);
+        }
+        let (mut words, mut rows) = (Vec32::zeroed((n + 31) / 32), Vec32::zeroed(8 * 11 * n));
+        ctx.check(unsafe {
+            sb200_verify_witness(ctx.raw, n as i64, SB200_POINTS_PROJECTIVE, 0, pk.as_ptr(), core::ptr::null(), u.as_ptr(),
+                                 r.as_ptr(), core::ptr::null(), m.as_ptr(), words.as_mut_ptr(), rows.as_mut_ptr())
+        })?;
+        Ok((bits(&words, n), witness_rows::<11>(&rows, n)))
     }
 
     /// Byte-level form: `PublicKey::from_bytes(pk)?.verify(&Signature::from_bytes(sig)?, BlsScalar::from_bytes(msg)?)`;
@@ -471,6 +509,30 @@ impl PublicKeyDouble {
         })?;
         Ok(bits(&words, n))
     }
+
+    /// `verify_batch` with the witness rows of each signature (`sb200_verify_witness`, scheme 1):
+    /// `u, R, R', PK, PK', m, c, SA, SB, SA', SB'` (points as (u, v); SA' = u G', SB' = c PK').
+    pub fn verify_batch_witness(ctx: &CudaCtx, pks: &[PublicKeyDouble], sigs: &[SignatureDouble], msgs: &[BlsScalar])
+                                -> Result<(Vec<bool>, Vec<[BlsScalar; 19]>), CudaError> {
+        let n = pks.len();
+        assert!(sigs.len() == n && msgs.len() == n);
+        let (mut pk, mut pkp, mut u, mut r, mut rp, mut m) = (Vec32::with_capacity(24 * n), Vec32::with_capacity(24 * n), Vec32::with_capacity(8 * n),
+                                                              Vec32::with_capacity(24 * n), Vec32::with_capacity(24 * n), Vec32::with_capacity(8 * n));
+        for i in 0..n {
+            push_point(&mut pk, pks[i].pk());
+            push_point(&mut pkp, pks[i].pk_prime());
+            push_scalar(&mut u, sigs[i].u());
+            push_point(&mut r, sigs[i].R());
+            push_point(&mut rp, sigs[i].R_prime());
+            push_fq(&mut m, &msgs[i]);
+        }
+        let (mut words, mut rows) = (Vec32::zeroed((n + 31) / 32), Vec32::zeroed(8 * 19 * n));
+        ctx.check(unsafe {
+            sb200_verify_witness(ctx.raw, n as i64, SB200_POINTS_PROJECTIVE, 1, pk.as_ptr(), pkp.as_ptr(), u.as_ptr(),
+                                 r.as_ptr(), rp.as_ptr(), m.as_ptr(), words.as_mut_ptr(), rows.as_mut_ptr())
+        })?;
+        Ok((bits(&words, n), witness_rows::<19>(&rows, n)))
+    }
 }
 
 #[cfg(feature = "var_generator")]
@@ -493,6 +555,29 @@ impl PublicKeyVarGen {
                                 r.as_ptr(), m.as_ptr(), words.as_mut_ptr(), core::ptr::null_mut())
         })?;
         Ok(bits(&words, n))
+    }
+
+    /// `verify_batch` with the witness rows of each signature (`sb200_verify_witness`, scheme 2):
+    /// `u, R, PK, GEN, m, c, SA, SB` (points as (u, v); SA = u GEN).
+    pub fn verify_batch_witness(ctx: &CudaCtx, pks: &[PublicKeyVarGen], sigs: &[SignatureVarGen], msgs: &[BlsScalar])
+                                -> Result<(Vec<bool>, Vec<[BlsScalar; 13]>), CudaError> {
+        let n = pks.len();
+        assert!(sigs.len() == n && msgs.len() == n);
+        let (mut pk, mut g, mut u, mut r, mut m) = (Vec32::with_capacity(24 * n), Vec32::with_capacity(24 * n), Vec32::with_capacity(8 * n),
+                                                    Vec32::with_capacity(24 * n), Vec32::with_capacity(8 * n));
+        for i in 0..n {
+            push_point(&mut pk, pks[i].public_key());
+            push_point(&mut g, pks[i].generator());
+            push_scalar(&mut u, sigs[i].u());
+            push_point(&mut r, sigs[i].R());
+            push_fq(&mut m, &msgs[i]);
+        }
+        let (mut words, mut rows) = (Vec32::zeroed((n + 31) / 32), Vec32::zeroed(8 * 13 * n));
+        ctx.check(unsafe {
+            sb200_verify_witness(ctx.raw, n as i64, SB200_POINTS_PROJECTIVE, 2, pk.as_ptr(), g.as_ptr(), u.as_ptr(),
+                                 r.as_ptr(), core::ptr::null(), m.as_ptr(), words.as_mut_ptr(), rows.as_mut_ptr())
+        })?;
+        Ok((bits(&words, n), witness_rows::<13>(&rows, n)))
     }
 }
 

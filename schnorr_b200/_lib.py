@@ -122,8 +122,12 @@ _PROTOTYPES = {  # every symbol of include/schnorr_b200.h: (restype, argtypes)
     "sb200_dbg_hades": (ci, [vp, i64, ci, u32p]),
     "sb200_dbg_scalar_mul": (ci, [vp, i64, u32, ci] + [u32p] * 3),
 }
+_WITNESS_PROTOTYPES = {  # every symbol of include/schnorr_b200_witness.h (verifier-side witness rows)
+    "sb200_verify_witness": (ci, [vp, i64, u32, ci] + [u32p] * 8),
+    "sb200_verify_witness_bytes": (ci, [vp, i64, u32, ci] + [u32p] * 6),
+}
 del vp, u32p, i64, u32, ci
-EXPORTED_SYMBOLS = list(_PROTOTYPES)
+EXPORTED_SYMBOLS = list(_PROTOTYPES)  # the symbols of include/schnorr_b200.h
 
 _lib = None
 
@@ -142,7 +146,7 @@ def load_library() -> ctypes.CDLL:
             f"{LIB_PATH} not found: build it with `python -c 'import __graft_entry__ as g; g.build()'` "
             "(nvcc, sm_100a). There is no CPU fallback.")
     lib = ctypes.CDLL(LIB_PATH)
-    for name, (res, args) in _PROTOTYPES.items():
+    for name, (res, args) in {**_PROTOTYPES, **_WITNESS_PROTOTYPES}.items():
         fn = getattr(lib, name)  # AttributeError if the library does not export a declared symbol
         fn.restype, fn.argtypes = res, args
     _lib = lib
@@ -475,6 +479,37 @@ class Engine:
                                           g.ctypes.data if g is not None else None, out.ctypes.data)
         self._check(rc, "sign_witness")
         return out
+
+    def verify_witness(self, scheme: int, pk, u, R, msg, pk2=None, Rp=None, affine=True, check_points=False):
+        """witness rows of received signatures (include/schnorr_b200_witness.h): (ok[n], rows[n, W, 8]) with the row
+        layout of sign_witness.  pk2 = PK' (scheme 1) or the generator (scheme 2); Rp = R' (scheme 1)."""
+        n = np.asarray(u).size // 8
+        pw = self._pw(affine)
+        fl = (POINTS_AFFINE if affine else POINTS_PROJECTIVE) | (CHECK_POINTS if check_points else 0)
+        pk, u, R, msg = _arr(pk, pw, n, "pk"), _arr(u, 8, n, "u"), _arr(R, pw, n, "R"), _arr(msg, 8, n, "msg")
+        pk2 = _arr(pk2, pw, n, "pk2") if scheme in (1, 2) else None
+        Rp = _arr(Rp, pw, n, "R'") if scheme == 1 else None
+        bm = aligned_empty(((n + 31) // 32,)); bm[...] = 0
+        rows = aligned_empty((n, self.WITNESS_WIDTH[scheme], 8))
+        rc = self._lib.sb200_verify_witness(self._h, n, fl, scheme, pk.ctypes.data, pk2.ctypes.data if pk2 is not None else None,
+                                            u.ctypes.data, R.ctypes.data, Rp.ctypes.data if Rp is not None else None,
+                                            msg.ctypes.data, bm.ctypes.data, rows.ctypes.data)
+        self._check(rc, "verify_witness")
+        return self._unpack_bits(bm, n), rows
+
+    def verify_witness_bytes(self, scheme: int, pk, sig, msg):
+        """the byte-level inputs of verify_bytes / verify_double_bytes / verify_vargen_bytes -> (ok[n], invalid[n],
+        rows[n, W, 8]); a tuple that does not decode has invalid set, verdict 0 and an all-zero row"""
+        pk = self._bytes_arr(pk, (32, 64, 64)[scheme], "pk")
+        sig, msg = self._bytes_arr(sig, (64, 96, 64)[scheme], "sig"), self._bytes_arr(msg, 32, "msg")
+        n = pk.shape[0]
+        bm = aligned_empty(((n + 31) // 32,)); bm[...] = 0
+        inv = aligned_empty(((n + 31) // 32,)); inv[...] = 0
+        rows = aligned_empty((n, self.WITNESS_WIDTH[scheme], 8))
+        rc = self._lib.sb200_verify_witness_bytes(self._h, n, 0, scheme, pk.ctypes.data, sig.ctypes.data, msg.ctypes.data,
+                                                  bm.ctypes.data, rows.ctypes.data, inv.ctypes.data)
+        self._check(rc, "verify_witness_bytes")
+        return self._unpack_bits(bm, n), self._unpack_bits(inv, n), rows
 
     def points_check(self, points, affine=True):
         """ok[n]: point i is on the curve with Z != 0 (what CHECK_POINTS applies inside the verify calls)"""

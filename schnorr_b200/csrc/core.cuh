@@ -561,4 +561,87 @@ SB_HD void witness_core(const uint32_t* sk, const uint32_t* nonce, const fq& m, 
   }
 }
 
+// The same rows for a party that did not sign: from the public tuple (PK, u, R, m) alone.  PK2 = PK' (SCHEME 1) or GEN
+// (SCHEME 2), Rp = R' (SCHEME 1); unused arguments are not read.  SA = u B and SB = c PK are both computed as scalar
+// multiples (never SB = R - SA: R is only claimed here), and the return value is the verdict SA + SB == R (and
+// SA' + SB' == R'), the same predicate sb200_verify* decides.  A tuple that fails keeps its true row; the row is zero
+// (and the verdict 0) when u >= r or, with `check_points`, when an input point is not well formed.  Only public data
+// enters, so both inversions are the Euclidean one.  Emits like witness_core; the zeroing masks the stores, the work
+// runs for every lane.
+template <int SCHEME, class Emit>
+SB_HD bool verify_witness_core(const point_in& PK, const point_in& PK2, const uint32_t* u_in, const point_in& R,
+                               const point_in& Rp, const fq& m, bool check_points, const uint32_t* combG,
+                               const uint32_t* combGp, Emit&& emit) {
+  constexpr int NB = SCHEME == 1 ? 2 : 1;                      // bases
+  constexpr int NP = SCHEME == 0 ? 2 : SCHEME == 1 ? 4 : 3;    // input points, in row order: R (, R'), PK (, PK' | GEN)
+  const point_in* P[4] = {&R, SCHEME == 1 ? &Rp : &PK, SCHEME == 1 ? &PK : &PK2, &PK2};
+  const bool lt = scalar_lt_r(u_in);
+  bool live = lt;
+  if (check_points) {  // warp-uniform
+#pragma unroll
+    for (int k = 0; k < NP; k++) live &= point_well_formed(*P[k]);
+  }
+  auto put = [&](int k, const fq& v) { emit(k, live ? v : fq_zero()); };
+  uint32_t u[8], c[8];
+#pragma unroll
+  for (int i = 0; i < 8; i++) u[i] = lt ? u_in[i] : 0u;  // in range for the comb; the row is zero anyway
+  put(0, scalar_to_bls(u));
+  // 1. the inputs in affine form: one inversion for all of them when they are projective (one flag for every point)
+  fq au[NP], av[NP];
+  if (R.affine) {
+#pragma unroll
+    for (int k = 0; k < NP; k++) {
+      au[k] = P[k]->U;
+      av[k] = P[k]->V;
+    }
+  } else {
+    fq z[NP], pre[NP];
+#pragma unroll
+    for (int k = 0; k < NP; k++) z[k] = P[k]->Z;
+    batch_inverse(z, pre, NP);
+#pragma unroll
+    for (int k = 0; k < NP; k++) {
+      au[k] = fq_mul(P[k]->U, z[k]);
+      av[k] = fq_mul(P[k]->V, z[k]);
+    }
+  }
+  int o = 1;
+#pragma unroll
+  for (int k = 0; k < NP; k++) {
+    put(o++, au[k]);
+    put(o++, av[k]);
+  }
+  // 2. the challenge
+  if (SCHEME == 1) chal5(au[0], av[0], au[1], av[1], m, c); else chal3(au[0], av[0], m, c);
+  put(o++, m);
+  put(o++, scalar_to_bls(c));
+  // 3. SA = u B (comb for G and G', window table for a variable generator), SB = c PK; 5. verdict SA + SB == R
+  ext S[2 * NB];
+  bool ok = live;
+#pragma unroll
+  for (int b = 0; b < NB; b++) {
+    const point_in key = {au[NB + b], av[NB + b], fq_one(), true};
+    if (SCHEME == 2) {
+      const point_in gen = {au[2], av[2], fq_one(), true};
+      S[2 * b] = var_base_mul(gen, u);
+    } else {
+      S[2 * b] = fixed_base_mul(b ? combGp : combG, u);
+    }
+    S[2 * b + 1] = var_base_mul(key, c);
+    const point_in rr = {au[b], av[b], fq_one(), true};
+    ok &= p1p1_equals(ed_add(S[2 * b], ext_to_pniels(S[2 * b + 1])), rr);
+  }
+  // 4. the outputs in affine form: one inversion
+  fq z[2 * NB], pre[2 * NB];
+#pragma unroll
+  for (int k = 0; k < 2 * NB; k++) z[k] = S[k].Z;
+  batch_inverse(z, pre, 2 * NB);
+#pragma unroll
+  for (int k = 0; k < 2 * NB; k++) {
+    put(o++, fq_mul(S[k].X, z[k]));
+    put(o++, fq_mul(S[k].Y, z[k]));
+  }
+  return ok;
+}
+
 }  // namespace sb200

@@ -20,6 +20,7 @@
 #include <thread>
 
 #include "../../include/schnorr_b200.h"
+#include "../../include/schnorr_b200_witness.h"
 #include "wire.cuh"
 #include "rng.cuh"
 #include "params_host.cuh"
@@ -49,10 +50,11 @@ constexpr int TPB = 128;
 #endif
 // CTAs per SM the register allocator must allow: 4 (128 registers/thread) everywhere except the two kernels that
 // keep a second point table live, which measure faster at 3 (168 registers, fewer spills).  [A/B timed on B200]
+// The verifier-side witness kernel (op 37, OP_VERIFY_WITNESS) spills 3.9 KB per thread at 128 registers: also 3.
 #ifndef SB_VERIFY_CTAS
 #define SB_VERIFY_CTAS SB_MIN_CTAS
 #endif
-constexpr int min_ctas(int op) { return (op == 0 || op == 19) ? SB_VERIFY_CTAS : (op == 25 || op == 27) ? SB_MIN_CTAS - 1 : (op == 1 || op == 2) ? SB_MIN_CTAS - 1 : SB_MIN_CTAS; }
+constexpr int min_ctas(int op) { return (op == 0 || op == 19) ? SB_VERIFY_CTAS : (op == 25 || op == 27 || op == 37) ? SB_MIN_CTAS - 1 : (op == 1 || op == 2) ? SB_MIN_CTAS - 1 : SB_MIN_CTAS; }
 constexpr int MAX_IN = 6, MAX_OUT = 4;
 constexpr int64_t CHUNK = 1 << 18;      // tuples per pipeline stage ...
 constexpr int64_t CHUNK_MIN = 1 << 14;  // ... shrunk towards this when a device's share is under 4 chunks, so that H2D still overlaps compute
@@ -64,8 +66,10 @@ enum Op : int {
   OP_VERIFY_DOUBLE_BYTES, OP_VERIFY_VARGEN_BYTES, OP_SIGN_DOUBLE_BYTES, OP_SIGN_VARGEN_BYTES,
   OP_CHALLENGE_DOUBLE, OP_VERIFY_DOUBLE_EC, OP_CHALLENGE_VARGEN, OP_VERIFY_VARGEN_EC, OP_POINTS_CHECK, OP_DBG_VERIFY_EC,
   OP_DECODE_VERIFY, OP_WITNESS, OP_DBG_LAT3,
-  OP_STDRNG, OP_SIGN_STDRNG, OP_SIGN_DOUBLE_STDRNG, OP_SIGN_VARGEN_STDRNG
+  OP_STDRNG, OP_SIGN_STDRNG, OP_SIGN_DOUBLE_STDRNG, OP_SIGN_VARGEN_STDRNG,
+  OP_VERIFY_WITNESS, OP_VERIFY_WITNESS_BYTES
 };
+static_assert(OP_VERIFY_WITNESS == 37, "min_ctas names the op by number");
 
 struct KArgs {
   int64_t n;
@@ -333,6 +337,31 @@ __global__ void __launch_bounds__(TPB, min_ctas(OP)) k_run(const KArgs a) {
     if (a.aux == 0) witness_core<0>(sk, nonce, m, point_in(), a.combG, a.combGp, emit);
     else if (a.aux == 1) witness_core<1>(sk, nonce, m, point_in(), a.combG, a.combGp, emit);
     else witness_core<2>(sk, nonce, m, ldg_point(a.in[3], i, aff), a.combG, a.combGp, emit);
+    return;
+  }
+  if (OP == OP_VERIFY_WITNESS) {  // aux = scheme; in: pk, u, R, m | pk, pk', u, R, R', m | pk, gen, u, R, m -> out0: rows, bitmap
+    // inv_mask (byte-level call): tuples whose from_bytes failed get a zero row and verdict 0, like the core's own zeroing
+    const bool keep = !a.inv_mask || !(a.inv_mask[i >> 5] >> (i & 31) & 1u);
+    const bool chk = (a.flags & SB200_CHECK_POINTS) != 0;
+    uint32_t u[8];
+    ldg_scalar(a.in[a.aux == 0 ? 1 : 2] + i * 8, u);
+    uint32_t* dst = a.out[0] + i * SB200_WITNESS_WIDTH(a.aux) * 8;
+    auto emit = [&](int k, const fq& v) {
+      const fq x = keep ? v : fq_zero();
+      if (active) stg8(dst + k * 8, x.v);
+    };
+    bool ok;
+    if (a.aux == 0)
+      ok = verify_witness_core<0>(ldg_point(a.in[0], i, aff), point_in(), u, ldg_point(a.in[2], i, aff), point_in(),
+                                  ldg_fq(a.in[3] + i * 8), chk, a.combG, a.combGp, emit);
+    else if (a.aux == 1)
+      ok = verify_witness_core<1>(ldg_point(a.in[0], i, aff), ldg_point(a.in[1], i, aff), u, ldg_point(a.in[3], i, aff),
+                                  ldg_point(a.in[4], i, aff), ldg_fq(a.in[5] + i * 8), chk, a.combG, a.combGp, emit);
+    else
+      ok = verify_witness_core<2>(ldg_point(a.in[0], i, aff), ldg_point(a.in[1], i, aff), u, ldg_point(a.in[3], i, aff),
+                                  point_in(), ldg_fq(a.in[4] + i * 8), chk, a.combG, a.combGp, emit);
+    unsigned word = __ballot_sync(0xffffffffu, ok && keep && active);
+    if ((threadIdx.x & 31) == 0 && active) a.bitmap[i >> 5] = word;
     return;
   }
   if (OP == OP_DBG_FQ) {
@@ -934,8 +963,8 @@ namespace {
 // FIXED: the k_fixed_batch `kernel` (or its SB200_SIGN_OBLIVIOUS form `ct`), fixed_k(op) tuples per thread.  VERIFY:
 // challenge kernel, then curve kernel, the challenges through c_out or scratch.  VERIFY_BYTES: decode kernel, then VERIFY
 // on the decoded rows.  SIGN_STDRNG: the nonces drawn into scratch, then the scheme's sign op.  DBG_VERIFY_EC: the curve
-// kernel alone, on the caller's challenges.
-enum Form : uint8_t { INTERNAL, ONE, FIXED, VERIFY, VERIFY_BYTES, SIGN_STDRNG, DBG_VERIFY_EC };
+// kernel alone, on the caller's challenges.  WITNESS_BYTES: decode kernel, then `kernel` on the decoded rows.
+enum Form : uint8_t { INTERNAL, ONE, FIXED, VERIFY, VERIFY_BYTES, SIGN_STDRNG, DBG_VERIFY_EC, WITNESS_BYTES };
 using KFn = void (*)(KArgs);
 struct OpInfo {
   Form form;
@@ -948,11 +977,12 @@ struct OpInfo {
   int scratch_arrays;   // challenges or nonces, and the decoded rows (points 64 B, u and m 32 B) and invalid bitmap
 };
 constexpr OpInfo row(Form form, uint32_t flags = 0, int scheme = 0, KFn kernel = nullptr, KFn ct = nullptr) {
-  const unsigned points = scheme == 0 ? 2 : scheme == 1 ? 4 : 3, rows = form == VERIFY_BYTES ? 64 * points + 64 : 0;
-  const bool handover = form == VERIFY || form == VERIFY_BYTES || form == SIGN_STDRNG;
+  const bool decode = form == VERIFY_BYTES || form == WITNESS_BYTES;
+  const unsigned points = scheme == 0 ? 2 : scheme == 1 ? 4 : 3, rows = decode ? 64 * points + 64 : 0;
+  const bool handover = form == VERIFY || form == VERIFY_BYTES || form == SIGN_STDRNG;  // + 32 B: the challenge row
   return {form, flags, scheme, kernel, ct, ct ? (size_t)(scheme == 1 ? 2 : 1) * CT_TABLE_WORDS * 4 : 0,
-          form == VERIFY_BYTES ? (uint32_t)SB200_POINTS_AFFINE : 0u, handover ? 32 + rows : 0u,
-          handover ? (rows ? (int)points + 4 : 1) : 0};
+          decode ? (uint32_t)SB200_POINTS_AFFINE : 0u, (handover ? 32u : 0u) + rows,
+          (handover ? 1 : 0) + (rows ? (int)points + 3 : 0)};
 }
 constexpr uint32_t D = SB200_DEVICE_PTRS, AD = SB200_POINTS_AFFINE | D, CHK = AD | SB200_CHECK_POINTS;
 constexpr uint32_t OBL = AD | SB200_SIGN_OBLIVIOUS, DUAL = SB_VERIFY_WS ? SB200_VERIFY_DUAL_PIPE : 0;
@@ -1003,8 +1033,10 @@ constexpr OpInfo OPS[] = {
     row(SIGN_STDRNG, D | SB200_SIGN_OBLIVIOUS, 0),  // OP_SIGN_STDRNG
     row(SIGN_STDRNG, D | SB200_SIGN_OBLIVIOUS, 1),  // OP_SIGN_DOUBLE_STDRNG
     row(SIGN_STDRNG, OBL, 2),                       // OP_SIGN_VARGEN_STDRNG
+    row(ONE, CHK, 0, k_run<OP_VERIFY_WITNESS>),     // the scheme is the call's aux
+    row(WITNESS_BYTES, D, 1, k_run<OP_VERIFY_WITNESS>),  // scheme 1: scratch for the widest decoded rows; the call's scheme is its aux
 };
-static_assert(sizeof(OPS) / sizeof(OPS[0]) == OP_SIGN_VARGEN_STDRNG + 1, "one row per Op");
+static_assert(sizeof(OPS) / sizeof(OPS[0]) == OP_VERIFY_WITNESS_BYTES + 1, "one row per Op");
 
 // ---- launches ---------------------------------------------------------------------------------------------------------
 struct Launcher {  // issues kernels on one stream and counts them (sb200_launch_count)
@@ -1068,23 +1100,28 @@ int launch(sb200_ctx* ctx, Op op, const KArgs& a, cudaStream_t st) {
     case VERIFY:  // a.out[0] is always set here: the caller's c_out or scratch
       rc = launch_verify(go, o.scheme, a, grid);
       break;
-    case VERIFY_BYTES: {  // decode kernel -> challenge kernel -> curve kernel, the decoded rows and the challenges in a.scratch
-      const int npk = o.scheme == 0 ? 1 : 2, nr = o.scheme == 1 ? 2 : 1, narr = npk + 1 + nr + 1;
+    case VERIFY_BYTES:      // decode kernel -> challenge kernel -> curve kernel, the decoded rows and the challenges in a.scratch
+    case WITNESS_BYTES: {   // decode kernel -> o.kernel (rows to out[0], `invalid` in out[1]), the decoded rows in a.scratch
+      const bool wit = o.form == WITNESS_BYTES;
+      const int scheme = wit ? a.aux : o.scheme;
+      const int npk = scheme == 0 ? 1 : 2, nr = scheme == 1 ? 2 : 1, narr = npk + 1 + nr + 1;
       uint8_t* p = a.scratch;
       auto carve = [&](size_t bytes) { uint8_t* r = p; p += (bytes + 63) & ~(size_t)63; return (uint32_t*)r; };
       KArgs dk = a, v = a;
-      dk.aux = o.scheme;
-      v.out[0] = carve((size_t)a.n * 32);
+      dk.aux = scheme;
+      if (!wit) v.out[0] = carve((size_t)a.n * 32);
       for (int k = 0; k < narr; k++) {
         const bool is_scalar = (k == npk) || (k == narr - 1);  // u and m are 8 words, points 16
         dk.dec[k] = carve((size_t)a.n * (is_scalar ? 32 : 64));
         v.in[k] = dk.dec[k];
       }
-      dk.bitmap = a.out[0] ? a.out[0] : carve((size_t)((a.n + 31) / 32) * 4);  // the caller's `invalid` or scratch
+      uint32_t* invalid = a.out[wit ? 1 : 0];
+      dk.bitmap = invalid ? invalid : carve((size_t)((a.n + 31) / 32) * 4);  // the caller's `invalid` or scratch
       v.inv_mask = dk.bitmap;
       for (int k = 1; k < MAX_OUT; k++) v.out[k] = nullptr;
       go(k_run<OP_DECODE_VERIFY>, grid, TPB, 0, dk);
-      rc = launch_verify(go, o.scheme, v, grid);
+      if (wit) go(o.kernel, grid, TPB, 0, v);
+      else rc = launch_verify(go, o.scheme, v, grid);
       break;
     }
     case DBG_VERIFY_EC: {  // in: pk, u, R, c -> bitmap: the production curve kernel, in the form the batch size picks,
@@ -1706,6 +1743,33 @@ int sb200_sign_witness(sb200_ctx* ctx, int64_t n, uint32_t flags, int scheme, co
   Desc d; d.op = OP_WITNESS; d.flags = flags; d.aux = scheme; d.nin = 4; d.nout = 1;
   IN(0, sk, 8); IN(1, msg, 8); IN(2, nonce, 8); IN(3, scheme == 2 ? generator : nullptr, scheme == 2 ? pt_words(flags) : 0);
   OUT(0, rows_out, 8 * width[scheme]);
+  return run(ctx, n, d);
+}
+int sb200_verify_witness(sb200_ctx* ctx, int64_t n, uint32_t flags, int scheme, const uint32_t* pk, const uint32_t* pk2,
+                         const uint32_t* sig_u, const uint32_t* sig_R, const uint32_t* sig_R_prime, const uint32_t* msg,
+                         uint32_t* verdicts, uint32_t* rows_out) {
+  if (scheme < 0 || scheme > 2) return SB200_ERR_ARG;
+  const int pw = pt_words(flags);
+  Desc d; d.op = OP_VERIFY_WITNESS; d.flags = flags; d.aux = scheme; d.nout = 1; BITMAP(verdicts);
+  int k = 0;  // the verify kernels' layout: pk, u, R, m | pk, pk', u, R, R', m | pk, gen, u, R, m
+  IN(k, pk, pw); k++;
+  if (scheme) { IN(k, pk2, pw); k++; }
+  IN(k, sig_u, 8); k++;
+  IN(k, sig_R, pw); k++;
+  if (scheme == 1) { IN(k, sig_R_prime, pw); k++; }
+  IN(k, msg, 8); k++;
+  d.nin = k;
+  OUT(0, rows_out, 8 * SB200_WITNESS_WIDTH(scheme));
+  return run(ctx, n, d);
+}
+int sb200_verify_witness_bytes(sb200_ctx* ctx, int64_t n, uint32_t flags, int scheme, const uint8_t* pk_bytes,
+                               const uint8_t* sig_bytes, const uint8_t* msg32, uint32_t* verdicts, uint32_t* rows_out,
+                               uint32_t* invalid) {
+  if (scheme < 0 || scheme > 2) return SB200_ERR_ARG;
+  Desc d; d.op = OP_VERIFY_WITNESS_BYTES; d.flags = flags; d.aux = scheme; d.nin = 3; d.nout = 2; BITMAP(verdicts);
+  IN(0, (const uint32_t*)pk_bytes, scheme == 0 ? 8 : 16); IN(1, (const uint32_t*)sig_bytes, scheme == 1 ? 24 : 16);
+  IN(2, (const uint32_t*)msg32, 8);
+  OUT(0, rows_out, 8 * SB200_WITNESS_WIDTH(scheme)); OPT_OUT(1, invalid, -1);
   return run(ctx, n, d);
 }
 int sb200_points_check(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* points, uint32_t* ok_bitmap) {

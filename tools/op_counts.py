@@ -1,5 +1,6 @@
 """Count the field operations / 32x32 limb products one tuple costs in each kernel, by running the
-instrumented HOST build of the very same per-tuple code (tests/host_arith.cpp).  Writes
+instrumented HOST build of the very same per-tuple code (tests/host_witness.cpp = tests/host_arith.cpp + the
+verifier-side witness rows).  Writes
 profiles/op_counts.json, which bench.py's roofline uses as "work per tuple"."""
 import json, os, sys, random
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -12,7 +13,7 @@ import hostlib as H, schnorr_oracle as o, vectors as V
 import ctypes, subprocess
 so16 = os.path.join(ROOT, "build", "host_arith16.so")
 subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-DSB_COMB_BITS=16", "-include",
-                       os.path.join(ROOT, "tests", "host_shim.h"), "-o", so16, os.path.join(ROOT, "tests", "host_arith.cpp")])
+                       os.path.join(ROOT, "tests", "host_shim.h"), "-o", so16, os.path.join(ROOT, "tests", "host_witness.cpp")])
 lib = ctypes.CDLL(so16)
 H.setup_hades(lib)  # Hades tables derived from the oracle's current round constants, as sb200_init_ex does
 W, NWIN, NENT = 16, 16, (1 << 15) + 1
@@ -81,6 +82,13 @@ vb["imad_wide_per_tuple"] += 120
 vb["fq_mul"] += 1
 vb["note"] = "decode kernel (2 point decompressions + message to Montgomery form) + challenge kernel + curve kernel"
 out["verify_bytes"] = vb
+# verifier-side witness rows (core.cuh verify_witness_core) of valid signatures, affine inputs: u G by comb (u G' too), u GEN
+# and c PK by 64-window variable-base multiplication, two batched Euclidean inversions
+rows = np.zeros(8 * 19, np.uint32)
+nul = np.zeros(24, np.uint32)
+out["verify_witness_single"] = measure(lambda: lib.h_verify_witness(0, H.ptr(H.pt_mont(pk)), H.ptr(nul), H.ptr(H.limbs(u)), H.ptr(H.pt_mont(Rp)), H.ptr(nul), H.ptr(H.mont(m)), 1, 0, H.ptr(tab[0]), H.ptr(tab[1]), H.ptr(rows)))
+out["verify_witness_double"] = measure(lambda: lib.h_verify_witness(1, H.ptr(H.pt_mont(pk)), H.ptr(H.pt_mont(pkp)), H.ptr(H.limbs(ud)), H.ptr(H.pt_mont(Rd)), H.ptr(H.pt_mont(Rdp)), H.ptr(H.mont(m)), 1, 0, H.ptr(tab[0]), H.ptr(tab[1]), H.ptr(rows)))
+out["verify_witness_vargen"] = measure(lambda: lib.h_verify_witness(2, H.ptr(H.pt_mont(pkv)), H.ptr(H.pt_mont(gen)), H.ptr(H.limbs(uvg)), H.ptr(H.pt_mont(Rvg)), H.ptr(nul), H.ptr(H.mont(m)), 1, 0, H.ptr(tab[0]), H.ptr(tab[1]), H.ptr(rows)))
 st = np.concatenate([H.mont(x) for x in range(5)])
 out["hades_perm_sparse"] = measure(lambda: lib.h_hades(H.ptr(st), 0))  # the production form: small-integer layers for the default MDS
 out["hades_perm_dense"] = measure(lambda: lib.h_hades(H.ptr(st), 1))
