@@ -6,4 +6,4 @@ Layout: `csrc/` holds the CUDA kernels and the C ABI (`include/schnorr_b200.h`);
 There is no CPU fallback anywhere in this package.
 """
 from ._lib import (ARK_CUMSUM, ARK_ENV, ARK_PLAIN, CHECK_POINTS, DEVICE_PTRS, POINTS_AFFINE, POINTS_PROJECTIVE, SIGN_OBLIVIOUS,  # noqa: F401
-                   VERIFY_DUAL_PIPE, Engine, Params, PinnedBuffer, SchnorrB200Error, default_params, load_library)
+                   VERIFY_DUAL_PIPE, Engine, KeySet, Params, PinnedBuffer, SchnorrB200Error, default_params, load_library)

@@ -7,6 +7,7 @@ from __future__ import annotations
 
 import ctypes
 import os
+import weakref
 from typing import Optional, Sequence
 
 import numpy as np
@@ -126,6 +127,11 @@ _WITNESS_PROTOTYPES = {  # every symbol of include/schnorr_b200_witness.h (verif
     "sb200_verify_witness": (ci, [vp, i64, u32, ci] + [u32p] * 8),
     "sb200_verify_witness_bytes": (ci, [vp, i64, u32, ci] + [u32p] * 6),
 }
+_KEYSET_PROTOTYPES = {  # every symbol of include/schnorr_b200_keyset.h (verification against registered keys)
+    "sb200_keyset_create": (ci, [vp, ci, i64, u32, u32p, u32p, u32p, ctypes.POINTER(vp)]),
+    "sb200_keyset_destroy": (None, [vp]),
+    "sb200_verify_keyset": (ci, [vp, vp, i64, u32] + [u32p] * 7),
+}
 del vp, u32p, i64, u32, ci
 EXPORTED_SYMBOLS = list(_PROTOTYPES)  # the symbols of include/schnorr_b200.h
 
@@ -146,7 +152,7 @@ def load_library() -> ctypes.CDLL:
             f"{LIB_PATH} not found: build it with `python -c 'import __graft_entry__ as g; g.build()'` "
             "(nvcc, sm_100a). There is no CPU fallback.")
     lib = ctypes.CDLL(LIB_PATH)
-    for name, (res, args) in {**_PROTOTYPES, **_WITNESS_PROTOTYPES}.items():
+    for name, (res, args) in {**_PROTOTYPES, **_WITNESS_PROTOTYPES, **_KEYSET_PROTOTYPES}.items():
         fn = getattr(lib, name)  # AttributeError if the library does not export a declared symbol
         fn.restype, fn.argtypes = res, args
     _lib = lib
@@ -219,9 +225,12 @@ class Engine:
             raise err
         self._h = h
         self.devices = devs
+        self._keysets = weakref.WeakSet()
 
     def close(self):
         if getattr(self, "_h", None):
+            for ks in list(self._keysets):  # sb200_destroy frees them: their handles die with the context
+                ks._h = None
             self._lib.sb200_destroy(self._h)
             self._h = None
 
@@ -511,6 +520,11 @@ class Engine:
         self._check(rc, "verify_witness_bytes")
         return self._unpack_bits(bm, n), self._unpack_bits(inv, n), rows
 
+    def keyset(self, scheme: int, pk, pk2=None, affine=True) -> "KeySet":
+        """register n_keys public keys (include/schnorr_b200_keyset.h): per-key comb tables built on every device.
+        pk2 = PK' (scheme 1) or the keys' generators (scheme 2)."""
+        return KeySet(self, scheme, pk, pk2, affine)
+
     def points_check(self, points, affine=True):
         """ok[n]: point i is on the curve with Z != 0 (what CHECK_POINTS applies inside the verify calls)"""
         n = np.asarray(points).size // self._pw(affine)
@@ -574,3 +588,59 @@ class Engine:
         rc = self._lib.sb200_dbg_scalar_mul(self._h, n, fl, base, p.ctypes.data if p is not None else None, k.ctypes.data, out.ctypes.data)
         self._check(rc, "dbg_scalar_mul")
         return out
+
+
+class KeySet:
+    """Public keys registered on every device of an Engine (include/schnorr_b200_keyset.h): `key_ok` (bool[n_keys]: every
+    point of the key is on the curve with Z != 0) and `verify`.  Frees its device memory on close() / exit / GC."""
+
+    def __init__(self, engine: Engine, scheme: int, pk, pk2=None, affine=True):
+        pw = engine._pw(affine)
+        n = np.asarray(pk).size // pw
+        pk = _arr(pk, pw, n, "pk")
+        pk2 = _arr(pk2, pw, n, "pk2") if scheme in (1, 2) else None
+        ok = aligned_empty(((n + 31) // 32 + 1,)); ok[...] = 0
+        h = ctypes.c_void_p()
+        rc = engine._lib.sb200_keyset_create(engine._h, scheme, n, POINTS_AFFINE if affine else POINTS_PROJECTIVE, pk.ctypes.data,
+                                             pk2.ctypes.data if pk2 is not None else None, ok.ctypes.data, ctypes.byref(h))
+        engine._check(rc, "keyset_create")
+        self._engine, self._h, self.scheme, self.n_keys = engine, h, scheme, n
+        self.key_ok = engine._unpack_bits(ok, n)
+        engine._keysets.add(self)
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._engine._lib.sb200_keyset_destroy(self._h)
+            self._h = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def verify(self, key_index, u, R, msg, Rp=None, affine=True, want_c=True, check_points=False):
+        """verdict i = the scheme's verify of (key key_index[i], u[i], R[i] (, Rp[i]), msg[i]): (ok[n], c[n, 8] or None).
+        An index >= n_keys or a key that is not key_ok gives verdict 0."""
+        e = self._engine
+        if not self._h:
+            raise SchnorrB200Error("verify: the keyset is closed")
+        idx = _arr(np.asarray(key_index).astype(np.uint32).reshape(-1), None, 0, "key_index")
+        n = idx.size
+        pw = e._pw(affine)
+        fl = (POINTS_AFFINE if affine else POINTS_PROJECTIVE) | (CHECK_POINTS if check_points else 0)
+        u, R, msg = _arr(u, 8, n, "u"), _arr(R, pw, n, "R"), _arr(msg, 8, n, "msg")
+        Rp = _arr(Rp, pw, n, "R'") if self.scheme == 1 else None
+        bm = aligned_empty(((n + 31) // 32,)); bm[...] = 0
+        c = aligned_empty((n, 8)) if want_c else None
+        rc = e._lib.sb200_verify_keyset(e._h, self._h, n, fl, idx.ctypes.data, u.ctypes.data, R.ctypes.data,
+                                        Rp.ctypes.data if Rp is not None else None, msg.ctypes.data, bm.ctypes.data,
+                                        c.ctypes.data if want_c else None)
+        e._check(rc, "verify_keyset")
+        return e._unpack_bits(bm, n), c

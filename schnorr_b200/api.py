@@ -558,3 +558,48 @@ class PublicKeyVarGen:
                                            _scalars([s._u for s in sigs]), _points([s._R for s in sigs]), _fqs(msgs),
                                            affine=False, want_c=False)
         return ok
+
+
+class PublicKeySet:
+    """A fixed set of public keys of one type (PublicKey, PublicKeyDouble or PublicKeyVarGen) registered once on the
+    device (include/schnorr_b200_keyset.h), for callers that verify many signatures of the same keys: each key gets
+    fixed-base tables, so a verification no longer multiplies by the key as a fresh point.  Not in the reference: an
+    addition of this library.  `verify_batch(indices, sigs, msgs)` returns what the type's
+    `verify_batch([keys[i] for i in indices], sigs, msgs)` returns (a key not on the curve verifies nothing)."""
+
+    _SCHEMES = {PublicKey: 0, PublicKeyDouble: 1, PublicKeyVarGen: 2}
+
+    def __init__(self, keys: Sequence):
+        keys = list(keys)
+        types = {type(k) for k in keys}
+        if len(types) != 1 or next(iter(types)) not in self._SCHEMES:
+            raise TypeError("PublicKeySet: a non-empty sequence of PublicKey, PublicKeyDouble or PublicKeyVarGen, one type")
+        self.keys = keys
+        self.scheme = self._SCHEMES[types.pop()]
+        pk2 = None
+        if self.scheme == 1:
+            pk2 = _points([k._pp for k in keys])
+        elif self.scheme == 2:
+            pk2 = _points([k._g for k in keys])
+        self._ks = get_engine().keyset(self.scheme, _points([k._p for k in keys]), pk2, affine=False)
+
+    def __len__(self):
+        return len(self.keys)
+
+    def close(self):
+        self._ks.close()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def verify_batch(self, indices: Sequence[int], sigs: Sequence, msgs: Sequence[int]) -> np.ndarray:
+        idx = np.asarray(indices, dtype=np.int64).reshape(-1)
+        if idx.size and (idx.min() < 0 or idx.max() >= len(self.keys)):
+            raise IndexError("PublicKeySet.verify_batch: key index out of range")
+        Rp = _points([s._Rp for s in sigs]) if self.scheme == 1 else None
+        ok, _ = self._ks.verify(idx.astype(np.uint32), _scalars([s._u for s in sigs]), _points([s._R for s in sigs]), _fqs(msgs),
+                                Rp=Rp, affine=False, want_c=False)
+        return ok

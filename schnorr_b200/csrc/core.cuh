@@ -408,6 +408,54 @@ SB_HD void batch_inverse(fq* z, fq* pre, int n) {
   z[0] = inv;
 }
 
+// Window j of P's per-key comb (ed.cuh, KS_*) into `win` (KS_ENTRIES x 24 words): B = 2^(8j) P by 8j doublings, then
+// 2B .. 128B by repeated addition, held as (X, Y) in the entry's own words and Z in z[e - 1]; one batched inversion of the
+// 128 Z (z and pre: KS_ENTRIES - 1 fq each of caller memory) and the affine Niels form in place.  Only public data enters:
+// the Euclidean inversion.  A P off the curve or with Z = 0 leaves garbage in this window and nowhere else.
+SB_HD void keyset_build_window(const ext& P, int j, uint32_t* win, fq* z, fq* pre) {
+  constexpr int NE = KS_ENTRIES - 1;  // entries 1..128
+  ext B = P;
+#pragma unroll 1
+  for (int i = 0; i < KS_BITS * j; i++) B = p1p1_to_ext(ed_dbl(B.X, B.Y, B.Z));
+  const pniels nb = ext_to_pniels(B);
+  ext cur = B;
+#pragma unroll 1
+  for (int e = 1; e <= NE; e++) {
+    if (e > 1) cur = p1p1_to_ext(ed_add(cur, nb));
+#pragma unroll
+    for (int i = 0; i < 8; i++) {
+      win[24 * e + i] = cur.X.v[i];
+      win[24 * e + 8 + i] = cur.Y.v[i];
+    }
+    z[e - 1] = cur.Z;
+  }
+  batch_inverse(z, pre, NE);
+#pragma unroll 1
+  for (int e = 1; e <= NE; e++) {
+    fq X, Y;
+#pragma unroll
+    for (int i = 0; i < 8; i++) {
+      X.v[i] = win[24 * e + i];
+      Y.v[i] = win[24 * e + 8 + i];
+    }
+    const fq zi = z[e - 1], x = fq_mul(X, zi), y = fq_mul(Y, zi);
+    const fq ypx = fq_add(y, x), ymx = fq_sub(y, x), t2d = fq_mul(fq_mul(x, y), ed_2d());
+#pragma unroll
+    for (int i = 0; i < 8; i++) {
+      win[24 * e + i] = ypx.v[i];
+      win[24 * e + 8 + i] = ymx.v[i];
+      win[24 * e + 16 + i] = t2d.v[i];
+    }
+  }
+  const fq one = fq_one();  // entry 0: the identity (1, 1, 0)
+#pragma unroll
+  for (int i = 0; i < 8; i++) {
+    win[i] = one.v[i];
+    win[8 + i] = one.v[i];
+    win[16 + i] = 0u;
+  }
+}
+
 // u = nonce - c * sk  (mod r)
 SB_HD void sign_finish(const uint32_t* nonce, const uint32_t* c, const uint32_t* sk, uint32_t* u_out) {
   fr a, b, n;
@@ -640,6 +688,52 @@ SB_HD bool verify_witness_core(const point_in& PK, const point_in& PK2, const ui
   for (int k = 0; k < 2 * NB; k++) {
     put(o++, fq_mul(S[k].X, z[k]));
     put(o++, fq_mul(S[k].Y, z[k]));
+  }
+  return ok;
+}
+
+// Verification against a registered key (include/schnorr_b200_keyset.h).  `tabs`: the keyset's per-key combs, key k's
+// at tabs + k * NT * KS_TABLE_WORDS (NT = 1 for SCHEME 0: PK; 2 for SCHEME 1: PK, PK'; 2 for SCHEME 2: PK, GEN), `key_ok`
+// bit k = every point of key k is well formed.  c_out = the challenge sb200_verify* writes; the verdict is the predicate
+// it decides (u B + c PK == R, and u G' + c PK' == R' for SCHEME 1), with u B by the 16-bit comb of G / G' or, for a
+// variable generator, by the key's own comb of GEN.  Exact on the whole curve: no short vector, no fallback.  The verdict
+// is 0 when u >= r, key >= n_keys (key 0's table is read instead, never past the end), key_ok is clear, or with
+// `check_points` R (R') is not well formed -- by mask: every lane runs the same work.
+template <int SCHEME>
+SB_HD bool verify_keyset_core(const uint32_t* tabs, int64_t n_keys, const uint32_t* key_ok, uint32_t key, const uint32_t* u_in,
+                              const point_in& R, const point_in& Rp, const fq& m, bool check_points, const uint32_t* combG,
+                              const uint32_t* combGp, uint32_t* c_out) {
+  constexpr int NT = SCHEME == 0 ? 1 : 2;
+  if (SCHEME == 1) verify_double_hash_core(R, Rp, m, c_out); else verify_hash_core(R, m, c_out);
+  const bool known = (int64_t)key < n_keys;
+  const uint64_t k = known ? key : 0u;
+  const bool lt = scalar_lt_r(u_in);
+  bool ok = known & ((key_ok[k >> 5] >> (k & 31) & 1u) != 0) & lt;
+  uint32_t u[8], c[8];
+#pragma unroll
+  for (int i = 0; i < 8; i++) {
+    u[i] = lt ? u_in[i] : 0u;  // in range for the recoding; the verdict is 0 anyway
+    c[i] = c_out[i];
+  }
+  recode_offset<KS_BITS>(c);
+  const uint32_t* tab = tabs + k * NT * KS_TABLE_WORDS;
+  if (SCHEME == 2) {  // u GEN + c PK, both from the key's combs
+    recode_offset<KS_BITS>(u);
+    p1p1 s = ed_comb_add_w<KS_BITS>(ext_identity(), tab + KS_TABLE_WORDS, u);
+    s = ed_comb_add_w<KS_BITS>(p1p1_to_ext(s), tab, c);
+    ok &= p1p1_equals(s, R);
+  } else {  // u G + c PK (and u G' + c PK'): one copy of the curve code
+    recode_offset<COMB_BITS>(u);
+#pragma unroll 1
+    for (int b = 0; b < NT; b++) {
+      p1p1 s = ed_comb_add(ext_identity(), b ? combGp : combG, u);
+      s = ed_comb_add_w<KS_BITS>(p1p1_to_ext(s), tab + b * KS_TABLE_WORDS, c);
+      ok &= p1p1_equals(s, b ? Rp : R);
+    }
+  }
+  if (check_points) {  // warp-uniform
+    ok &= point_well_formed(R);
+    if (SCHEME == 1) ok &= point_well_formed(Rp);
   }
   return ok;
 }

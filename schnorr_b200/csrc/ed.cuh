@@ -501,6 +501,47 @@ SB_HD p1p1 ed_comb_add(ext acc, const uint32_t* table, const uint32_t* k_rec) {
 }
 
 // ------------------------------------------------------------------------------------------
+// per-key comb of a registered public key (include/schnorr_b200_keyset.h): the layout of the G comb with a fixed 8-bit
+// window on the device and in the host build alike (independent of SB_COMB_BITS).  Window j, entry e (0..128) =
+// e * 2^(8j) * P in affine Niels form, entry 0 = identity: 32 windows x 129 entries x 96 B = 396 288 B per point, and
+// k * P (k < 2^252: 32 signed digits in [-128, 127]) is 32 mixed additions with no doubling.  Every entry is an exact
+// integer multiple of P, so the sum is k * P on the whole curve, torsion points included.  Width 4 would take 55 KB and
+// 64 additions per point; width 8 halves the additions for 7x the memory.  180 GB hold about 450 000 single-key keys
+// (225 000 double-key or variable-generator keys, which have two points each) less the batch buffers: 2^16 single-key
+// keys take 26 GB.
+// ------------------------------------------------------------------------------------------
+constexpr int KS_BITS = 8;
+constexpr int KS_WINDOWS = 256 / KS_BITS;
+constexpr int KS_ENTRIES = (1 << (KS_BITS - 1)) + 1;
+constexpr size_t KS_TABLE_WORDS = (size_t)KS_WINDOWS * KS_ENTRIES * 24;  // 99 072 words per point
+
+SB_HD aniels aniels_load(const uint32_t* entry) {  // one 96-byte affine Niels entry (six 16-byte loads)
+  const uint4* p = reinterpret_cast<const uint4*>(entry);
+  uint4 q0 = p[0], q1 = p[1], q2 = p[2], q3 = p[3], q4 = p[4], q5 = p[5];
+  aniels r;
+  r.YpX = {{q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, q1.z, q1.w}};
+  r.YmX = {{q2.x, q2.y, q2.z, q2.w, q3.x, q3.y, q3.z, q3.w}};
+  r.T2d = {{q4.x, q4.y, q4.z, q4.w, q5.x, q5.y, q5.z, q5.w}};
+  return r;
+}
+
+// acc (extended) += k*B for the comb of W-bit windows (2^(W-1) + 1 entries each) at `table`; k offset-recoded for W.
+// ed_comb_add's loop with the table layout as a parameter.
+template <int W>
+SB_HD p1p1 ed_comb_add_w(ext acc, const uint32_t* table, const uint32_t* k_rec) {
+  constexpr int NW = 256 / W, NE = (1 << (W - 1)) + 1;
+  p1p1 c;
+#pragma unroll 1
+  for (int j = 0; j < NW; j++) {
+    const int d = recode_digit<W>(k_rec, j);
+    const bool neg = d < 0;
+    c = ed_add(acc, aniels_cneg(aniels_load(table + (size_t)(j * NE + (neg ? -d : d)) * 24), neg));
+    if (j + 1 < NW) acc = p1p1_to_ext(c);
+  }
+  return c;
+}
+
+// ------------------------------------------------------------------------------------------
 // Address-oblivious scalar multiplication (SB200_SIGN_OBLIVIOUS): the same group elements as above with no
 // memory address and no branch depending on the (secret) scalar -- the property of the reference's ladder
 // (`acc += select(identity, P, bit)`, dusk-jubjub) that the 16-bit comb gives up by indexing a 50 MB table with

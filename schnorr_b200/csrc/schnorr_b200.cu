@@ -21,6 +21,7 @@
 
 #include "../../include/schnorr_b200.h"
 #include "../../include/schnorr_b200_witness.h"
+#include "../../include/schnorr_b200_keyset.h"
 #include "wire.cuh"
 #include "rng.cuh"
 #include "params_host.cuh"
@@ -67,7 +68,7 @@ enum Op : int {
   OP_CHALLENGE_DOUBLE, OP_VERIFY_DOUBLE_EC, OP_CHALLENGE_VARGEN, OP_VERIFY_VARGEN_EC, OP_POINTS_CHECK, OP_DBG_VERIFY_EC,
   OP_DECODE_VERIFY, OP_WITNESS, OP_DBG_LAT3,
   OP_STDRNG, OP_SIGN_STDRNG, OP_SIGN_DOUBLE_STDRNG, OP_SIGN_VARGEN_STDRNG,
-  OP_VERIFY_WITNESS, OP_VERIFY_WITNESS_BYTES
+  OP_VERIFY_WITNESS, OP_VERIFY_WITNESS_BYTES, OP_VERIFY_KEYSET
 };
 static_assert(OP_VERIFY_WITNESS == 37, "min_ctas names the op by number");
 
@@ -91,6 +92,13 @@ struct KArgs {
   uint32_t* dec[MAX_IN];     // decode kernel: where the decoded arrays of the byte-level verify calls go
   uint32_t rng_key[8];       // OP_STDRNG: the StdRng seed (secret: it reaches the device only as this kernel parameter)
   uint64_t rng_word;         // OP_STDRNG: keystream word position of tuple 0 of this launch
+};
+// The keyset of an OP_VERIFY_KEYSET launch, as this device's copy: a second kernel parameter rather than more KArgs
+// fields, so that the parameter offsets of the existing two-parameter kernels (k_curve_p) stay where they are.
+struct KsArgs {
+  const uint32_t* tab = nullptr;  // per-key combs
+  int64_t n = 0;                  // number of keys
+  const uint32_t* ok = nullptr;   // key_ok bitmap
 };
 
 // scheduling state of one warp-specialised launch (k_verify_ws): the next-tile counter, reset before every launch,
@@ -861,6 +869,63 @@ __global__ void __launch_bounds__(TPB) k_comb_build(uint32_t* table, const fq bu
   comb_build_entry(bu, bv, t / COMB_ENTRIES, t % COMB_ENTRIES, table + (size_t)t * 24);
 }
 
+// Verification against a keyset (include/schnorr_b200_keyset.h).  aux = scheme; in: key index, u, R, (R',) m -> bitmap,
+// out0 (nullable): c
+__global__ void __launch_bounds__(TPB, SB_MIN_CTAS) k_verify_keyset(const KArgs a, const KsArgs ks) {
+  int64_t i = (int64_t)blockIdx.x * TPB + threadIdx.x;
+  const bool active = i < a.n;
+  if (!active) i = a.n - 1;  // idle lanes redo the last tuple so the warp stays converged
+  const bool aff = (a.flags & SB200_POINTS_AFFINE) != 0, chk = (a.flags & SB200_CHECK_POINTS) != 0;
+  const uint32_t key = __ldg(a.in[0] + i);
+  uint32_t u[8], c[8];
+  ldg_scalar(a.in[1] + i * 8, u);
+  bool ok;
+  if (a.aux == 0)
+    ok = verify_keyset_core<0>(ks.tab, ks.n, ks.ok, key, u, ldg_point(a.in[2], i, aff), point_in(), ldg_fq(a.in[3] + i * 8), chk,
+                               a.combG, a.combGp, c);
+  else if (a.aux == 1)
+    ok = verify_keyset_core<1>(ks.tab, ks.n, ks.ok, key, u, ldg_point(a.in[2], i, aff), ldg_point(a.in[3], i, aff),
+                               ldg_fq(a.in[4] + i * 8), chk, a.combG, a.combGp, c);
+  else
+    ok = verify_keyset_core<2>(ks.tab, ks.n, ks.ok, key, u, ldg_point(a.in[2], i, aff), point_in(), ldg_fq(a.in[3] + i * 8), chk,
+                               a.combG, a.combGp, c);
+  unsigned word = __ballot_sync(0xffffffffu, ok && active);
+  if ((threadIdx.x & 31) == 0 && active) a.bitmap[i >> 5] = word;
+  if (a.out[0] && active) stg8(a.out[0] + i * 8, c);
+}
+
+// Per-key combs of a keyset (include/schnorr_b200_keyset.h): one warp per key of [key0, key0 + nk), one lane per window
+// (keyset_build_window), the key's NT points one after the other, then its key_ok bit.  Lane-divergent doubling counts
+// (8 j for window j): a one-off build, not a hot path.  scratch: 2 x (KS_ENTRIES - 1) fq per thread of the launch.
+constexpr int64_t KS_BUILD_KEYS = 2048;  // keys per build launch: 536 MB of scratch
+struct KsBuild {
+  uint32_t* tab;
+  uint32_t* ok;
+  const uint32_t* pk;
+  const uint32_t* pk2;
+  int64_t key0, nk;
+  int nt;
+  bool aff;
+  fq* scratch;
+};
+__global__ void __launch_bounds__(TPB) k_keyset_build(const KsBuild b) {
+  static_assert(KS_WINDOWS == 32, "one lane per window");
+  const int64_t t = (int64_t)blockIdx.x * TPB + threadIdx.x, w = t >> 5;
+  const int lane = threadIdx.x & 31;
+  if (w >= b.nk) return;  // warp-uniform
+  const int64_t k = b.key0 + w;
+  fq* z = b.scratch + (size_t)t * 2 * (KS_ENTRIES - 1);
+  bool well = true;
+#pragma unroll 1
+  for (int p = 0; p < b.nt; p++) {
+    const point_in P = ldg_point(p ? b.pk2 : b.pk, k, b.aff);
+    well &= point_well_formed(P);
+    keyset_build_window(point_to_ext(P), lane, b.tab + ((size_t)k * b.nt + p) * KS_TABLE_WORDS + (size_t)lane * KS_ENTRIES * 24, z,
+                        z + (KS_ENTRIES - 1));
+  }
+  if (lane == 0 && well) atomicOr(b.ok + (k >> 5), 1u << (k & 31));
+}
+
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
@@ -906,6 +971,7 @@ struct Desc {
   int out_words[MAX_OUT] = {};
   uint32_t* bitmap = nullptr;
   const sb200_stdrng* rng = nullptr;  // OP_STDRNG and the seeded signers: key and word position of tuple 0
+  const sb200_keyset* ks = nullptr;   // OP_VERIFY_KEYSET: whose per-device tables the kernels read
   unsigned need = 0;  // outputs that may not be null: bit k for out[k], bit MAX_OUT for the bitmap
 };
 
@@ -941,10 +1007,22 @@ struct sb200_ctx {
   sb200_params params;
   HadesTables tables;
   int persist = 0;  // environment variable SB200_CURVE_PERSISTENT at context creation: "always" | "never" | unset (by batch size)
+  std::vector<sb200_keyset*> keysets;  // alive keysets of this context (sb200_destroy frees them)
   void set_err(const std::string& e) {
     std::lock_guard<std::mutex> l(err_mu);
     if (err.empty() || e.empty()) err = e;
   }
+};
+
+struct sb200_keyset {
+  struct Dev {
+    uint32_t* tab = nullptr;  // n_keys x (scheme == 0 ? 1 : 2) x KS_TABLE_WORDS
+    uint32_t* ok = nullptr;   // key_ok bitmap
+  };
+  sb200_ctx* ctx;
+  int scheme;
+  int64_t n_keys;
+  std::vector<Dev> dev;  // one copy per device of ctx, in ctx->devs order
 };
 
 namespace {
@@ -963,8 +1041,9 @@ namespace {
 // FIXED: the k_fixed_batch `kernel` (or its SB200_SIGN_OBLIVIOUS form `ct`), fixed_k(op) tuples per thread.  VERIFY:
 // challenge kernel, then curve kernel, the challenges through c_out or scratch.  VERIFY_BYTES: decode kernel, then VERIFY
 // on the decoded rows.  SIGN_STDRNG: the nonces drawn into scratch, then the scheme's sign op.  DBG_VERIFY_EC: the curve
-// kernel alone, on the caller's challenges.  WITNESS_BYTES: decode kernel, then `kernel` on the decoded rows.
-enum Form : uint8_t { INTERNAL, ONE, FIXED, VERIFY, VERIFY_BYTES, SIGN_STDRNG, DBG_VERIFY_EC, WITNESS_BYTES };
+// kernel alone, on the caller's challenges.  WITNESS_BYTES: decode kernel, then `kernel` on the decoded rows.  KEYSET:
+// k_verify_keyset, one tuple per thread, with the keyset's tables of the launching device.
+enum Form : uint8_t { INTERNAL, ONE, FIXED, VERIFY, VERIFY_BYTES, SIGN_STDRNG, DBG_VERIFY_EC, WITNESS_BYTES, KEYSET };
 using KFn = void (*)(KArgs);
 struct OpInfo {
   Form form;
@@ -1035,8 +1114,9 @@ constexpr OpInfo OPS[] = {
     row(SIGN_STDRNG, OBL, 2),                       // OP_SIGN_VARGEN_STDRNG
     row(ONE, CHK, 0, k_run<OP_VERIFY_WITNESS>),     // the scheme is the call's aux
     row(WITNESS_BYTES, D, 1, k_run<OP_VERIFY_WITNESS>),  // scheme 1: scratch for the widest decoded rows; the call's scheme is its aux
+    row(KEYSET, CHK),                               // OP_VERIFY_KEYSET: the keyset's scheme is the call's aux
 };
-static_assert(sizeof(OPS) / sizeof(OPS[0]) == OP_VERIFY_WITNESS_BYTES + 1, "one row per Op");
+static_assert(sizeof(OPS) / sizeof(OPS[0]) == OP_VERIFY_KEYSET + 1, "one row per Op");
 
 // ---- launches ---------------------------------------------------------------------------------------------------------
 struct Launcher {  // issues kernels on one stream and counts them (sb200_launch_count)
@@ -1075,7 +1155,7 @@ int launch_verify(const Launcher& go, int scheme, const KArgs& a, unsigned grid)
   return launch_curve(go, scheme, a, grid);
 }
 
-int launch(sb200_ctx* ctx, Op op, const KArgs& a, cudaStream_t st) {
+int launch(sb200_ctx* ctx, Op op, const KArgs& a, cudaStream_t st, const KsArgs& ks = KsArgs()) {
   if (a.n <= 0) return SB200_OK;
   const OpInfo& o = OPS[op];
   const Launcher go{ctx, st};
@@ -1124,6 +1204,9 @@ int launch(sb200_ctx* ctx, Op op, const KArgs& a, cudaStream_t st) {
       else rc = launch_verify(go, o.scheme, v, grid);
       break;
     }
+    case KEYSET:
+      go(k_verify_keyset, grid, TPB, 0, a, ks);
+      break;
     case DBG_VERIFY_EC: {  // in: pk, u, R, c -> bitmap: the production curve kernel, in the form the batch size picks,
                            // fed the caller's challenges where the challenge kernel would have written them
       KArgs v = a;
@@ -1176,6 +1259,15 @@ KArgs kargs(const sb200_ctx* ctx, const DevCtx& dc, int slot, const Desc& d, int
     a.rng_word = d.rng->word_pos + 16u * (uint64_t)first;
   }
   return a;
+}
+// the keyset tables of one device's copy (OP_VERIFY_KEYSET), none for every other op
+KsArgs ks_args(const sb200_ctx* ctx, const DevCtx& dc, const Desc& d) {
+  KsArgs k;
+  if (d.ks) {
+    const sb200_keyset::Dev& kd = d.ks->dev[&dc - ctx->devs.data()];
+    k.tab = kd.tab; k.n = d.ks->n_keys; k.ok = kd.ok;
+  }
+  return k;
 }
 
 bool host_pinned(const void* p) {
@@ -1265,7 +1357,7 @@ int run_device(sb200_ctx* ctx, DevCtx& dc, const Desc& d, int64_t lo, int64_t hi
     }
     uint32_t* dbm = nullptr;
     if (d.bitmap) a.bitmap = dbm = (uint32_t*)carve(p, bm_bytes);
-    if ((rc = launch(ctx, d.op, a, st))) return rc;
+    if ((rc = launch(ctx, d.op, a, st, ks_args(ctx, dc, d)))) return rc;
     auto d2h = [&](uint32_t* host_dst, const uint32_t* dev_src, size_t bytes, bool pinned) -> int {
       uint8_t* dst = (uint8_t*)host_dst;
       if (!pinned) {
@@ -1336,7 +1428,7 @@ int run(sb200_ctx* ctx, int64_t n, Desc d) {
       a.scratch = (uint8_t*)dc.cscratch;
       if (splits_with_scratch(d)) a.out[0] = dc.cscratch;
     }
-    int rc = launch(ctx, d.op, a, st);
+    int rc = launch(ctx, d.op, a, st, ks_args(ctx, dc, d));
     if (rc) return rc;
     CU(cudaEventRecord(dc.user_ev, st));
     dc.user_ev_valid = true;
@@ -1407,6 +1499,18 @@ void release_device(DevCtx& dc) {
     if (it != g_dev_params.end() && --it->second.refs <= 0) g_dev_params.erase(it);
   }
   dc = DevCtx();
+}
+
+// a keyset's device memory on every device of its context (work of earlier SB200_DEVICE_PTRS calls may still read it)
+void keyset_free(sb200_keyset* ks) {
+  for (size_t di = 0; di < ks->dev.size(); di++) {
+    DevCtx& dc = ks->ctx->devs[di];
+    cudaSetDevice(dc.dev);
+    if (dc.user_ev_valid) cudaEventSynchronize(dc.user_ev);
+    if (ks->dev[di].tab) cudaFree(ks->dev[di].tab);
+    if (ks->dev[di].ok) cudaFree(ks->dev[di].ok);
+  }
+  delete ks;
 }
 
 // parameters -> validated, derived, self-checked tables.  Host only.
@@ -1548,6 +1652,7 @@ void sb200_destroy(sb200_ctx* ctx) {
   if (!ctx) return;
   {
     DeviceGuard guard;
+    for (sb200_keyset* ks : ctx->keysets) keyset_free(ks);
     for (auto& dc : ctx->devs) release_device(dc);
   }
   delete ctx;
@@ -1770,6 +1875,107 @@ int sb200_verify_witness_bytes(sb200_ctx* ctx, int64_t n, uint32_t flags, int sc
   IN(0, (const uint32_t*)pk_bytes, scheme == 0 ? 8 : 16); IN(1, (const uint32_t*)sig_bytes, scheme == 1 ? 24 : 16);
   IN(2, (const uint32_t*)msg32, 8);
   OUT(0, rows_out, 8 * SB200_WITNESS_WIDTH(scheme)); OPT_OUT(1, invalid, -1);
+  return run(ctx, n, d);
+}
+int sb200_keyset_create(sb200_ctx* ctx, int scheme, int64_t n_keys, uint32_t flags, const uint32_t* pk, const uint32_t* pk2,
+                        uint32_t* key_ok, sb200_keyset** out) {
+  if (out) *out = nullptr;
+  const int nt = scheme == 0 ? 1 : 2;
+  const bool devptrs = (flags & SB200_DEVICE_PTRS) != 0;
+  if (!ctx || !out || scheme < 0 || scheme > 2 || n_keys < 1 || n_keys > (int64_t)UINT32_MAX ||
+      (flags & ~(SB200_POINTS_AFFINE | SB200_DEVICE_PTRS)))
+    return SB200_ERR_ARG;
+  if (!pk || ((uintptr_t)pk & 15) || (nt == 2 && (!pk2 || ((uintptr_t)pk2 & 15)))) return SB200_ERR_ARG;
+  if (devptrs && ctx->devs.size() != 1) return SB200_ERR_ARG;
+  std::lock_guard<std::mutex> lock(ctx->mu);
+  ctx->set_err("");
+  DeviceGuard guard;
+  const size_t ndev = ctx->devs.size(), pt_bytes = (size_t)n_keys * pt_words(flags) * 4;
+  const size_t tab_bytes = (size_t)n_keys * nt * KS_TABLE_WORDS * 4, ok_bytes = (size_t)((n_keys + 31) / 32) * 4;
+  const int64_t batch = std::min<int64_t>(n_keys, KS_BUILD_KEYS);
+  const size_t scr_bytes = (size_t)batch * 32 * 2 * (KS_ENTRIES - 1) * sizeof(fq);
+  sb200_keyset* ks = new sb200_keyset{ctx, scheme, n_keys, std::vector<sb200_keyset::Dev>(ndev)};
+  std::vector<uint8_t*> tmp(3 * ndev, nullptr);  // per device: scratch, and the copies of pk, pk2 (host inputs)
+  auto fail = [&](int code, const char* what) {
+    for (size_t di = 0; di < ndev; di++) {
+      cudaSetDevice(ctx->devs[di].dev);
+      if (devptrs) cudaStreamSynchronize(ctx->user_stream);
+      for (int k = 0; k < 3; k++)
+        if (tmp[3 * di + k]) cudaFree(tmp[3 * di + k]);
+    }
+    if (code != SB200_OK) {
+      cudaGetLastError();  // a failed allocation is not the next call's error
+      keyset_free(ks);
+      ctx->set_err(what);
+    }
+    return code;
+  };
+  for (size_t di = 0; di < ndev; di++) {
+    DevCtx& dc = ctx->devs[di];
+    if (cudaSetDevice(dc.dev) != cudaSuccess) return fail(SB200_ERR_CUDA, "cudaSetDevice");
+    sb200_keyset::Dev& kd = ks->dev[di];
+    if (cudaMalloc(&kd.tab, tab_bytes) != cudaSuccess || cudaMalloc(&kd.ok, ok_bytes) != cudaSuccess ||
+        cudaMalloc(&tmp[3 * di], scr_bytes) != cudaSuccess)
+      return fail(SB200_ERR_NOMEM, "cudaMalloc keyset");
+    // SB200_DEVICE_PTRS: on the caller's stream, after the work that produced the keys
+    cudaStream_t st = devptrs ? ctx->user_stream : dc.stream[0];
+    const uint32_t* src[2] = {pk, pk2};
+    if (!devptrs)
+      for (int p = 0; p < nt; p++) {
+        if (cudaMalloc(&tmp[3 * di + 1 + p], pt_bytes) != cudaSuccess) return fail(SB200_ERR_NOMEM, "cudaMalloc keyset input");
+        if (cudaMemcpyAsync(tmp[3 * di + 1 + p], src[p], pt_bytes, cudaMemcpyHostToDevice, st) != cudaSuccess)
+          return fail(SB200_ERR_CUDA, "cudaMemcpyAsync keyset input");
+        src[p] = (const uint32_t*)tmp[3 * di + 1 + p];
+      }
+    if (cudaMemsetAsync(kd.ok, 0, ok_bytes, st) != cudaSuccess) return fail(SB200_ERR_CUDA, "cudaMemsetAsync key_ok");
+    const Launcher go{ctx, st};
+    for (int64_t k0 = 0; k0 < n_keys; k0 += batch) {
+      const KsBuild b{kd.tab, kd.ok, src[0], nt == 2 ? src[1] : nullptr, k0, std::min(batch, n_keys - k0), nt,
+                      (flags & SB200_POINTS_AFFINE) != 0, (fq*)tmp[3 * di]};
+      go(k_keyset_build, (unsigned)((b.nk * 32 + TPB - 1) / TPB), TPB, 0, b);
+    }
+    if (cudaGetLastError() != cudaSuccess) return fail(SB200_ERR_CUDA, "k_keyset_build launch");
+  }
+  for (size_t di = 0; di < ndev; di++) {  // the builds of all devices run concurrently
+    DevCtx& dc = ctx->devs[di];
+    if (cudaSetDevice(dc.dev) != cudaSuccess || cudaStreamSynchronize(devptrs ? ctx->user_stream : dc.stream[0]) != cudaSuccess)
+      return fail(SB200_ERR_CUDA, "k_keyset_build");
+  }
+  if (key_ok) {
+    cudaSetDevice(ctx->devs[0].dev);
+    if (cudaMemcpy(key_ok, ks->dev[0].ok, ok_bytes, cudaMemcpyDeviceToHost) != cudaSuccess) return fail(SB200_ERR_CUDA, "key_ok copy");
+  }
+  fail(SB200_OK, "");  // frees the temporaries only
+  ctx->keysets.push_back(ks);
+  *out = ks;
+  return SB200_OK;
+}
+void sb200_keyset_destroy(sb200_keyset* ks) {
+  if (!ks) return;
+  sb200_ctx* ctx = ks->ctx;
+  std::lock_guard<std::mutex> lock(ctx->mu);
+  DeviceGuard guard;
+  ctx->keysets.erase(std::remove(ctx->keysets.begin(), ctx->keysets.end(), ks), ctx->keysets.end());
+  keyset_free(ks);
+}
+int sb200_verify_keyset(sb200_ctx* ctx, const sb200_keyset* ks, int64_t n, uint32_t flags, const uint32_t* key_index,
+                        const uint32_t* sig_u, const uint32_t* sig_R, const uint32_t* sig_R_prime, const uint32_t* msg,
+                        uint32_t* verdicts, uint32_t* c_out) {
+  if (!ctx || !ks) return SB200_ERR_ARG;
+  {  // a keyset of this context that is still alive
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    if (std::find(ctx->keysets.begin(), ctx->keysets.end(), ks) == ctx->keysets.end()) return SB200_ERR_ARG;
+  }
+  const int pw = pt_words(flags);
+  Desc d; d.op = OP_VERIFY_KEYSET; d.flags = flags; d.aux = ks->scheme; d.ks = ks; d.nout = 1; BITMAP(verdicts);
+  int k = 0;  // key index, u, R, (R',) m
+  IN(k, key_index, 1); k++;
+  IN(k, sig_u, 8); k++;
+  IN(k, sig_R, pw); k++;
+  if (ks->scheme == 1) { IN(k, sig_R_prime, pw); k++; }
+  IN(k, msg, 8); k++;
+  d.nin = k;
+  OPT_OUT(0, c_out, 8);
   return run(ctx, n, d);
 }
 int sb200_points_check(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* points, uint32_t* ok_bitmap) {

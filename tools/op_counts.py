@@ -43,7 +43,7 @@ fill(o.sign_double(sk, nonce, m, mul=V.mul)[0])
 cnt = np.zeros(10, np.uint64)
 buf = np.zeros(8, np.uint32)
 
-def measure(fn):
+def measure(fn, lib=lib):
     lib.h_counts_reset(); fn(); lib.h_counts_get(H.ptr(cnt))
     w, mul, sqr, addsub, frm, dot5, dfma = (int(x) for x in cnt[:7])
     return {"imad_wide_per_tuple": w, "fq_mul": mul, "fq_sqr": sqr, "fq_dot5": dot5, "fq_addsub": addsub, "fr_mont_mul": frm, "dfma": dfma}
@@ -89,6 +89,27 @@ nul = np.zeros(24, np.uint32)
 out["verify_witness_single"] = measure(lambda: lib.h_verify_witness(0, H.ptr(H.pt_mont(pk)), H.ptr(nul), H.ptr(H.limbs(u)), H.ptr(H.pt_mont(Rp)), H.ptr(nul), H.ptr(H.mont(m)), 1, 0, H.ptr(tab[0]), H.ptr(tab[1]), H.ptr(rows)))
 out["verify_witness_double"] = measure(lambda: lib.h_verify_witness(1, H.ptr(H.pt_mont(pk)), H.ptr(H.pt_mont(pkp)), H.ptr(H.limbs(ud)), H.ptr(H.pt_mont(Rd)), H.ptr(H.pt_mont(Rdp)), H.ptr(H.mont(m)), 1, 0, H.ptr(tab[0]), H.ptr(tab[1]), H.ptr(rows)))
 out["verify_witness_vargen"] = measure(lambda: lib.h_verify_witness(2, H.ptr(H.pt_mont(pkv)), H.ptr(H.pt_mont(gen)), H.ptr(H.limbs(uvg)), H.ptr(H.pt_mont(Rvg)), H.ptr(nul), H.ptr(H.mont(m)), 1, 0, H.ptr(tab[0]), H.ptr(tab[1]), H.ptr(rows)))
+# verification against a registered key (core.cuh verify_keyset_core, tests/host_keyset.cpp) of valid signatures, affine:
+# the challenge hash, u G by the 16-bit comb (u G' too) or u GEN by the key's 8-bit comb, c PK by the key's 8-bit comb
+sok = os.path.join(ROOT, "build", "host_keyset16.so")
+subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-DSB_COMB_BITS=16", "-include",
+                       os.path.join(ROOT, "tests", "host_shim.h"), "-o", sok, os.path.join(ROOT, "tests", "host_keyset.cpp")])
+klib = ctypes.CDLL(sok)
+H.setup_hades(klib)
+klib.h_verify_keyset.argtypes = [ctypes.c_int, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_uint32] + \
+    [ctypes.c_void_p] * 4 + [ctypes.c_int, ctypes.c_int] + [ctypes.c_void_p] * 3
+def ktabs(*pts):  # the keyset's combs of one key (the build is not counted)
+    t = [np.zeros(32 * 129 * 24, np.uint32) for _ in pts]
+    for x, p in zip(t, pts):
+        klib.h_keyset_table(H.ptr(H.pt_mont(p)), 1, H.ptr(x))
+    return np.concatenate(t)
+kok = np.ones(1, np.uint32)
+ks = [ktabs(pk), ktabs(pk, pkp), ktabs(pkv, gen)]
+kargs = lambda s, uu, R1, R2: (s, H.ptr(ks[s]), 1, H.ptr(kok), 0, H.ptr(H.limbs(uu)), H.ptr(H.pt_mont(R1)), H.ptr(R2), H.ptr(H.mont(m)), 1, 0,
+                               H.ptr(tab[0]), H.ptr(tab[1]), H.ptr(buf))
+out["keyset_verify_single"] = measure(lambda: klib.h_verify_keyset(*kargs(0, u, Rp, nul)), klib)
+out["keyset_verify_double"] = measure(lambda: klib.h_verify_keyset(*kargs(1, ud, Rd, H.pt_mont(Rdp))), klib)
+out["keyset_verify_vargen"] = measure(lambda: klib.h_verify_keyset(*kargs(2, uvg, Rvg, nul)), klib)
 st = np.concatenate([H.mont(x) for x in range(5)])
 out["hades_perm_sparse"] = measure(lambda: lib.h_hades(H.ptr(st), 0))  # the production form: small-integer layers for the default MDS
 out["hades_perm_dense"] = measure(lambda: lib.h_hades(H.ptr(st), 1))
