@@ -200,38 +200,38 @@ SB_HD void blk_red_odd_q(uint32_t* y, uint32_t m, uint32_t t0, uint32_t q3, uint
 }
 
 // ------------------------------------------------------------------------------------------
-// blocks of the dedicated squaring / separated Montgomery reduction
+// blocks of the dedicated squaring and of the schoolbook products / separated Montgomery reduction
 // ------------------------------------------------------------------------------------------
-// acc[0..2N) += a * (b0, b1, .. at 64-bit strides), carry out added to acc[2N] (small-valued limb, cannot overflow)
-SB_HD void blk_mac1c(uint32_t* acc, uint32_t a, uint32_t b0) {
+// acc[0..2N) += a * (b0, b1, .. at 64-bit strides), carry out added to `top` (a limb the caller knows cannot overflow)
+SB_HD void blk_mac1c(uint32_t* acc, uint32_t& top, uint32_t a, uint32_t b0) {
 #if defined(__CUDA_ARCH__)
   asm("mad.lo.cc.u32 %0, %3, %4, %0;\n\t"
       "madc.hi.cc.u32 %1, %3, %4, %1;\n\t"
       "addc.u32 %2, %2, 0;"
-      : "+r"(acc[0]), "+r"(acc[1]), "+r"(acc[2])
+      : "+r"(acc[0]), "+r"(acc[1]), "+r"(top)
       : "r"(a), "r"(b0));
 #else
   SB_COUNT(wide, 1);
-  acc[2] += emu::add_at(acc, 2, 0, (uint64_t)a * b0, 0);
+  top += emu::add_at(acc, 2, 0, (uint64_t)a * b0, 0);
 #endif
 }
-SB_HD void blk_mac2c(uint32_t* acc, uint32_t a, uint32_t b0, uint32_t b1) {
+SB_HD void blk_mac2c(uint32_t* acc, uint32_t& top, uint32_t a, uint32_t b0, uint32_t b1) {
 #if defined(__CUDA_ARCH__)
   asm("mad.lo.cc.u32 %0, %5, %6, %0;\n\t"
       "madc.hi.cc.u32 %1, %5, %6, %1;\n\t"
       "madc.lo.cc.u32 %2, %5, %7, %2;\n\t"
       "madc.hi.cc.u32 %3, %5, %7, %3;\n\t"
       "addc.u32 %4, %4, 0;"
-      : "+r"(acc[0]), "+r"(acc[1]), "+r"(acc[2]), "+r"(acc[3]), "+r"(acc[4])
+      : "+r"(acc[0]), "+r"(acc[1]), "+r"(acc[2]), "+r"(acc[3]), "+r"(top)
       : "r"(a), "r"(b0), "r"(b1));
 #else
   SB_COUNT(wide, 2);
   uint32_t c = emu::add_at(acc, 4, 0, (uint64_t)a * b0, 0);
   c += emu::add_at(acc, 4, 2, (uint64_t)a * b1, 0);
-  acc[4] += c;
+  top += c;
 #endif
 }
-SB_HD void blk_mac3c(uint32_t* acc, uint32_t a, uint32_t b0, uint32_t b1, uint32_t b2) {
+SB_HD void blk_mac3c(uint32_t* acc, uint32_t& top, uint32_t a, uint32_t b0, uint32_t b1, uint32_t b2) {
 #if defined(__CUDA_ARCH__)
   asm("mad.lo.cc.u32 %0, %7, %8, %0;\n\t"
       "madc.hi.cc.u32 %1, %7, %8, %1;\n\t"
@@ -240,47 +240,77 @@ SB_HD void blk_mac3c(uint32_t* acc, uint32_t a, uint32_t b0, uint32_t b1, uint32
       "madc.lo.cc.u32 %4, %7, %10, %4;\n\t"
       "madc.hi.cc.u32 %5, %7, %10, %5;\n\t"
       "addc.u32 %6, %6, 0;"
-      : "+r"(acc[0]), "+r"(acc[1]), "+r"(acc[2]), "+r"(acc[3]), "+r"(acc[4]), "+r"(acc[5]), "+r"(acc[6])
+      : "+r"(acc[0]), "+r"(acc[1]), "+r"(acc[2]), "+r"(acc[3]), "+r"(acc[4]), "+r"(acc[5]), "+r"(top)
       : "r"(a), "r"(b0), "r"(b1), "r"(b2));
 #else
   SB_COUNT(wide, 3);
   uint32_t c = emu::add_at(acc, 6, 0, (uint64_t)a * b0, 0);
   c += emu::add_at(acc, 6, 2, (uint64_t)a * b1, 0);
   c += emu::add_at(acc, 6, 4, (uint64_t)a * b2, 0);
-  acc[6] += c;
+  top += c;
 #endif
 }
-SB_HD void blk_mac4c(uint32_t* acc, uint32_t a, uint32_t b0, uint32_t b1, uint32_t b2, uint32_t b3) {
+SB_HD void blk_mac4c(uint32_t* acc, uint32_t a, uint32_t b0, uint32_t b1, uint32_t b2, uint32_t b3) {  // top = acc[8]
   blk_mac_even(acc, acc[8], a, b0, b1, b2, b3);
 }
 
-// t[0..15] += (a0^2, a1^2, .., a7^2) at 64-bit strides: one chain of 8 wide products (the total fits 16 limbs)
-SB_HD void blk_sqr_diag(uint32_t* t, const uint32_t* a) {
+// acc[0..2N) += a * (b0, b1, .. at 64-bit strides); the caller knows the sum fits (no carry out of acc[2N - 1])
+SB_HD void blk_mac1(uint32_t* acc, uint32_t a, uint32_t b0) {
 #if defined(__CUDA_ARCH__)
-  asm("mad.lo.cc.u32 %0, %16, %16, %0;\n\t"
-      "madc.hi.cc.u32 %1, %16, %16, %1;\n\t"
-      "madc.lo.cc.u32 %2, %17, %17, %2;\n\t"
-      "madc.hi.cc.u32 %3, %17, %17, %3;\n\t"
-      "madc.lo.cc.u32 %4, %18, %18, %4;\n\t"
-      "madc.hi.cc.u32 %5, %18, %18, %5;\n\t"
-      "madc.lo.cc.u32 %6, %19, %19, %6;\n\t"
-      "madc.hi.cc.u32 %7, %19, %19, %7;\n\t"
-      "madc.lo.cc.u32 %8, %20, %20, %8;\n\t"
-      "madc.hi.cc.u32 %9, %20, %20, %9;\n\t"
-      "madc.lo.cc.u32 %10, %21, %21, %10;\n\t"
-      "madc.hi.cc.u32 %11, %21, %21, %11;\n\t"
-      "madc.lo.cc.u32 %12, %22, %22, %12;\n\t"
-      "madc.hi.cc.u32 %13, %22, %22, %13;\n\t"
-      "madc.lo.cc.u32 %14, %23, %23, %14;\n\t"
-      "madc.hi.u32 %15, %23, %23, %15;"
-      : "+r"(t[0]), "+r"(t[1]), "+r"(t[2]), "+r"(t[3]), "+r"(t[4]), "+r"(t[5]), "+r"(t[6]), "+r"(t[7]), "+r"(t[8]),
-        "+r"(t[9]), "+r"(t[10]), "+r"(t[11]), "+r"(t[12]), "+r"(t[13]), "+r"(t[14]), "+r"(t[15])
-      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(a[4]), "r"(a[5]), "r"(a[6]), "r"(a[7]));
+  asm("mad.lo.cc.u32 %0, %2, %3, %0;\n\t"
+      "madc.hi.u32 %1, %2, %3, %1;"
+      : "+r"(acc[0]), "+r"(acc[1])
+      : "r"(a), "r"(b0));
 #else
-  SB_COUNT(wide, 8);
-  uint32_t c = 0;
-  for (int i = 0; i < 8; i++) c += emu::add_at(t, 16, 2 * i, (uint64_t)a[i] * a[i], 0);
-  (void)c;
+  SB_COUNT(wide, 1);
+  emu::add_at(acc, 2, 0, (uint64_t)a * b0, 0);
+#endif
+}
+
+// One Montgomery row of the squaring.  The row adds (m + 1) q with m + 1 = 2^32 - t0 in [1, 2^32] (t0 = the window's limb 0
+// after the fold), so limb 0 always carries exactly 1 and no carry is deferred to the next row.  With q0 = 1 and
+// q1 = 2^32 - 1:  t0 + (m + 1)(q0 + q1 2^32) = (t0 + 1) 2^32 + m 2^64, and m = ~t0 fits 32 bits.  The part of (m + 1) q that
+// does not depend on t0, 2^32 + (q >> 64) 2^64, is left out of every row (fq_sqr_inl feeds the sum over its rows into the
+// window instead); what remains is t0 at limb 1 and m (q2 + 1, q3, .., q7) from limb 2:
+//   x0 += xf;  t0 = x0;  m = ~t0;  x1 += t0 + (carry of the fold);  x[2..7] += m (q2 + 1, q4, q6), carry out into y[7];
+//   y[2..7] += m (q3, q5, q7)  (the window fits 9 limbs: no carry out).
+// Six wide products and four other instructions; m is formed as t0 ^ q1 with q1 in a register (see fq_mul_inl).
+SB_HD void blk_sqr_red_row(uint32_t* x, uint32_t* y, uint32_t xf, uint32_t q1, uint32_t q2p, uint32_t q3, uint32_t q4,
+                           uint32_t q5, uint32_t q6, uint32_t q7) {
+#if defined(__CUDA_ARCH__)
+  asm("{\n\t.reg .u32 m;\n\t"
+      "add.cc.u32 %0, %0, %14;\n\t"
+      "xor.b32 m, %0, %15;\n\t"
+      "addc.cc.u32 %1, %1, %0;\n\t"
+      "madc.lo.cc.u32 %2, m, %16, %2;\n\t"
+      "madc.hi.cc.u32 %3, m, %16, %3;\n\t"
+      "madc.lo.cc.u32 %4, m, %18, %4;\n\t"
+      "madc.hi.cc.u32 %5, m, %18, %5;\n\t"
+      "madc.lo.cc.u32 %6, m, %20, %6;\n\t"
+      "madc.hi.cc.u32 %7, m, %20, %7;\n\t"
+      "addc.u32 %13, %13, 0;\n\t"
+      "mad.lo.cc.u32 %8, m, %17, %8;\n\t"
+      "madc.hi.cc.u32 %9, m, %17, %9;\n\t"
+      "madc.lo.cc.u32 %10, m, %19, %10;\n\t"
+      "madc.hi.cc.u32 %11, m, %19, %11;\n\t"
+      "madc.lo.cc.u32 %12, m, %21, %12;\n\t"
+      "madc.hi.u32 %13, m, %21, %13;\n\t}"
+      : "+r"(x[0]), "+r"(x[1]), "+r"(x[2]), "+r"(x[3]), "+r"(x[4]), "+r"(x[5]), "+r"(x[6]), "+r"(x[7]), "+r"(y[2]),
+        "+r"(y[3]), "+r"(y[4]), "+r"(y[5]), "+r"(y[6]), "+r"(y[7])
+      : "r"(xf), "r"(q1), "r"(q2p), "r"(q3), "r"(q4), "r"(q5), "r"(q6), "r"(q7));
+#else
+  SB_COUNT(wide, 6);
+  uint64_t t = (uint64_t)x[0] + xf;
+  x[0] = (uint32_t)t;
+  const uint32_t m = x[0] ^ q1;
+  uint32_t c = emu::add_at(x, 8, 1, x[0], (uint32_t)(t >> 32));
+  c += emu::add_at(x, 8, 2, (uint64_t)m * q2p, 0);
+  c += emu::add_at(x, 8, 4, (uint64_t)m * q4, 0);
+  c += emu::add_at(x, 8, 6, (uint64_t)m * q6, 0);
+  y[7] += c;
+  emu::add_at(y, 8, 2, (uint64_t)m * q3, 0);
+  emu::add_at(y, 8, 4, (uint64_t)m * q5, 0);
+  emu::add_at(y, 8, 6, (uint64_t)m * q7, 0);
 #endif
 }
 
@@ -686,36 +716,86 @@ SB_HD fq mont_reduce16(const uint32_t* t) {
   return r;
 }
 
-// Dedicated squaring: 28 off-diagonal products (accumulated in an even- and an odd-aligned array so every
-// chain fuses), doubled by a 1-bit funnel shift, plus the 8 diagonal squares in one chain; then the
-// separated reduction.  36 + 56 = 92 wide products instead of 120.
+// Row r < 7 of the square, one limb later than its place (see fq_sqr_inl): a_r times b = (a_r, 2 a_{r+1} mod 2^32,
+// d_{r+2}, .., d_7) with the limbs d_j of 2a (d_{r+1} also holds a_r's top bit, which belongs to a_r * a_r);
+// sum_r a_r b 2^(64 r) = a^2.  Limb j of b lands on window limb j - 1: odd j on X (carry out into Y[7]), even j on Y
+// (carry out into Y[6]; both are limbs the previous shift left holding only a constant).  Row 0 leaves out a_0 * a_0.
+SB_HD void sqr_row(uint32_t* X, uint32_t* Y, const uint32_t* a, const uint32_t* d, int r) {
+  uint32_t b[8];
+#pragma unroll
+  for (int j = 0; j < 8; j++) b[j] = j == r ? a[r] : j == r + 1 ? a[j] << 1 : d[j];
+  const uint32_t ar = a[r];
+  switch ((r | 1) / 2) {  // first odd limb: (r | 1), X pair (r | 1) / 2 .. 3
+    case 0: blk_mac_even(X, Y[7], ar, b[1], b[3], b[5], b[7]); break;
+    case 1: blk_mac3c(X + 2, Y[7], ar, b[3], b[5], b[7]); break;
+    case 2: blk_mac2c(X + 4, Y[7], ar, b[5], b[7]); break;
+    default: blk_mac1c(X + 6, Y[7], ar, b[7]); break;
+  }
+  switch ((r + 1) / 2) {  // first even limb: 2 (r + 1) / 2, 2 at least; Y pair (r + 1) / 2 - 1 .. 2
+    case 0:
+    case 1: blk_mac3c(Y, Y[6], ar, b[2], b[4], b[6]); break;
+    case 2: blk_mac2c(Y + 2, Y[6], ar, b[4], b[6]); break;
+    default: blk_mac1c(Y + 4, Y[6], ar, b[6]); break;
+  }
+}
+
+// Dedicated squaring, a < q: the rows of the square interleaved with Montgomery rows on the 9-limb window of fq_mul_inl
+// (X = even-aligned limb pairs, Y = odd-aligned).  36 + 8 x 6 = 84 wide products; besides them, four instructions per
+// Montgomery row, two carries per row of the square, the limbs of 2a, the final merge and subtraction.
+//  * Row r of the square is added after Montgomery row r, one limb right of its schoolbook place.  Before the shift of
+//    row i >= 1 the window then holds (A (2a - A) + M q) / 2^(32 i) + (part of K, below), with A = a mod 2^(32 i) (rows
+//    0..i-1 of the square) and M = sum_{j <= i} (m_j + 1) 2^(32 j) < 2^(32 (i+1)) (1 + 2^-31): below 2a + 2^32 q (1 + 2^-31)
+//    + 2^257 < 2^288.  At its place, row i (a_i times about 2a) would bring it to 2^32 (2a + q), which does not fit 9 limbs.
+//    Only a_0 * a_0 goes in first: limb 0 sets the first m.
+//  * blk_sqr_red_row leaves the t0-independent part of every row's (m + 1) q out.  Their sum over the 8 rows plus l q
+//    (l < 2^224, which only adds to M), K = SB200_FQ_SQR_K_INIT, has limbs 0..6 zero; it enters the window limb by limb,
+//    limb i + 7 as the constant on the limb that the shift before row i frees (Y[6]).  It adds < 2^257 to the window.
+//  * Result (a^2 + M q) / 2^256 < q^2 / 2^256 + q (1 + 2^-31) < 1.46 q: one conditional subtraction.
 SB_HD fq fq_sqr_inl(const fq& x) {
   SB_COUNT(fq_sqr, 1);
   const uint32_t* a = x.v;
-  uint32_t E[16], O[16];
+  const uint32_t k[16] = SB200_FQ_SQR_K_INIT;
+  uint32_t d[8], X[8], Y[8], xf = 0;
+  d[0] = 0;
 #pragma unroll
-  for (int i = 0; i < 16; i++) E[i] = O[i] = 0;
-  // row i: a_i * a_j for j > i; j - i odd -> odd-aligned array (index = position - 1), even -> even-aligned
-  blk_mac4c(O + 0, a[0], a[1], a[3], a[5], a[7]);
-  blk_mac3c(E + 2, a[0], a[2], a[4], a[6]);
-  blk_mac3c(O + 2, a[1], a[2], a[4], a[6]);
-  blk_mac3c(E + 4, a[1], a[3], a[5], a[7]);
-  blk_mac3c(O + 4, a[2], a[3], a[5], a[7]);
-  blk_mac2c(E + 6, a[2], a[4], a[6]);
-  blk_mac2c(O + 6, a[3], a[4], a[6]);
-  blk_mac2c(E + 8, a[3], a[5], a[7]);
-  blk_mac2c(O + 8, a[4], a[5], a[7]);
-  blk_mac1c(E + 10, a[4], a[6]);
-  blk_mac1c(O + 10, a[5], a[6]);
-  blk_mac1c(E + 12, a[5], a[7]);
-  blk_mac1c(O + 12, a[6], a[7]);
-  uint32_t S[16], T[16];
-  merge_eo16(S, E, O);
-  T[0] = S[0] << 1;
+  for (int j = 1; j < 8; j++) {
+#if defined(__CUDA_ARCH__)
+    d[j] = __funnelshift_l(a[j - 1], a[j], 1);
+#else
+    d[j] = (a[j] << 1) | (a[j - 1] >> 31);
+#endif
+  }
 #pragma unroll
-  for (int i = 1; i < 16; i++) T[i] = (S[i] << 1) | (S[i - 1] >> 31);
-  blk_sqr_diag(T, a);
-  return mont_reduce16(T);
+  for (int i = 0; i < 8; i++) X[i] = Y[i] = 0;
+  Y[6] = k[7];
+  const uint32_t q1 = SB_FQ_MOD(1), q2p = FqP::p(2) + 1u, q3 = SB_FQ_MOD(3), q4 = SB_FQ_MOD(4), q5 = SB_FQ_MOD(5),
+                 q6 = SB_FQ_MOD(6), q7 = SB_FQ_MOD(7);
+  blk_mac1(X, a[0], a[0]);
+#pragma unroll
+  for (int i = 0; i < 8; i++) {
+    if (i > 0) sqr_row(X, Y, a, d, i - 1);
+    blk_sqr_red_row(X, Y, xf, q1, q2p, q3, q4, q5, q6, q7);
+    // divide by 2^32 (limb 0 is t0 + m + 1 = 2^32: its carry is in X[1] already); X[1] is folded in by the next row
+    xf = X[1];
+    uint32_t nx[8], ny[8];
+#pragma unroll
+    for (int j = 0; j < 8; j++) nx[j] = Y[j];
+#pragma unroll
+    for (int j = 0; j < 6; j++) ny[j] = X[j + 2];
+    ny[6] = k[i + 8];
+    ny[7] = 0;
+#pragma unroll
+    for (int j = 0; j < 8; j++) {
+      X[j] = nx[j];
+      Y[j] = ny[j];
+    }
+  }
+  blk_mac1(X + 6, a[7], a[7]);  // row 7, a_7 * a_7 (limb 14 = limb 6 of the result)
+  fq r;
+  const uint32_t s[8] = {xf, Y[0], Y[1], Y[2], Y[3], Y[4], Y[5], Y[6]};
+  add8(r.v, X, s);
+  cond_sub_p<FqP>(r.v);
+  return r;
 }
 
 // ------------------------------------------------------------------------------------------

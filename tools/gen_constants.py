@@ -350,6 +350,14 @@ def main():
     w("#define SB200_8R_INIT %s   // 8 r = the order of the whole curve group (cofactor 8)" % fmt(8 * R))
     w("#define SB200_FQ_ONE_INIT %s   // 2^256 mod q" % fmt(RADIX % Q))
     w("#define SB200_FQ_R2_INIT %s    // 2^512 mod q" % fmt(RADIX * RADIX % Q))
+    # fq_sqr reduces every row with m + 1 = 2^32 - t0 and leaves out the part of (m + 1) q that does not depend on t0,
+    # 2^32 + (q >> 64) 2^64 per row.  It feeds the sum of those parts over its 8 rows into its window instead, as
+    # K = that sum + l q with l < 2^224 chosen so that limbs 0..6 of K are zero (l q only adds l < 2^224 to M).
+    K = sum(((1 << 32) + ((Q >> 64) << 64)) << (32 * i) for i in range(8))
+    K += (-K * pow(Q, -1, 1 << 224)) % (1 << 224) * Q
+    assert K % (1 << 224) == 0 and K >> 480 == 0
+    w("#define SB200_FQ_SQR_K_INIT {%s}   // fq_sqr's row constants (limbs 0..15)"
+      % ", ".join("0x%08xu" % ((K >> (32 * i)) & 0xFFFFFFFF) for i in range(16)))
     w("#define SB200_FR_R2_INIT %s    // 2^512 mod r" % fmt(RADIX * RADIX % R))
     w("#define SB200_FR_NINV 0x%08xu  // -r^-1 mod 2^32" % ((-pow(R, -1, 1 << 32)) % (1 << 32)))
     w("#define SB200_FQ_NINV 0x%08xu  // -q^-1 mod 2^32" % ((-pow(Q, -1, 1 << 32)) % (1 << 32)))
