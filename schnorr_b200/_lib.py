@@ -132,6 +132,13 @@ _KEYSET_PROTOTYPES = {  # every symbol of include/schnorr_b200_keyset.h (verific
     "sb200_keyset_destroy": (None, [vp]),
     "sb200_verify_keyset": (ci, [vp, vp, i64, u32] + [u32p] * 7),
 }
+_KEYSET_LIVE_PROTOTYPES = {  # every symbol of include/schnorr_b200_keyset_live.h (byte-level keysets, live updates)
+    "sb200_verify_keyset_bytes": (ci, [vp, vp, i64, u32] + [u32p] * 5),
+    "sb200_keyset_create_bytes": (ci, [vp, ci, i64, u32, u32p, u32p, ctypes.POINTER(vp)]),
+    "sb200_keyset_update": (ci, [vp, i64, u32] + [u32p] * 4),
+    "sb200_keyset_update_bytes": (ci, [vp, i64, u32] + [u32p] * 3),
+    "sb200_keyset_revoke": (ci, [vp, i64, u32p]),
+}
 del vp, u32p, i64, u32, ci
 EXPORTED_SYMBOLS = list(_PROTOTYPES)  # the symbols of include/schnorr_b200.h
 
@@ -152,7 +159,7 @@ def load_library() -> ctypes.CDLL:
             f"{LIB_PATH} not found: build it with `python -c 'import __graft_entry__ as g; g.build()'` "
             "(nvcc, sm_100a). There is no CPU fallback.")
     lib = ctypes.CDLL(LIB_PATH)
-    for name, (res, args) in {**_PROTOTYPES, **_WITNESS_PROTOTYPES, **_KEYSET_PROTOTYPES}.items():
+    for name, (res, args) in {**_PROTOTYPES, **_WITNESS_PROTOTYPES, **_KEYSET_PROTOTYPES, **_KEYSET_LIVE_PROTOTYPES}.items():
         fn = getattr(lib, name)  # AttributeError if the library does not export a declared symbol
         fn.restype, fn.argtypes = res, args
     _lib = lib
@@ -525,6 +532,11 @@ class Engine:
         pk2 = PK' (scheme 1) or the keys' generators (scheme 2)."""
         return KeySet(self, scheme, pk, pk2, affine)
 
+    def keyset_from_bytes(self, scheme: int, pk_bytes) -> "KeySet":
+        """register n_keys public keys given as their to_bytes() form (include/schnorr_b200_keyset_live.h): 32 B per key
+        for scheme 0, 64 B (pk || pk' or pk || generator) for schemes 1 and 2.  key_ok[k] = the key's from_bytes succeeds."""
+        return KeySet(self, scheme, None, pk_bytes=pk_bytes)
+
     def points_check(self, points, affine=True):
         """ok[n]: point i is on the curve with Z != 0 (what CHECK_POINTS applies inside the verify calls)"""
         n = np.asarray(points).size // self._pw(affine)
@@ -592,17 +604,28 @@ class Engine:
 
 class KeySet:
     """Public keys registered on every device of an Engine (include/schnorr_b200_keyset.h): `key_ok` (bool[n_keys]: every
-    point of the key is on the curve with Z != 0) and `verify`.  Frees its device memory on close() / exit / GC."""
+    point of the key is on the curve with Z != 0, kept current by update and revoke), `verify`, and the calls of
+    include/schnorr_b200_keyset_live.h: `verify_bytes`, `update`, `update_bytes`, `revoke`.  Frees its device memory on
+    close() / exit / GC."""
 
-    def __init__(self, engine: Engine, scheme: int, pk, pk2=None, affine=True):
-        pw = engine._pw(affine)
-        n = np.asarray(pk).size // pw
-        pk = _arr(pk, pw, n, "pk")
-        pk2 = _arr(pk2, pw, n, "pk2") if scheme in (1, 2) else None
-        ok = aligned_empty(((n + 31) // 32 + 1,)); ok[...] = 0
+    KEY_BYTES = (32, 64, 64)  # to_bytes() of PublicKey, PublicKeyDouble, PublicKeyVarGen
+    SIG_BYTES = (64, 96, 64)  # to_bytes() of Signature, SignatureDouble, SignatureVarGen
+
+    def __init__(self, engine: Engine, scheme: int, pk, pk2=None, affine=True, pk_bytes=None):
         h = ctypes.c_void_p()
-        rc = engine._lib.sb200_keyset_create(engine._h, scheme, n, POINTS_AFFINE if affine else POINTS_PROJECTIVE, pk.ctypes.data,
-                                             pk2.ctypes.data if pk2 is not None else None, ok.ctypes.data, ctypes.byref(h))
+        if pk_bytes is not None:
+            b = engine._bytes_arr(pk_bytes, self.KEY_BYTES[scheme], "pk_bytes")
+            n = b.shape[0]
+            ok = aligned_empty(((n + 31) // 32 + 1,)); ok[...] = 0
+            rc = engine._lib.sb200_keyset_create_bytes(engine._h, scheme, n, 0, b.ctypes.data, ok.ctypes.data, ctypes.byref(h))
+        else:
+            pw = engine._pw(affine)
+            n = np.asarray(pk).size // pw
+            pk = _arr(pk, pw, n, "pk")
+            pk2 = _arr(pk2, pw, n, "pk2") if scheme in (1, 2) else None
+            ok = aligned_empty(((n + 31) // 32 + 1,)); ok[...] = 0
+            rc = engine._lib.sb200_keyset_create(engine._h, scheme, n, POINTS_AFFINE if affine else POINTS_PROJECTIVE, pk.ctypes.data,
+                                                 pk2.ctypes.data if pk2 is not None else None, ok.ctypes.data, ctypes.byref(h))
         engine._check(rc, "keyset_create")
         self._engine, self._h, self.scheme, self.n_keys = engine, h, scheme, n
         self.key_ok = engine._unpack_bits(ok, n)
@@ -644,3 +667,65 @@ class KeySet:
                                         c.ctypes.data if want_c else None)
         e._check(rc, "verify_keyset")
         return e._unpack_bits(bm, n), c
+
+    def _open(self, what: str) -> Engine:
+        if not self._h:
+            raise SchnorrB200Error(f"{what}: the keyset is closed")
+        return self._engine
+
+    @staticmethod
+    def _slots(slots) -> np.ndarray:
+        return _arr(np.asarray(slots).astype(np.uint32).reshape(-1), None, 0, "slots")
+
+    def verify_bytes(self, key_index, sig_bytes, msg_bytes):
+        """wire-format signatures (the type's to_bytes()) and 32-byte canonical messages against the keys key_index[i]:
+        (ok[n], invalid[n]).  invalid = the signature's or the message's from_bytes fails; an index >= n_keys, a key that is
+        not key_ok or a revoked slot gives verdict 0 with invalid 0."""
+        e = self._open("verify_bytes")
+        idx = self._slots(key_index)
+        n = idx.size
+        sig, msg = e._bytes_arr(sig_bytes, self.SIG_BYTES[self.scheme], "sig"), e._bytes_arr(msg_bytes, 32, "msg")
+        if sig.shape[0] != n or msg.shape[0] != n:
+            raise SchnorrB200Error(f"verify_bytes: {n} key indices, {sig.shape[0]} signatures, {msg.shape[0]} messages")
+        bm = aligned_empty(((n + 31) // 32,)); bm[...] = 0
+        inv = aligned_empty(((n + 31) // 32,)); inv[...] = 0
+        rc = e._lib.sb200_verify_keyset_bytes(e._h, self._h, n, 0, idx.ctypes.data, sig.ctypes.data, msg.ctypes.data,
+                                              bm.ctypes.data, inv.ctypes.data)
+        e._check(rc, "verify_keyset_bytes")
+        return e._unpack_bits(bm, n), e._unpack_bits(inv, n)
+
+    def _updated(self, rc: int, what: str, slots: np.ndarray, ok: np.ndarray) -> np.ndarray:
+        self._engine._check(rc, what)
+        new = self._engine._unpack_bits(ok, slots.size)
+        self.key_ok[slots] = new
+        return new
+
+    def update(self, slots, pk, pk2=None, affine=True) -> np.ndarray:
+        """rebuild the distinct slots `slots` in place with m new keys (layout of the constructor): the new key_ok[m]"""
+        e = self._open("update")
+        s = self._slots(slots)
+        m, pw = s.size, e._pw(affine)
+        pk = _arr(pk, pw, m, "pk")
+        pk2 = _arr(pk2, pw, m, "pk2") if self.scheme in (1, 2) else None
+        ok = aligned_empty(((m + 31) // 32 + 1,)); ok[...] = 0
+        rc = e._lib.sb200_keyset_update(self._h, m, POINTS_AFFINE if affine else POINTS_PROJECTIVE, s.ctypes.data, pk.ctypes.data,
+                                        pk2.ctypes.data if pk2 is not None else None, ok.ctypes.data)
+        return self._updated(rc, "keyset_update", s, ok)
+
+    def update_bytes(self, slots, pk_bytes) -> np.ndarray:
+        """update from the keys' to_bytes() form: the new key_ok[m] (False where a key does not decode)"""
+        e = self._open("update_bytes")
+        s = self._slots(slots)
+        b = e._bytes_arr(pk_bytes, self.KEY_BYTES[self.scheme], "pk_bytes")
+        if b.shape[0] != s.size:
+            raise SchnorrB200Error(f"update_bytes: {s.size} slots, {b.shape[0]} keys")
+        ok = aligned_empty(((s.size + 31) // 32 + 1,)); ok[...] = 0
+        rc = e._lib.sb200_keyset_update_bytes(self._h, s.size, 0, s.ctypes.data, b.ctypes.data, ok.ctypes.data)
+        return self._updated(rc, "keyset_update_bytes", s, ok)
+
+    def revoke(self, slots) -> None:
+        """clear the key_ok bits of the distinct slots `slots`: tuples naming them verify to False until an update"""
+        e = self._open("revoke")
+        s = self._slots(slots)
+        e._check(e._lib.sb200_keyset_revoke(self._h, s.size, s.ctypes.data), "keyset_revoke")
+        self.key_ok[s] = False

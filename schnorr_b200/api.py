@@ -565,7 +565,9 @@ class PublicKeySet:
     device (include/schnorr_b200_keyset.h), for callers that verify many signatures of the same keys: each key gets
     fixed-base tables, so a verification no longer multiplies by the key as a fresh point.  Not in the reference: an
     addition of this library.  `verify_batch(indices, sigs, msgs)` returns what the type's
-    `verify_batch([keys[i] for i in indices], sigs, msgs)` returns (a key not on the curve verifies nothing)."""
+    `verify_batch([keys[i] for i in indices], sigs, msgs)` returns (a key not on the curve verifies nothing).
+    `verify_batch_bytes` takes the signatures and messages as received bytes; `replace` and `remove` change single keys
+    of the live set in place (include/schnorr_b200_keyset_live.h)."""
 
     _SCHEMES = {PublicKey: 0, PublicKeyDouble: 1, PublicKeyVarGen: 2}
 
@@ -596,10 +598,39 @@ class PublicKeySet:
         self.close()
 
     def verify_batch(self, indices: Sequence[int], sigs: Sequence, msgs: Sequence[int]) -> np.ndarray:
-        idx = np.asarray(indices, dtype=np.int64).reshape(-1)
-        if idx.size and (idx.min() < 0 or idx.max() >= len(self.keys)):
-            raise IndexError("PublicKeySet.verify_batch: key index out of range")
+        idx = self._indices(indices, "verify_batch")
         Rp = _points([s._Rp for s in sigs]) if self.scheme == 1 else None
         ok, _ = self._ks.verify(idx.astype(np.uint32), _scalars([s._u for s in sigs]), _points([s._R for s in sigs]), _fqs(msgs),
                                 Rp=Rp, affine=False, want_c=False)
         return ok
+
+    def _indices(self, indices: Sequence[int], what: str) -> np.ndarray:
+        idx = np.asarray(indices, dtype=np.int64).reshape(-1)
+        if idx.size and (idx.min() < 0 or idx.max() >= len(self.keys)):
+            raise IndexError(f"PublicKeySet.{what}: key index out of range")
+        return idx
+
+    def verify_batch_bytes(self, indices: Sequence[int], sigs: Sequence[bytes], msgs: Sequence[bytes]) -> Tuple[np.ndarray, np.ndarray]:
+        """signatures as `Signature*::to_bytes()` and messages as 32 canonical bytes, decoded on the device: (ok, invalid),
+        invalid[i] = `Signature*::from_bytes` or `BlsScalar::from_bytes` of tuple i fails (its verdict is False)"""
+        idx = self._indices(indices, "verify_batch_bytes")
+        return self._ks.verify_bytes(idx.astype(np.uint32), b"".join(sigs), b"".join(msgs))
+
+    def replace(self, indices: Sequence[int], keys: Sequence) -> None:
+        """key indices[j] becomes keys[j] (same type as the set's keys); a removed index is registered again"""
+        idx = self._indices(indices, "replace")
+        keys = list(keys)
+        if len(keys) != idx.size or any(type(k) is not type(self.keys[0]) for k in keys):
+            raise TypeError(f"PublicKeySet.replace: {idx.size} keys of type {type(self.keys[0]).__name__}")
+        pk2 = None
+        if self.scheme == 1:
+            pk2 = _points([k._pp for k in keys])
+        elif self.scheme == 2:
+            pk2 = _points([k._g for k in keys])
+        self._ks.update(idx, _points([k._p for k in keys]), pk2, affine=False)
+        for i, k in zip(idx, keys):
+            self.keys[i] = k
+
+    def remove(self, indices: Sequence[int]) -> None:
+        """later verifications of these indices return False (until `replace` registers a key there again)"""
+        self._ks.revoke(self._indices(indices, "remove"))

@@ -22,6 +22,7 @@
 #include "../../include/schnorr_b200.h"
 #include "../../include/schnorr_b200_witness.h"
 #include "../../include/schnorr_b200_keyset.h"
+#include "../../include/schnorr_b200_keyset_live.h"
 #include "wire.cuh"
 #include "rng.cuh"
 #include "params_host.cuh"
@@ -68,7 +69,8 @@ enum Op : int {
   OP_CHALLENGE_DOUBLE, OP_VERIFY_DOUBLE_EC, OP_CHALLENGE_VARGEN, OP_VERIFY_VARGEN_EC, OP_POINTS_CHECK, OP_DBG_VERIFY_EC,
   OP_DECODE_VERIFY, OP_WITNESS, OP_DBG_LAT3,
   OP_STDRNG, OP_SIGN_STDRNG, OP_SIGN_DOUBLE_STDRNG, OP_SIGN_VARGEN_STDRNG,
-  OP_VERIFY_WITNESS, OP_VERIFY_WITNESS_BYTES, OP_VERIFY_KEYSET
+  OP_VERIFY_WITNESS, OP_VERIFY_WITNESS_BYTES, OP_VERIFY_KEYSET,
+  OP_DECODE_KEYSET, OP_VERIFY_KEYSET_BYTES, OP_DECODE_KEYS
 };
 static_assert(OP_VERIFY_WITNESS == 37, "min_ctas names the op by number");
 
@@ -287,6 +289,51 @@ __global__ void __launch_bounds__(TPB, min_ctas(OP)) k_run(const KArgs a) {
     }
     unsigned inv = __ballot_sync(0xffffffffu, !ok && active);
     if ((threadIdx.x & 31) == 0 && active) a.bitmap[i >> 5] = inv;
+    return;
+  }
+  // First kernel of sb200_verify_keyset_bytes: the signature's and the message's from_bytes as in OP_DECODE_VERIFY, into the
+  // rows k_verify_keyset reads (key index, u, R, (R',) m), and the invalid bitmap.  The key index is forwarded, or replaced
+  // by UINT32_MAX where a from_bytes fails: never below n_keys (<= 2^32 - 1), so the unchanged keyset kernel gives verdict 0.
+  // aux = scheme.  in: key index, sig bytes (64 | 96 | 64 B), msg32.
+  if (OP == OP_DECODE_KEYSET) {
+    const int nr = a.aux == 1 ? 2 : 1;
+    bool ok = true;
+#pragma unroll 1
+    for (int k = 0; k < nr; k++) {
+      uint32_t b[8];
+      fq u, v;
+      ldg_scalar(a.in[1] + i * (8 + 8 * nr) + 8 + 8 * k, b);
+      ok &= point_decompress(b, u, v);
+      if (active) stg_point(a.dec[2 + k], i, u, v);
+    }
+    uint32_t us[8], mb[8];
+    fq m;
+    ldg_scalar(a.in[1] + i * (8 + 8 * nr), us);
+    ldg_scalar(a.in[2] + i * 8, mb);
+    ok &= scalar_lt_r(us);
+    ok &= msg_from_bytes(mb, m);
+    const uint32_t key = __ldg(a.in[0] + i);
+    if (active) {
+      a.dec[0][i] = ok ? key : 0xffffffffu;
+      stg8(a.dec[1] + i * 8, us);
+      stg8(a.dec[2 + nr] + i * 8, m.v);
+    }
+    unsigned inv = __ballot_sync(0xffffffffu, !ok && active);
+    if ((threadIdx.x & 31) == 0 && active) a.bitmap[i >> 5] = inv;
+    return;
+  }
+  // Keys in their to_bytes() form (sb200_keyset_create_bytes, sb200_keyset_update_bytes) -> affine points for the table
+  // build.  aux = points per key; in: 32 B per point -> dec[0..aux).  A point whose from_bytes fails is stored as (0, 0),
+  // which is off the curve: the build records the key as malformed (key_ok bit clear).
+  if (OP == OP_DECODE_KEYS) {
+#pragma unroll 1
+    for (int k = 0; k < a.aux; k++) {
+      uint32_t b[8];
+      fq u, v;
+      ldg_scalar(a.in[0] + i * 8 * a.aux + 8 * k, b);
+      const bool ok = point_decompress(b, u, v);
+      if (active) stg_point(a.dec[k], i, ok ? u : fq_zero(), ok ? v : fq_zero());
+    }
     return;
   }
 
@@ -925,6 +972,36 @@ __global__ void __launch_bounds__(TPB) k_keyset_build(const KsBuild b) {
   }
   if (lane == 0 && well) atomicOr(b.ok + (k >> 5), 1u << (k & 31));
 }
+// The slot-indexed build of an update (include/schnorr_b200_keyset_live.h): warp w rebuilds slot slots[key0 + w] from key row
+// key0 + w of pk / pk2, in place, and sets or clears the slot's key_ok bit -- an update may write a malformed key over a good
+// one.  The slots of one update are distinct, so no two warps write the same table.
+__global__ void __launch_bounds__(TPB) k_keyset_update(const KsBuild b, const uint32_t* slots) {
+  const int64_t t = (int64_t)blockIdx.x * TPB + threadIdx.x, w = t >> 5;
+  const int lane = threadIdx.x & 31;
+  if (w >= b.nk) return;  // warp-uniform
+  const int64_t j = b.key0 + w, k = __ldg(slots + j);
+  fq* z = b.scratch + (size_t)t * 2 * (KS_ENTRIES - 1);
+  bool well = true;
+#pragma unroll 1
+  for (int p = 0; p < b.nt; p++) {
+    const point_in P = ldg_point(p ? b.pk2 : b.pk, j, b.aff);
+    well &= point_well_formed(P);
+    keyset_build_window(point_to_ext(P), lane, b.tab + ((size_t)k * b.nt + p) * KS_TABLE_WORDS + (size_t)lane * KS_ENTRIES * 24, z,
+                        z + (KS_ENTRIES - 1));
+  }
+  if (lane == 0) {
+    const uint32_t bit = 1u << (k & 31);
+    if (well) atomicOr(b.ok + (k >> 5), bit);
+    else atomicAnd(b.ok + (k >> 5), ~bit);
+  }
+}
+// sb200_keyset_revoke: clears the key_ok bits of slots[0..m); no table is touched
+__global__ void __launch_bounds__(TPB) k_keyset_revoke(uint32_t* ok, const uint32_t* slots, int64_t m) {
+  const int64_t j = (int64_t)blockIdx.x * TPB + threadIdx.x;
+  if (j >= m) return;
+  const uint32_t k = slots[j];
+  atomicAnd(ok + (k >> 5), ~(1u << (k & 31)));
+}
 
 // ------------------------------------------------------------------------------------------------
 // host side
@@ -982,6 +1059,11 @@ struct DevParams {
 };
 std::mutex g_params_mu;
 std::map<int, DevParams> g_dev_params;
+
+// Every live keyset of the process: the calls that take a keyset without its context (sb200_keyset_update*, _revoke) look
+// a handle up here before they dereference it.
+std::mutex g_keysets_mu;
+std::vector<const sb200_keyset*> g_keysets;
 
 uint64_t fnv1a(const void* p, size_t n) {
   const uint8_t* b = (const uint8_t*)p;
@@ -1042,8 +1124,9 @@ namespace {
 // challenge kernel, then curve kernel, the challenges through c_out or scratch.  VERIFY_BYTES: decode kernel, then VERIFY
 // on the decoded rows.  SIGN_STDRNG: the nonces drawn into scratch, then the scheme's sign op.  DBG_VERIFY_EC: the curve
 // kernel alone, on the caller's challenges.  WITNESS_BYTES: decode kernel, then `kernel` on the decoded rows.  KEYSET:
-// k_verify_keyset, one tuple per thread, with the keyset's tables of the launching device.
-enum Form : uint8_t { INTERNAL, ONE, FIXED, VERIFY, VERIFY_BYTES, SIGN_STDRNG, DBG_VERIFY_EC, WITNESS_BYTES, KEYSET };
+// k_verify_keyset, one tuple per thread, with the keyset's tables of the launching device.  KEYSET_BYTES: the keyset decode
+// kernel, then KEYSET on the decoded rows.
+enum Form : uint8_t { INTERNAL, ONE, FIXED, VERIFY, VERIFY_BYTES, SIGN_STDRNG, DBG_VERIFY_EC, WITNESS_BYTES, KEYSET, KEYSET_BYTES };
 using KFn = void (*)(KArgs);
 struct OpInfo {
   Form form;
@@ -1056,12 +1139,13 @@ struct OpInfo {
   int scratch_arrays;   // challenges or nonces, and the decoded rows (points 64 B, u and m 32 B) and invalid bitmap
 };
 constexpr OpInfo row(Form form, uint32_t flags = 0, int scheme = 0, KFn kernel = nullptr, KFn ct = nullptr) {
-  const bool decode = form == VERIFY_BYTES || form == WITNESS_BYTES;
+  const bool decode = form == VERIFY_BYTES || form == WITNESS_BYTES, ks = form == KEYSET_BYTES;
   const unsigned points = scheme == 0 ? 2 : scheme == 1 ? 4 : 3, rows = decode ? 64 * points + 64 : 0;
+  const unsigned sig_points = scheme == 1 ? 2 : 1;  // KEYSET_BYTES rows: key index 4 B, u 32 B, R (R') 64 B each, m 32 B
   const bool handover = form == VERIFY || form == VERIFY_BYTES || form == SIGN_STDRNG;  // + 32 B: the challenge row
   return {form, flags, scheme, kernel, ct, ct ? (size_t)(scheme == 1 ? 2 : 1) * CT_TABLE_WORDS * 4 : 0,
-          decode ? (uint32_t)SB200_POINTS_AFFINE : 0u, (handover ? 32u : 0u) + rows,
-          (handover ? 1 : 0) + (rows ? (int)points + 3 : 0)};
+          decode || ks ? (uint32_t)SB200_POINTS_AFFINE : 0u, (handover ? 32u : 0u) + rows + (ks ? 68 + 64 * sig_points : 0u),
+          (handover ? 1 : 0) + (rows ? (int)points + 3 : 0) + (ks ? (int)sig_points + 3 : 0)};
 }
 constexpr uint32_t D = SB200_DEVICE_PTRS, AD = SB200_POINTS_AFFINE | D, CHK = AD | SB200_CHECK_POINTS;
 constexpr uint32_t OBL = AD | SB200_SIGN_OBLIVIOUS, DUAL = SB_VERIFY_WS ? SB200_VERIFY_DUAL_PIPE : 0;
@@ -1115,8 +1199,11 @@ constexpr OpInfo OPS[] = {
     row(ONE, CHK, 0, k_run<OP_VERIFY_WITNESS>),     // the scheme is the call's aux
     row(WITNESS_BYTES, D, 1, k_run<OP_VERIFY_WITNESS>),  // scheme 1: scratch for the widest decoded rows; the call's scheme is its aux
     row(KEYSET, CHK),                               // OP_VERIFY_KEYSET: the keyset's scheme is the call's aux
+    row(INTERNAL),                                  // OP_DECODE_KEYSET
+    row(KEYSET_BYTES, D, 1),  // OP_VERIFY_KEYSET_BYTES: scratch for the widest decoded rows; the keyset's scheme is the call's aux
+    row(INTERNAL),                                  // OP_DECODE_KEYS: launched by the keyset builds
 };
-static_assert(sizeof(OPS) / sizeof(OPS[0]) == OP_VERIFY_KEYSET + 1, "one row per Op");
+static_assert(sizeof(OPS) / sizeof(OPS[0]) == OP_DECODE_KEYS + 1, "one row per Op");
 
 // ---- launches ---------------------------------------------------------------------------------------------------------
 struct Launcher {  // issues kernels on one stream and counts them (sb200_launch_count)
@@ -1207,6 +1294,21 @@ int launch(sb200_ctx* ctx, Op op, const KArgs& a, cudaStream_t st, const KsArgs&
     case KEYSET:
       go(k_verify_keyset, grid, TPB, 0, a, ks);
       break;
+    case KEYSET_BYTES: {  // decode kernel -> k_verify_keyset, the decoded rows in a.scratch, `invalid` in out[0]
+      const int nr = a.aux == 1 ? 2 : 1, narr = nr + 3;  // key index, u, R, (R',) m
+      uint8_t* p = a.scratch;
+      auto carve = [&](size_t bytes) { uint8_t* r = p; p += (bytes + 63) & ~(size_t)63; return (uint32_t*)r; };
+      KArgs dk = a, v = a;
+      for (int k = 0; k < narr; k++) {
+        dk.dec[k] = carve((size_t)a.n * (k == 0 ? 4 : (k == 1 || k == narr - 1) ? 32 : 64));
+        v.in[k] = dk.dec[k];
+      }
+      dk.bitmap = a.out[0] ? a.out[0] : carve((size_t)((a.n + 31) / 32) * 4);
+      for (int k = 0; k < MAX_OUT; k++) v.out[k] = nullptr;  // no c_out
+      go(k_run<OP_DECODE_KEYSET>, grid, TPB, 0, dk);
+      go(k_verify_keyset, grid, TPB, 0, v, ks);
+      break;
+    }
     case DBG_VERIFY_EC: {  // in: pk, u, R, c -> bitmap: the production curve kernel, in the form the batch size picks,
                            // fed the caller's challenges where the challenge kernel would have written them
       KArgs v = a;
@@ -1510,7 +1612,164 @@ void keyset_free(sb200_keyset* ks) {
     if (ks->dev[di].tab) cudaFree(ks->dev[di].tab);
     if (ks->dev[di].ok) cudaFree(ks->dev[di].ok);
   }
+  {
+    std::lock_guard<std::mutex> l(g_keysets_mu);
+    g_keysets.erase(std::remove(g_keysets.begin(), g_keysets.end(), ks), g_keysets.end());
+  }
   delete ks;
+}
+
+// The table builds of a keyset.  Key j in [0, nk) -- limbs pk / pk2 in the layout of `flags`, or with pk_bytes its to_bytes()
+// form, decoded on the device first (OP_DECODE_KEYS) -- goes to slot j when slots == nullptr (creation: the tables and the
+// key_ok bitmap are allocated here, k_keyset_build) or to slot slots[j] (an update: those tables are rebuilt in place,
+// k_keyset_update).  Every device of the context builds its copy; an update first waits for the context's SB200_DEVICE_PTRS
+// work, so that a verification enqueued before it reads the old keys.  Nothing is launched before every allocation has
+// succeeded, and the call returns when every device has finished.  key_ok (nullable, host): bit j = the new key_ok bit of
+// key j.  The caller holds ctx->mu.
+int keyset_build(sb200_keyset* ks, int64_t nk, uint32_t flags, const uint32_t* slots, const uint32_t* pk, const uint32_t* pk2,
+                 const uint8_t* pk_bytes, uint32_t* key_ok) {
+  sb200_ctx* ctx = ks->ctx;
+  const int nt = ks->scheme == 0 ? 1 : 2;
+  const bool devptrs = (flags & SB200_DEVICE_PTRS) != 0, create = slots == nullptr;
+  const size_t ndev = ctx->devs.size(), ok_bytes = (size_t)((ks->n_keys + 31) / 32) * 4;
+  const int64_t batch = std::min<int64_t>(nk, KS_BUILD_KEYS);
+  // per device: [0] build scratch, [1] [2] device copies of the host inputs (pk, pk2 or the key bytes), [3] [4] decoded keys,
+  // [5] the slots
+  const size_t bytes[6] = {(size_t)batch * 32 * 2 * (KS_ENTRIES - 1) * sizeof(fq),
+                           pk_bytes ? (size_t)nk * nt * 32 : (size_t)nk * pt_words(flags) * 4,
+                           pk_bytes || nt == 1 ? 0 : (size_t)nk * pt_words(flags) * 4,
+                           pk_bytes ? (size_t)nk * 64 : 0,
+                           pk_bytes && nt == 2 ? (size_t)nk * 64 : 0,
+                           create ? 0 : (size_t)nk * 4};
+  std::vector<uint8_t*> tmp(6 * ndev, nullptr);
+  auto finish = [&](int code, const char* what) {
+    for (size_t di = 0; di < ndev; di++) {
+      cudaSetDevice(ctx->devs[di].dev);
+      cudaStreamSynchronize(devptrs ? ctx->user_stream : ctx->devs[di].stream[0]);
+      for (int k = 0; k < 6; k++)
+        if (tmp[6 * di + k]) cudaFree(tmp[6 * di + k]);
+    }
+    if (code != SB200_OK) {
+      cudaGetLastError();  // a failed allocation is not the next call's error
+      ctx->set_err(what);
+    }
+    return code;
+  };
+  for (size_t di = 0; di < ndev; di++) {
+    if (cudaSetDevice(ctx->devs[di].dev) != cudaSuccess) return finish(SB200_ERR_CUDA, "cudaSetDevice");
+    sb200_keyset::Dev& kd = ks->dev[di];
+    if (create && (cudaMalloc(&kd.tab, (size_t)ks->n_keys * nt * KS_TABLE_WORDS * 4) != cudaSuccess ||
+                   cudaMalloc(&kd.ok, ok_bytes) != cudaSuccess))
+      return finish(SB200_ERR_NOMEM, "cudaMalloc keyset");
+    for (int k = 0; k < 6; k++)
+      if (bytes[k] && !(devptrs && (k == 1 || k == 2)) && cudaMalloc(&tmp[6 * di + k], bytes[k]) != cudaSuccess)
+        return finish(SB200_ERR_NOMEM, "cudaMalloc keyset scratch");
+  }
+  for (size_t di = 0; di < ndev; di++) {
+    DevCtx& dc = ctx->devs[di];
+    sb200_keyset::Dev& kd = ks->dev[di];
+    uint8_t** t = &tmp[6 * di];
+    if (cudaSetDevice(dc.dev) != cudaSuccess) return finish(SB200_ERR_CUDA, "cudaSetDevice");
+    // SB200_DEVICE_PTRS: on the caller's stream, after the work that produced the keys
+    cudaStream_t st = devptrs ? ctx->user_stream : dc.stream[0];
+    if (!create && dc.user_ev_valid && cudaStreamWaitEvent(st, dc.user_ev, 0) != cudaSuccess)
+      return finish(SB200_ERR_CUDA, "cudaStreamWaitEvent");
+    if (create && cudaMemsetAsync(kd.ok, 0, ok_bytes, st) != cudaSuccess) return finish(SB200_ERR_CUDA, "cudaMemsetAsync key_ok");
+    const void* src[2] = {pk_bytes ? (const void*)pk_bytes : pk, pk2};
+    for (int k = 0; k < 2; k++) {
+      if (devptrs || !bytes[1 + k]) continue;
+      if (cudaMemcpyAsync(t[1 + k], src[k], bytes[1 + k], cudaMemcpyHostToDevice, st) != cudaSuccess)
+        return finish(SB200_ERR_CUDA, "cudaMemcpyAsync keyset input");
+      src[k] = t[1 + k];
+    }
+    if (!create && cudaMemcpyAsync(t[5], slots, bytes[5], cudaMemcpyHostToDevice, st) != cudaSuccess)
+      return finish(SB200_ERR_CUDA, "cudaMemcpyAsync slots");
+    const Launcher go{ctx, st};
+    if (pk_bytes) {
+      KArgs a{};
+      a.n = nk; a.aux = nt; a.in[0] = (const uint32_t*)src[0]; a.dec[0] = (uint32_t*)t[3]; a.dec[1] = (uint32_t*)t[4];
+      go(k_run<OP_DECODE_KEYS>, (unsigned)((nk + TPB - 1) / TPB), TPB, 0, a);
+      src[0] = t[3]; src[1] = t[4];
+    }
+    const bool aff = pk_bytes || (flags & SB200_POINTS_AFFINE);
+    for (int64_t k0 = 0; k0 < nk; k0 += batch) {
+      const KsBuild b{kd.tab, kd.ok, (const uint32_t*)src[0], nt == 2 ? (const uint32_t*)src[1] : nullptr, k0,
+                      std::min(batch, nk - k0), nt, aff, (fq*)t[0]};
+      const unsigned grid = (unsigned)((b.nk * 32 + TPB - 1) / TPB);
+      if (create) go(k_keyset_build, grid, TPB, 0, b);
+      else go(k_keyset_update, grid, TPB, 0, b, (const uint32_t*)t[5]);
+    }
+    if (cudaGetLastError() != cudaSuccess) return finish(SB200_ERR_CUDA, "keyset build launch");
+  }
+  for (size_t di = 0; di < ndev; di++) {  // the builds of all devices run concurrently
+    DevCtx& dc = ctx->devs[di];
+    if (cudaSetDevice(dc.dev) != cudaSuccess || cudaStreamSynchronize(devptrs ? ctx->user_stream : dc.stream[0]) != cudaSuccess)
+      return finish(SB200_ERR_CUDA, "keyset build");
+  }
+  if (key_ok) {
+    cudaSetDevice(ctx->devs[0].dev);
+    std::vector<uint32_t> all(create ? 0 : ok_bytes / 4);
+    if (cudaMemcpy(create ? key_ok : all.data(), ks->dev[0].ok, ok_bytes, cudaMemcpyDeviceToHost) != cudaSuccess)
+      return finish(SB200_ERR_CUDA, "key_ok copy");
+    if (!create) {  // gathered: bit j of key_ok = bit slots[j] of the keyset's bitmap
+      memset(key_ok, 0, (size_t)((nk + 31) / 32) * 4);
+      for (int64_t j = 0; j < nk; j++)
+        if (all[slots[j] >> 5] >> (slots[j] & 31) & 1u) key_ok[j >> 5] |= 1u << (j & 31);
+    }
+  }
+  return finish(SB200_OK, "");
+}
+
+// ks's context if ks is a live keyset, else nullptr (a destroyed handle is not dereferenced)
+sb200_ctx* live_keyset_ctx(const sb200_keyset* ks) {
+  std::lock_guard<std::mutex> l(g_keysets_mu);
+  return std::find(g_keysets.begin(), g_keysets.end(), ks) != g_keysets.end() ? ks->ctx : nullptr;
+}
+// ks is alive and belongs to ctx; the caller holds ctx->mu
+bool keyset_of(const sb200_ctx* ctx, const sb200_keyset* ks) {
+  return std::find(ctx->keysets.begin(), ctx->keysets.end(), ks) != ctx->keysets.end();
+}
+// slots[0..m) are distinct and below the keyset's n_keys
+bool slots_valid(const sb200_keyset* ks, int64_t m, const uint32_t* slots) {
+  std::vector<uint32_t> s(slots, slots + m);
+  std::sort(s.begin(), s.end());
+  return std::adjacent_find(s.begin(), s.end()) == s.end() && (int64_t)s.back() < ks->n_keys;
+}
+
+int keyset_create(sb200_ctx* ctx, int scheme, int64_t n_keys, uint32_t flags, const uint32_t* pk, const uint32_t* pk2,
+                  const uint8_t* pk_bytes, uint32_t* key_ok, sb200_keyset** out) {
+  std::lock_guard<std::mutex> lock(ctx->mu);
+  ctx->set_err("");
+  DeviceGuard guard;
+  sb200_keyset* ks = new sb200_keyset{ctx, scheme, n_keys, std::vector<sb200_keyset::Dev>(ctx->devs.size())};
+  const int rc = keyset_build(ks, n_keys, flags, nullptr, pk, pk2, pk_bytes, key_ok);
+  if (rc != SB200_OK) {
+    keyset_free(ks);
+    return rc;
+  }
+  ctx->keysets.push_back(ks);
+  {
+    std::lock_guard<std::mutex> l(g_keysets_mu);
+    g_keysets.push_back(ks);
+  }
+  *out = ks;
+  return SB200_OK;
+}
+
+// sb200_keyset_update / _update_bytes: the host-side checks, then the slot-indexed build
+int keyset_update(sb200_keyset* ks, int64_t m, uint32_t flags, uint32_t allowed, const uint32_t* slots, const uint32_t* pk,
+                  const uint32_t* pk2, const uint8_t* pk_bytes, uint32_t* key_ok) {
+  sb200_ctx* ctx = live_keyset_ctx(ks);
+  if (!ctx || m < 0 || (flags & ~allowed) || !slots || ((uintptr_t)slots & 15)) return SB200_ERR_ARG;
+  const auto bad = [](const void* p) { return !p || ((uintptr_t)p & 15); };
+  if (allowed & SB200_POINTS_AFFINE ? bad(pk) || (ks->scheme != 0 && bad(pk2)) : bad(pk_bytes)) return SB200_ERR_ARG;
+  if ((flags & SB200_DEVICE_PTRS) && ctx->devs.size() != 1) return SB200_ERR_ARG;
+  if (m == 0) return SB200_OK;
+  std::lock_guard<std::mutex> lock(ctx->mu);
+  if (!keyset_of(ctx, ks) || !slots_valid(ks, m, slots)) return SB200_ERR_ARG;
+  ctx->set_err("");
+  DeviceGuard guard;
+  return keyset_build(ks, m, flags, slots, pk, pk2, pk_bytes, key_ok);
 }
 
 // parameters -> validated, derived, self-checked tables.  Host only.
@@ -1881,74 +2140,12 @@ int sb200_keyset_create(sb200_ctx* ctx, int scheme, int64_t n_keys, uint32_t fla
                         uint32_t* key_ok, sb200_keyset** out) {
   if (out) *out = nullptr;
   const int nt = scheme == 0 ? 1 : 2;
-  const bool devptrs = (flags & SB200_DEVICE_PTRS) != 0;
   if (!ctx || !out || scheme < 0 || scheme > 2 || n_keys < 1 || n_keys > (int64_t)UINT32_MAX ||
       (flags & ~(SB200_POINTS_AFFINE | SB200_DEVICE_PTRS)))
     return SB200_ERR_ARG;
   if (!pk || ((uintptr_t)pk & 15) || (nt == 2 && (!pk2 || ((uintptr_t)pk2 & 15)))) return SB200_ERR_ARG;
-  if (devptrs && ctx->devs.size() != 1) return SB200_ERR_ARG;
-  std::lock_guard<std::mutex> lock(ctx->mu);
-  ctx->set_err("");
-  DeviceGuard guard;
-  const size_t ndev = ctx->devs.size(), pt_bytes = (size_t)n_keys * pt_words(flags) * 4;
-  const size_t tab_bytes = (size_t)n_keys * nt * KS_TABLE_WORDS * 4, ok_bytes = (size_t)((n_keys + 31) / 32) * 4;
-  const int64_t batch = std::min<int64_t>(n_keys, KS_BUILD_KEYS);
-  const size_t scr_bytes = (size_t)batch * 32 * 2 * (KS_ENTRIES - 1) * sizeof(fq);
-  sb200_keyset* ks = new sb200_keyset{ctx, scheme, n_keys, std::vector<sb200_keyset::Dev>(ndev)};
-  std::vector<uint8_t*> tmp(3 * ndev, nullptr);  // per device: scratch, and the copies of pk, pk2 (host inputs)
-  auto fail = [&](int code, const char* what) {
-    for (size_t di = 0; di < ndev; di++) {
-      cudaSetDevice(ctx->devs[di].dev);
-      if (devptrs) cudaStreamSynchronize(ctx->user_stream);
-      for (int k = 0; k < 3; k++)
-        if (tmp[3 * di + k]) cudaFree(tmp[3 * di + k]);
-    }
-    if (code != SB200_OK) {
-      cudaGetLastError();  // a failed allocation is not the next call's error
-      keyset_free(ks);
-      ctx->set_err(what);
-    }
-    return code;
-  };
-  for (size_t di = 0; di < ndev; di++) {
-    DevCtx& dc = ctx->devs[di];
-    if (cudaSetDevice(dc.dev) != cudaSuccess) return fail(SB200_ERR_CUDA, "cudaSetDevice");
-    sb200_keyset::Dev& kd = ks->dev[di];
-    if (cudaMalloc(&kd.tab, tab_bytes) != cudaSuccess || cudaMalloc(&kd.ok, ok_bytes) != cudaSuccess ||
-        cudaMalloc(&tmp[3 * di], scr_bytes) != cudaSuccess)
-      return fail(SB200_ERR_NOMEM, "cudaMalloc keyset");
-    // SB200_DEVICE_PTRS: on the caller's stream, after the work that produced the keys
-    cudaStream_t st = devptrs ? ctx->user_stream : dc.stream[0];
-    const uint32_t* src[2] = {pk, pk2};
-    if (!devptrs)
-      for (int p = 0; p < nt; p++) {
-        if (cudaMalloc(&tmp[3 * di + 1 + p], pt_bytes) != cudaSuccess) return fail(SB200_ERR_NOMEM, "cudaMalloc keyset input");
-        if (cudaMemcpyAsync(tmp[3 * di + 1 + p], src[p], pt_bytes, cudaMemcpyHostToDevice, st) != cudaSuccess)
-          return fail(SB200_ERR_CUDA, "cudaMemcpyAsync keyset input");
-        src[p] = (const uint32_t*)tmp[3 * di + 1 + p];
-      }
-    if (cudaMemsetAsync(kd.ok, 0, ok_bytes, st) != cudaSuccess) return fail(SB200_ERR_CUDA, "cudaMemsetAsync key_ok");
-    const Launcher go{ctx, st};
-    for (int64_t k0 = 0; k0 < n_keys; k0 += batch) {
-      const KsBuild b{kd.tab, kd.ok, src[0], nt == 2 ? src[1] : nullptr, k0, std::min(batch, n_keys - k0), nt,
-                      (flags & SB200_POINTS_AFFINE) != 0, (fq*)tmp[3 * di]};
-      go(k_keyset_build, (unsigned)((b.nk * 32 + TPB - 1) / TPB), TPB, 0, b);
-    }
-    if (cudaGetLastError() != cudaSuccess) return fail(SB200_ERR_CUDA, "k_keyset_build launch");
-  }
-  for (size_t di = 0; di < ndev; di++) {  // the builds of all devices run concurrently
-    DevCtx& dc = ctx->devs[di];
-    if (cudaSetDevice(dc.dev) != cudaSuccess || cudaStreamSynchronize(devptrs ? ctx->user_stream : dc.stream[0]) != cudaSuccess)
-      return fail(SB200_ERR_CUDA, "k_keyset_build");
-  }
-  if (key_ok) {
-    cudaSetDevice(ctx->devs[0].dev);
-    if (cudaMemcpy(key_ok, ks->dev[0].ok, ok_bytes, cudaMemcpyDeviceToHost) != cudaSuccess) return fail(SB200_ERR_CUDA, "key_ok copy");
-  }
-  fail(SB200_OK, "");  // frees the temporaries only
-  ctx->keysets.push_back(ks);
-  *out = ks;
-  return SB200_OK;
+  if ((flags & SB200_DEVICE_PTRS) && ctx->devs.size() != 1) return SB200_ERR_ARG;
+  return keyset_create(ctx, scheme, n_keys, flags, pk, pk2, nullptr, key_ok, out);
 }
 void sb200_keyset_destroy(sb200_keyset* ks) {
   if (!ks) return;
@@ -1964,7 +2161,7 @@ int sb200_verify_keyset(sb200_ctx* ctx, const sb200_keyset* ks, int64_t n, uint3
   if (!ctx || !ks) return SB200_ERR_ARG;
   {  // a keyset of this context that is still alive
     std::lock_guard<std::mutex> lock(ctx->mu);
-    if (std::find(ctx->keysets.begin(), ctx->keysets.end(), ks) == ctx->keysets.end()) return SB200_ERR_ARG;
+    if (!keyset_of(ctx, ks)) return SB200_ERR_ARG;
   }
   const int pw = pt_words(flags);
   Desc d; d.op = OP_VERIFY_KEYSET; d.flags = flags; d.aux = ks->scheme; d.ks = ks; d.nout = 1; BITMAP(verdicts);
@@ -1977,6 +2174,75 @@ int sb200_verify_keyset(sb200_ctx* ctx, const sb200_keyset* ks, int64_t n, uint3
   d.nin = k;
   OPT_OUT(0, c_out, 8);
   return run(ctx, n, d);
+}
+int sb200_verify_keyset_bytes(sb200_ctx* ctx, const sb200_keyset* ks, int64_t n, uint32_t flags, const uint32_t* key_index,
+                              const uint8_t* sig_bytes, const uint8_t* msg32, uint32_t* verdicts, uint32_t* invalid) {
+  if (!ctx || !ks) return SB200_ERR_ARG;
+  {
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    if (!keyset_of(ctx, ks)) return SB200_ERR_ARG;
+  }
+  Desc d; d.op = OP_VERIFY_KEYSET_BYTES; d.flags = flags; d.aux = ks->scheme; d.ks = ks; d.nin = 3; d.nout = 1; BITMAP(verdicts);
+  IN(0, key_index, 1); IN(1, (const uint32_t*)sig_bytes, ks->scheme == 1 ? 24 : 16); IN(2, (const uint32_t*)msg32, 8);
+  OPT_OUT(0, invalid, -1);  // bitmap-shaped output: one word per 32 tuples
+  return run(ctx, n, d);
+}
+int sb200_keyset_create_bytes(sb200_ctx* ctx, int scheme, int64_t n_keys, uint32_t flags, const uint8_t* pk_bytes,
+                              uint32_t* key_ok, sb200_keyset** out) {
+  if (out) *out = nullptr;
+  if (!ctx || !out || scheme < 0 || scheme > 2 || n_keys < 1 || n_keys > (int64_t)UINT32_MAX || (flags & ~SB200_DEVICE_PTRS))
+    return SB200_ERR_ARG;
+  if (!pk_bytes || ((uintptr_t)pk_bytes & 15)) return SB200_ERR_ARG;
+  if ((flags & SB200_DEVICE_PTRS) && ctx->devs.size() != 1) return SB200_ERR_ARG;
+  return keyset_create(ctx, scheme, n_keys, flags, nullptr, nullptr, pk_bytes, key_ok, out);
+}
+int sb200_keyset_update(sb200_keyset* ks, int64_t m, uint32_t flags, const uint32_t* slots, const uint32_t* pk, const uint32_t* pk2,
+                        uint32_t* key_ok) {
+  return keyset_update(ks, m, flags, SB200_POINTS_AFFINE | SB200_DEVICE_PTRS, slots, pk, pk2, nullptr, key_ok);
+}
+int sb200_keyset_update_bytes(sb200_keyset* ks, int64_t m, uint32_t flags, const uint32_t* slots, const uint8_t* pk_bytes,
+                              uint32_t* key_ok) {
+  return keyset_update(ks, m, flags, SB200_DEVICE_PTRS, slots, nullptr, nullptr, pk_bytes, key_ok);
+}
+int sb200_keyset_revoke(sb200_keyset* ks, int64_t m, const uint32_t* slots) {
+  sb200_ctx* ctx = live_keyset_ctx(ks);
+  if (!ctx || m < 0 || !slots || ((uintptr_t)slots & 15)) return SB200_ERR_ARG;
+  if (m == 0) return SB200_OK;
+  std::lock_guard<std::mutex> lock(ctx->mu);
+  if (!keyset_of(ctx, ks) || !slots_valid(ks, m, slots)) return SB200_ERR_ARG;
+  ctx->set_err("");
+  DeviceGuard guard;
+  std::vector<uint32_t*> dslots(ctx->devs.size(), nullptr);
+  auto finish = [&](int code, const char* what) {
+    for (size_t di = 0; di < dslots.size(); di++) {
+      cudaSetDevice(ctx->devs[di].dev);
+      cudaStreamSynchronize(ctx->devs[di].stream[0]);
+      if (dslots[di]) cudaFree(dslots[di]);
+    }
+    if (code != SB200_OK) {
+      cudaGetLastError();
+      ctx->set_err(what);
+    }
+    return code;
+  };
+  for (size_t di = 0; di < dslots.size(); di++) {
+    if (cudaSetDevice(ctx->devs[di].dev) != cudaSuccess) return finish(SB200_ERR_CUDA, "cudaSetDevice");
+    if (cudaMalloc(&dslots[di], (size_t)m * 4) != cudaSuccess) return finish(SB200_ERR_NOMEM, "cudaMalloc slots");
+  }
+  for (size_t di = 0; di < dslots.size(); di++) {  // after the context's SB200_DEVICE_PTRS work, like an update
+    DevCtx& dc = ctx->devs[di];
+    cudaStream_t st = dc.stream[0];
+    if (cudaSetDevice(dc.dev) != cudaSuccess) return finish(SB200_ERR_CUDA, "cudaSetDevice");
+    if (dc.user_ev_valid && cudaStreamWaitEvent(st, dc.user_ev, 0) != cudaSuccess) return finish(SB200_ERR_CUDA, "cudaStreamWaitEvent");
+    if (cudaMemcpyAsync(dslots[di], slots, (size_t)m * 4, cudaMemcpyHostToDevice, st) != cudaSuccess)
+      return finish(SB200_ERR_CUDA, "cudaMemcpyAsync slots");
+    Launcher{ctx, st}(k_keyset_revoke, (unsigned)((m + TPB - 1) / TPB), TPB, 0, ks->dev[di].ok, (const uint32_t*)dslots[di], m);
+    if (cudaGetLastError() != cudaSuccess) return finish(SB200_ERR_CUDA, "k_keyset_revoke launch");
+  }
+  for (size_t di = 0; di < dslots.size(); di++)
+    if (cudaSetDevice(ctx->devs[di].dev) != cudaSuccess || cudaStreamSynchronize(ctx->devs[di].stream[0]) != cudaSuccess)
+      return finish(SB200_ERR_CUDA, "k_keyset_revoke");
+  return finish(SB200_OK, "");
 }
 int sb200_points_check(sb200_ctx* ctx, int64_t n, uint32_t flags, const uint32_t* points, uint32_t* ok_bitmap) {
   Desc d; d.op = OP_POINTS_CHECK; d.flags = flags; d.nin = 1; d.nout = 0; BITMAP(ok_bitmap);
