@@ -139,6 +139,10 @@ _KEYSET_LIVE_PROTOTYPES = {  # every symbol of include/schnorr_b200_keyset_live.
     "sb200_keyset_update_bytes": (ci, [vp, i64, u32] + [u32p] * 3),
     "sb200_keyset_revoke": (ci, [vp, i64, u32p]),
 }
+_KEYSET_WITNESS_PROTOTYPES = {  # every symbol of include/schnorr_b200_keyset_witness.h (witness rows against a keyset)
+    "sb200_verify_witness_keyset": (ci, [vp, vp, i64, u32] + [u32p] * 7),
+    "sb200_verify_witness_keyset_bytes": (ci, [vp, vp, i64, u32] + [u32p] * 6),
+}
 del vp, u32p, i64, u32, ci
 EXPORTED_SYMBOLS = list(_PROTOTYPES)  # the symbols of include/schnorr_b200.h
 
@@ -159,7 +163,8 @@ def load_library() -> ctypes.CDLL:
             f"{LIB_PATH} not found: build it with `python -c 'import __graft_entry__ as g; g.build()'` "
             "(nvcc, sm_100a). There is no CPU fallback.")
     lib = ctypes.CDLL(LIB_PATH)
-    for name, (res, args) in {**_PROTOTYPES, **_WITNESS_PROTOTYPES, **_KEYSET_PROTOTYPES, **_KEYSET_LIVE_PROTOTYPES}.items():
+    for name, (res, args) in {**_PROTOTYPES, **_WITNESS_PROTOTYPES, **_KEYSET_PROTOTYPES, **_KEYSET_LIVE_PROTOTYPES,
+                              **_KEYSET_WITNESS_PROTOTYPES}.items():
         fn = getattr(lib, name)  # AttributeError if the library does not export a declared symbol
         fn.restype, fn.argtypes = res, args
     _lib = lib
@@ -604,8 +609,9 @@ class Engine:
 
 class KeySet:
     """Public keys registered on every device of an Engine (include/schnorr_b200_keyset.h): `key_ok` (bool[n_keys]: every
-    point of the key is on the curve with Z != 0, kept current by update and revoke), `verify`, and the calls of
-    include/schnorr_b200_keyset_live.h: `verify_bytes`, `update`, `update_bytes`, `revoke`.  Frees its device memory on
+    point of the key is on the curve with Z != 0, kept current by update and revoke), `verify`, the calls of
+    include/schnorr_b200_keyset_live.h: `verify_bytes`, `update`, `update_bytes`, `revoke`, and those of
+    include/schnorr_b200_keyset_witness.h: `verify_witness`, `verify_witness_bytes`.  Frees its device memory on
     close() / exit / GC."""
 
     KEY_BYTES = (32, 64, 64)  # to_bytes() of PublicKey, PublicKeyDouble, PublicKeyVarGen
@@ -693,6 +699,42 @@ class KeySet:
                                               bm.ctypes.data, inv.ctypes.data)
         e._check(rc, "verify_keyset_bytes")
         return e._unpack_bits(bm, n), e._unpack_bits(inv, n)
+
+    def verify_witness(self, key_index, u, R, msg, Rp=None, affine=True, check_points=False):
+        """witness rows of received signatures against the keys key_index[i] (include/schnorr_b200_keyset_witness.h):
+        (ok[n], rows[n, W, 8]) with the layout and values of Engine.verify_witness on the gathered keys.  An index >=
+        n_keys, a key that is not key_ok or u >= r gives an all-zero row and verdict 0."""
+        e = self._open("verify_witness")
+        idx = self._slots(key_index)
+        n = idx.size
+        pw = e._pw(affine)
+        fl = (POINTS_AFFINE if affine else POINTS_PROJECTIVE) | (CHECK_POINTS if check_points else 0)
+        u, R, msg = _arr(u, 8, n, "u"), _arr(R, pw, n, "R"), _arr(msg, 8, n, "msg")
+        Rp = _arr(Rp, pw, n, "R'") if self.scheme == 1 else None
+        bm = aligned_empty(((n + 31) // 32,)); bm[...] = 0
+        rows = aligned_empty((n, Engine.WITNESS_WIDTH[self.scheme], 8))
+        rc = e._lib.sb200_verify_witness_keyset(e._h, self._h, n, fl, idx.ctypes.data, u.ctypes.data, R.ctypes.data,
+                                                Rp.ctypes.data if Rp is not None else None, msg.ctypes.data, bm.ctypes.data,
+                                                rows.ctypes.data)
+        e._check(rc, "verify_witness_keyset")
+        return e._unpack_bits(bm, n), rows
+
+    def verify_witness_bytes(self, key_index, sig_bytes, msg_bytes):
+        """verify_witness on wire-format signatures and 32-byte canonical messages: (ok[n], invalid[n], rows[n, W, 8]);
+        a tuple whose signature or message does not decode has invalid set, verdict 0 and an all-zero row"""
+        e = self._open("verify_witness_bytes")
+        idx = self._slots(key_index)
+        n = idx.size
+        sig, msg = e._bytes_arr(sig_bytes, self.SIG_BYTES[self.scheme], "sig"), e._bytes_arr(msg_bytes, 32, "msg")
+        if sig.shape[0] != n or msg.shape[0] != n:
+            raise SchnorrB200Error(f"verify_witness_bytes: {n} key indices, {sig.shape[0]} signatures, {msg.shape[0]} messages")
+        bm = aligned_empty(((n + 31) // 32,)); bm[...] = 0
+        inv = aligned_empty(((n + 31) // 32,)); inv[...] = 0
+        rows = aligned_empty((n, Engine.WITNESS_WIDTH[self.scheme], 8))
+        rc = e._lib.sb200_verify_witness_keyset_bytes(e._h, self._h, n, 0, idx.ctypes.data, sig.ctypes.data, msg.ctypes.data,
+                                                      bm.ctypes.data, rows.ctypes.data, inv.ctypes.data)
+        e._check(rc, "verify_witness_keyset_bytes")
+        return e._unpack_bits(bm, n), e._unpack_bits(inv, n), rows
 
     def _updated(self, rc: int, what: str, slots: np.ndarray, ok: np.ndarray) -> np.ndarray:
         self._engine._check(rc, what)

@@ -567,7 +567,8 @@ class PublicKeySet:
     addition of this library.  `verify_batch(indices, sigs, msgs)` returns what the type's
     `verify_batch([keys[i] for i in indices], sigs, msgs)` returns (a key not on the curve verifies nothing).
     `verify_batch_bytes` takes the signatures and messages as received bytes; `replace` and `remove` change single keys
-    of the live set in place (include/schnorr_b200_keyset_live.h)."""
+    of the live set in place (include/schnorr_b200_keyset_live.h).  `witness_batch` / `witness_batch_bytes` return the
+    PLONK witness rows of the signatures together with the verdicts (include/schnorr_b200_keyset_witness.h)."""
 
     _SCHEMES = {PublicKey: 0, PublicKeyDouble: 1, PublicKeyVarGen: 2}
 
@@ -615,6 +616,21 @@ class PublicKeySet:
         invalid[i] = `Signature*::from_bytes` or `BlsScalar::from_bytes` of tuple i fails (its verdict is False)"""
         idx = self._indices(indices, "verify_batch_bytes")
         return self._ks.verify_bytes(idx.astype(np.uint32), b"".join(sigs), b"".join(msgs))
+
+    def witness_batch(self, indices: Sequence[int], sigs: Sequence, msgs: Sequence[int]) -> Tuple[np.ndarray, np.ndarray]:
+        """(ok, rows): the verdicts of verify_batch and, per signature, the witness row that `Signature*::append` and the
+        `verify_signature*` gadgets allocate ([n, 11 | 19 | 13, 8] Montgomery limbs: u, R(, R'), PK(, PK' | GEN), m, c,
+        SA, SB(, SA', SB')); all zero for a key not on the curve or a removed key"""
+        idx = self._indices(indices, "witness_batch")
+        Rp = _points([s._Rp for s in sigs]) if self.scheme == 1 else None
+        return self._ks.verify_witness(idx.astype(np.uint32), _scalars([s._u for s in sigs]), _points([s._R for s in sigs]),
+                                       _fqs(msgs), Rp=Rp, affine=False)
+
+    def witness_batch_bytes(self, indices: Sequence[int], sigs: Sequence[bytes], msgs: Sequence[bytes]) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """witness_batch on signatures as `Signature*::to_bytes()` and 32-byte canonical messages: (ok, invalid, rows);
+        a signature or message that does not decode has invalid set, verdict False and an all-zero row"""
+        idx = self._indices(indices, "witness_batch_bytes")
+        return self._ks.verify_witness_bytes(idx.astype(np.uint32), b"".join(sigs), b"".join(msgs))
 
     def replace(self, indices: Sequence[int], keys: Sequence) -> None:
         """key indices[j] becomes keys[j] (same type as the set's keys); a removed index is registered again"""

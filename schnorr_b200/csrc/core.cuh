@@ -738,4 +738,107 @@ SB_HD bool verify_keyset_core(const uint32_t* tabs, int64_t n_keys, const uint32
   return ok;
 }
 
+// a / 2 for canonical a: (a + q) / 2 when a is odd (q < 2^255, so a + q has no carry out); canonical, and the Montgomery
+// form of x / 2 when a is that of x
+SB_HD fq fq_half(const fq& a) {
+  fq t = a;
+  if (a.v[0] & 1u) {
+    const uint32_t q[8] = SB200_FQ_MOD_INIT;
+    add8(t.v, a.v, q);
+  }
+  fq r;
+#pragma unroll
+  for (int i = 0; i < 7; i++) r.v[i] = (t.v[i] >> 1) | (t.v[i + 1] << 31);
+  r.v[7] = t.v[7] >> 1;
+  return r;
+}
+// k P from a key's 8-bit comb (k < 2^252)
+SB_HD ext keyset_comb_mul(const uint32_t* tab, const uint32_t* k) {
+  uint32_t kr[8];
+#pragma unroll
+  for (int i = 0; i < 8; i++) kr[i] = k[i];
+  recode_offset<KS_BITS>(kr);
+  return p1p1_to_ext(ed_comb_add_w<KS_BITS>(ext_identity(), tab, kr));
+}
+
+// The rows of verify_witness_core for a key registered in a keyset (include/schnorr_b200_keyset_witness.h): same layout,
+// same values.  PK (PK', GEN) is read back from entry 1 of window 0 of the key's comb, (y + x, y - x, ..) -> (x, y), so the
+// key's coordinates are the canonical affine ones verify_witness_core writes.  The challenge is the one verify_keyset_core
+// computes.  SA = u G (u G') by the 16-bit comb, or u GEN by the key's comb of its generator; SB = c PK (c PK') by the key's
+// comb: both exact multiples (never SB = R - SA), so the row does not depend on which table made them.  The verdict is
+// SA + SB == R (and SA' + SB' == R').  The row is zero and the verdict 0 -- by masked stores, every lane runs the work --
+// when u >= r, key >= n_keys (key 0's table is read instead), key_ok is clear, or with `check_points` R (R') is not well
+// formed.  A good key with a wrong signature keeps its true row.
+template <int SCHEME, class Emit>
+SB_HD bool verify_witness_keyset_core(const uint32_t* tabs, int64_t n_keys, const uint32_t* key_ok, uint32_t key,
+                                      const uint32_t* u_in, const point_in& R, const point_in& Rp, const fq& m,
+                                      bool check_points, const uint32_t* combG, const uint32_t* combGp, Emit&& emit) {
+  constexpr int NB = SCHEME == 1 ? 2 : 1;  // bases
+  constexpr int NT = SCHEME == 0 ? 1 : 2;  // combs per key: PK (, PK' | GEN)
+  const bool known = (int64_t)key < n_keys;
+  const uint64_t k = known ? key : 0u;
+  const bool lt = scalar_lt_r(u_in);
+  bool live = known & ((key_ok[k >> 5] >> (k & 31) & 1u) != 0) & lt;
+  if (check_points) {  // warp-uniform
+    live &= point_well_formed(R);
+    if (SCHEME == 1) live &= point_well_formed(Rp);
+  }
+  auto put = [&](int i, const fq& v) { emit(i, live ? v : fq_zero()); };
+  const uint32_t* tab = tabs + k * NT * KS_TABLE_WORDS;
+  uint32_t u[8], c[8];
+#pragma unroll
+  for (int i = 0; i < 8; i++) u[i] = lt ? u_in[i] : 0u;  // in range for the combs; the row is zero anyway
+  put(0, scalar_to_bls(u));
+  // 1. R (, R') in affine form: one inversion for both when they are projective; then the key's points
+  fq ru[NB], rv[NB];
+  if (R.affine) {
+    ru[0] = R.U; rv[0] = R.V;
+    if (SCHEME == 1) { ru[NB - 1] = Rp.U; rv[NB - 1] = Rp.V; }
+  } else {
+    fq z[NB], pre[NB];
+    z[0] = R.Z;
+    if (SCHEME == 1) z[NB - 1] = Rp.Z;
+    batch_inverse(z, pre, NB);
+    ru[0] = fq_mul(R.U, z[0]); rv[0] = fq_mul(R.V, z[0]);
+    if (SCHEME == 1) { ru[NB - 1] = fq_mul(Rp.U, z[NB - 1]); rv[NB - 1] = fq_mul(Rp.V, z[NB - 1]); }
+  }
+  int o = 1;
+#pragma unroll
+  for (int b = 0; b < NB; b++) {
+    put(o++, ru[b]);
+    put(o++, rv[b]);
+  }
+#pragma unroll
+  for (int t = 0; t < NT; t++) {  // entry 1 of window 0 = the point itself: x = (A - B) / 2, y = (A + B) / 2
+    const aniels e = aniels_load(tab + t * KS_TABLE_WORDS + 24);
+    put(o++, fq_half(fq_sub(e.YpX, e.YmX)));
+    put(o++, fq_half(fq_add(e.YpX, e.YmX)));
+  }
+  // 2. the challenge
+  if (SCHEME == 1) chal5(ru[0], rv[0], ru[1], rv[1], m, c); else chal3(ru[0], rv[0], m, c);
+  put(o++, m);
+  put(o++, scalar_to_bls(c));
+  // 3. SA = u B, SB = c PK (one copy of the curve code for both bases); the verdict SA + SB == R
+  ext S[2 * NB];
+  bool ok = live;
+#pragma unroll 1
+  for (int b = 0; b < NB; b++) {
+    S[2 * b] = SCHEME == 2 ? keyset_comb_mul(tab + KS_TABLE_WORDS, u) : fixed_base_mul(b ? combGp : combG, u);
+    S[2 * b + 1] = keyset_comb_mul(tab + b * KS_TABLE_WORDS, c);
+    const point_in rr = {ru[b], rv[b], fq_one(), true};
+    ok &= p1p1_equals(ed_add(S[2 * b], ext_to_pniels(S[2 * b + 1])), rr);
+  }
+  // 4. the outputs in affine form: one inversion
+  fq z[2 * NB], pre[2 * NB];
+#pragma unroll
+  for (int i = 0; i < 2 * NB; i++) z[i] = S[i].Z;
+  batch_inverse(z, pre, 2 * NB);
+#pragma unroll
+  for (int i = 0; i < 2 * NB; i++) {
+    put(o++, fq_mul(S[i].X, z[i]));
+    put(o++, fq_mul(S[i].Y, z[i]));
+  }
+  return ok;
+}
+
 }  // namespace sb200

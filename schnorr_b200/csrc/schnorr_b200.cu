@@ -23,6 +23,7 @@
 #include "../../include/schnorr_b200_witness.h"
 #include "../../include/schnorr_b200_keyset.h"
 #include "../../include/schnorr_b200_keyset_live.h"
+#include "../../include/schnorr_b200_keyset_witness.h"
 #include "wire.cuh"
 #include "rng.cuh"
 #include "params_host.cuh"
@@ -56,7 +57,11 @@ constexpr int TPB = 128;
 #ifndef SB_VERIFY_CTAS
 #define SB_VERIFY_CTAS SB_MIN_CTAS
 #endif
-constexpr int min_ctas(int op) { return (op == 0 || op == 19) ? SB_VERIFY_CTAS : (op == 25 || op == 27 || op == 37) ? SB_MIN_CTAS - 1 : (op == 1 || op == 2) ? SB_MIN_CTAS - 1 : SB_MIN_CTAS; }
+// The keyset witness kernel (op 43, OP_VERIFY_WITNESS_KEYSET): SB_KSW_CTAS, timed against one CTA fewer in DESIGN.md 4.10.
+#ifndef SB_KSW_CTAS
+#define SB_KSW_CTAS SB_MIN_CTAS
+#endif
+constexpr int min_ctas(int op) { return (op == 0 || op == 19) ? SB_VERIFY_CTAS : (op == 25 || op == 27 || op == 37) ? SB_MIN_CTAS - 1 : (op == 1 || op == 2) ? SB_MIN_CTAS - 1 : op == 43 ? SB_KSW_CTAS : SB_MIN_CTAS; }
 constexpr int MAX_IN = 6, MAX_OUT = 4;
 constexpr int64_t CHUNK = 1 << 18;      // tuples per pipeline stage ...
 constexpr int64_t CHUNK_MIN = 1 << 14;  // ... shrunk towards this when a device's share is under 4 chunks, so that H2D still overlaps compute
@@ -70,9 +75,11 @@ enum Op : int {
   OP_DECODE_VERIFY, OP_WITNESS, OP_DBG_LAT3,
   OP_STDRNG, OP_SIGN_STDRNG, OP_SIGN_DOUBLE_STDRNG, OP_SIGN_VARGEN_STDRNG,
   OP_VERIFY_WITNESS, OP_VERIFY_WITNESS_BYTES, OP_VERIFY_KEYSET,
-  OP_DECODE_KEYSET, OP_VERIFY_KEYSET_BYTES, OP_DECODE_KEYS
+  OP_DECODE_KEYSET, OP_VERIFY_KEYSET_BYTES, OP_DECODE_KEYS,
+  OP_VERIFY_WITNESS_KEYSET, OP_VERIFY_WITNESS_KEYSET_BYTES
 };
 static_assert(OP_VERIFY_WITNESS == 37, "min_ctas names the op by number");
+static_assert(OP_VERIFY_WITNESS_KEYSET == 43, "min_ctas names the op by number");
 
 struct KArgs {
   int64_t n;
@@ -941,6 +948,32 @@ __global__ void __launch_bounds__(TPB, SB_MIN_CTAS) k_verify_keyset(const KArgs 
   if (a.out[0] && active) stg8(a.out[0] + i * 8, c);
 }
 
+// Witness rows against a keyset (include/schnorr_b200_keyset_witness.h).  aux = scheme; in: key index, u, R, (R',) m ->
+// out0: rows, bitmap: verdicts.  Also the second kernel of the byte-level call, on the rows of k_run<OP_DECODE_KEYSET>.
+__global__ void __launch_bounds__(TPB, min_ctas(OP_VERIFY_WITNESS_KEYSET)) k_verify_witness_keyset(const KArgs a, const KsArgs ks) {
+  int64_t i = (int64_t)blockIdx.x * TPB + threadIdx.x;
+  const bool active = i < a.n;
+  if (!active) i = a.n - 1;  // idle lanes redo the last tuple so the warp stays converged
+  const bool aff = (a.flags & SB200_POINTS_AFFINE) != 0, chk = (a.flags & SB200_CHECK_POINTS) != 0;
+  const uint32_t key = __ldg(a.in[0] + i);
+  uint32_t u[8];
+  ldg_scalar(a.in[1] + i * 8, u);
+  uint32_t* dst = a.out[0] + i * SB200_WITNESS_WIDTH(a.aux) * 8;
+  auto emit = [&](int k, const fq& v) { if (active) stg8(dst + k * 8, v.v); };
+  bool ok;
+  if (a.aux == 0)
+    ok = verify_witness_keyset_core<0>(ks.tab, ks.n, ks.ok, key, u, ldg_point(a.in[2], i, aff), point_in(), ldg_fq(a.in[3] + i * 8),
+                                       chk, a.combG, a.combGp, emit);
+  else if (a.aux == 1)
+    ok = verify_witness_keyset_core<1>(ks.tab, ks.n, ks.ok, key, u, ldg_point(a.in[2], i, aff), ldg_point(a.in[3], i, aff),
+                                       ldg_fq(a.in[4] + i * 8), chk, a.combG, a.combGp, emit);
+  else
+    ok = verify_witness_keyset_core<2>(ks.tab, ks.n, ks.ok, key, u, ldg_point(a.in[2], i, aff), point_in(), ldg_fq(a.in[3] + i * 8),
+                                       chk, a.combG, a.combGp, emit);
+  unsigned word = __ballot_sync(0xffffffffu, ok && active);
+  if ((threadIdx.x & 31) == 0 && active) a.bitmap[i >> 5] = word;
+}
+
 // Per-key combs of a keyset (include/schnorr_b200_keyset.h): one warp per key of [key0, key0 + nk), one lane per window
 // (keyset_build_window), the key's NT points one after the other, then its key_ok bit.  Lane-divergent doubling counts
 // (8 j for window j): a one-off build, not a hot path.  scratch: 2 x (KS_ENTRIES - 1) fq per thread of the launch.
@@ -1048,7 +1081,7 @@ struct Desc {
   int out_words[MAX_OUT] = {};
   uint32_t* bitmap = nullptr;
   const sb200_stdrng* rng = nullptr;  // OP_STDRNG and the seeded signers: key and word position of tuple 0
-  const sb200_keyset* ks = nullptr;   // OP_VERIFY_KEYSET: whose per-device tables the kernels read
+  const sb200_keyset* ks = nullptr;   // KEYSET, KEYSET_BYTES ops: whose per-device tables the kernels read
   unsigned need = 0;  // outputs that may not be null: bit k for out[k], bit MAX_OUT for the bitmap
 };
 
@@ -1124,10 +1157,11 @@ namespace {
 // challenge kernel, then curve kernel, the challenges through c_out or scratch.  VERIFY_BYTES: decode kernel, then VERIFY
 // on the decoded rows.  SIGN_STDRNG: the nonces drawn into scratch, then the scheme's sign op.  DBG_VERIFY_EC: the curve
 // kernel alone, on the caller's challenges.  WITNESS_BYTES: decode kernel, then `kernel` on the decoded rows.  KEYSET:
-// k_verify_keyset, one tuple per thread, with the keyset's tables of the launching device.  KEYSET_BYTES: the keyset decode
-// kernel, then KEYSET on the decoded rows.
+// `ks_kernel` (k_verify_keyset or k_verify_witness_keyset), one tuple per thread, with the keyset's tables of the launching
+// device.  KEYSET_BYTES: the keyset decode kernel, then KEYSET on the decoded rows.
 enum Form : uint8_t { INTERNAL, ONE, FIXED, VERIFY, VERIFY_BYTES, SIGN_STDRNG, DBG_VERIFY_EC, WITNESS_BYTES, KEYSET, KEYSET_BYTES };
 using KFn = void (*)(KArgs);
+using KsFn = void (*)(KArgs, KsArgs);
 struct OpInfo {
   Form form;
   uint32_t flags;       // the SB200_* flags the op accepts: any other one is SB200_ERR_ARG
@@ -1137,6 +1171,7 @@ struct OpInfo {
   uint32_t forced;      // flags the op always runs with: the byte-level verifications hand affine points between kernels
   unsigned scratch;     // device-only bytes per tuple between the kernels of one call, in `scratch_arrays` arrays: the
   int scratch_arrays;   // challenges or nonces, and the decoded rows (points 64 B, u and m 32 B) and invalid bitmap
+  KsFn ks_kernel;       // KEYSET, KEYSET_BYTES: the kernel that reads the keyset
 };
 constexpr OpInfo row(Form form, uint32_t flags = 0, int scheme = 0, KFn kernel = nullptr, KFn ct = nullptr) {
   const bool decode = form == VERIFY_BYTES || form == WITNESS_BYTES, ks = form == KEYSET_BYTES;
@@ -1145,7 +1180,12 @@ constexpr OpInfo row(Form form, uint32_t flags = 0, int scheme = 0, KFn kernel =
   const bool handover = form == VERIFY || form == VERIFY_BYTES || form == SIGN_STDRNG;  // + 32 B: the challenge row
   return {form, flags, scheme, kernel, ct, ct ? (size_t)(scheme == 1 ? 2 : 1) * CT_TABLE_WORDS * 4 : 0,
           decode || ks ? (uint32_t)SB200_POINTS_AFFINE : 0u, (handover ? 32u : 0u) + rows + (ks ? 68 + 64 * sig_points : 0u),
-          (handover ? 1 : 0) + (rows ? (int)points + 3 : 0) + (ks ? (int)sig_points + 3 : 0)};
+          (handover ? 1 : 0) + (rows ? (int)points + 3 : 0) + (ks ? (int)sig_points + 3 : 0), nullptr};
+}
+constexpr OpInfo ks_row(Form form, uint32_t flags, int scheme, KsFn kernel) {
+  OpInfo o = row(form, flags, scheme);
+  o.ks_kernel = kernel;
+  return o;
 }
 constexpr uint32_t D = SB200_DEVICE_PTRS, AD = SB200_POINTS_AFFINE | D, CHK = AD | SB200_CHECK_POINTS;
 constexpr uint32_t OBL = AD | SB200_SIGN_OBLIVIOUS, DUAL = SB_VERIFY_WS ? SB200_VERIFY_DUAL_PIPE : 0;
@@ -1198,12 +1238,14 @@ constexpr OpInfo OPS[] = {
     row(SIGN_STDRNG, OBL, 2),                       // OP_SIGN_VARGEN_STDRNG
     row(ONE, CHK, 0, k_run<OP_VERIFY_WITNESS>),     // the scheme is the call's aux
     row(WITNESS_BYTES, D, 1, k_run<OP_VERIFY_WITNESS>),  // scheme 1: scratch for the widest decoded rows; the call's scheme is its aux
-    row(KEYSET, CHK),                               // OP_VERIFY_KEYSET: the keyset's scheme is the call's aux
+    ks_row(KEYSET, CHK, 0, k_verify_keyset),        // OP_VERIFY_KEYSET: the keyset's scheme is the call's aux
     row(INTERNAL),                                  // OP_DECODE_KEYSET
-    row(KEYSET_BYTES, D, 1),  // OP_VERIFY_KEYSET_BYTES: scratch for the widest decoded rows; the keyset's scheme is the call's aux
+    ks_row(KEYSET_BYTES, D, 1, k_verify_keyset),  // OP_VERIFY_KEYSET_BYTES: scratch for the widest decoded rows; scheme = aux
     row(INTERNAL),                                  // OP_DECODE_KEYS: launched by the keyset builds
+    ks_row(KEYSET, CHK, 0, k_verify_witness_keyset),        // OP_VERIFY_WITNESS_KEYSET: scheme = aux
+    ks_row(KEYSET_BYTES, D, 1, k_verify_witness_keyset),  // OP_VERIFY_WITNESS_KEYSET_BYTES: as OP_VERIFY_KEYSET_BYTES
 };
-static_assert(sizeof(OPS) / sizeof(OPS[0]) == OP_DECODE_KEYS + 1, "one row per Op");
+static_assert(sizeof(OPS) / sizeof(OPS[0]) == OP_VERIFY_WITNESS_KEYSET_BYTES + 1, "one row per Op");
 
 // ---- launches ---------------------------------------------------------------------------------------------------------
 struct Launcher {  // issues kernels on one stream and counts them (sb200_launch_count)
@@ -1292,10 +1334,12 @@ int launch(sb200_ctx* ctx, Op op, const KArgs& a, cudaStream_t st, const KsArgs&
       break;
     }
     case KEYSET:
-      go(k_verify_keyset, grid, TPB, 0, a, ks);
+      go(o.ks_kernel, grid, TPB, 0, a, ks);
       break;
-    case KEYSET_BYTES: {  // decode kernel -> k_verify_keyset, the decoded rows in a.scratch, `invalid` in out[0]
+    case KEYSET_BYTES: {  // decode kernel -> o.ks_kernel, the decoded rows in a.scratch, `invalid` in the output after the
+                          // kernel's own: out[0] for k_verify_keyset (no c_out), out[1] for k_verify_witness_keyset (rows)
       const int nr = a.aux == 1 ? 2 : 1, narr = nr + 3;  // key index, u, R, (R',) m
+      const int kout = o.ks_kernel == k_verify_witness_keyset ? 1 : 0;
       uint8_t* p = a.scratch;
       auto carve = [&](size_t bytes) { uint8_t* r = p; p += (bytes + 63) & ~(size_t)63; return (uint32_t*)r; };
       KArgs dk = a, v = a;
@@ -1303,10 +1347,10 @@ int launch(sb200_ctx* ctx, Op op, const KArgs& a, cudaStream_t st, const KsArgs&
         dk.dec[k] = carve((size_t)a.n * (k == 0 ? 4 : (k == 1 || k == narr - 1) ? 32 : 64));
         v.in[k] = dk.dec[k];
       }
-      dk.bitmap = a.out[0] ? a.out[0] : carve((size_t)((a.n + 31) / 32) * 4);
-      for (int k = 0; k < MAX_OUT; k++) v.out[k] = nullptr;  // no c_out
+      dk.bitmap = a.out[kout] ? a.out[kout] : carve((size_t)((a.n + 31) / 32) * 4);
+      for (int k = kout; k < MAX_OUT; k++) v.out[k] = nullptr;  // no c_out
       go(k_run<OP_DECODE_KEYSET>, grid, TPB, 0, dk);
-      go(k_verify_keyset, grid, TPB, 0, v, ks);
+      go(o.ks_kernel, grid, TPB, 0, v, ks);
       break;
     }
     case DBG_VERIFY_EC: {  // in: pk, u, R, c -> bitmap: the production curve kernel, in the form the batch size picks,
@@ -1362,7 +1406,7 @@ KArgs kargs(const sb200_ctx* ctx, const DevCtx& dc, int slot, const Desc& d, int
   }
   return a;
 }
-// the keyset tables of one device's copy (OP_VERIFY_KEYSET), none for every other op
+// the keyset tables of one device's copy (KEYSET, KEYSET_BYTES ops), none for every other op
 KsArgs ks_args(const sb200_ctx* ctx, const DevCtx& dc, const Desc& d) {
   KsArgs k;
   if (d.ks) {
@@ -2185,6 +2229,40 @@ int sb200_verify_keyset_bytes(sb200_ctx* ctx, const sb200_keyset* ks, int64_t n,
   Desc d; d.op = OP_VERIFY_KEYSET_BYTES; d.flags = flags; d.aux = ks->scheme; d.ks = ks; d.nin = 3; d.nout = 1; BITMAP(verdicts);
   IN(0, key_index, 1); IN(1, (const uint32_t*)sig_bytes, ks->scheme == 1 ? 24 : 16); IN(2, (const uint32_t*)msg32, 8);
   OPT_OUT(0, invalid, -1);  // bitmap-shaped output: one word per 32 tuples
+  return run(ctx, n, d);
+}
+int sb200_verify_witness_keyset(sb200_ctx* ctx, const sb200_keyset* ks, int64_t n, uint32_t flags, const uint32_t* key_index,
+                                const uint32_t* sig_u, const uint32_t* sig_R, const uint32_t* sig_R_prime, const uint32_t* msg,
+                                uint32_t* verdicts, uint32_t* rows_out) {
+  if (!ctx || !ks) return SB200_ERR_ARG;
+  {
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    if (!keyset_of(ctx, ks)) return SB200_ERR_ARG;
+  }
+  const int pw = pt_words(flags);
+  Desc d; d.op = OP_VERIFY_WITNESS_KEYSET; d.flags = flags; d.aux = ks->scheme; d.ks = ks; d.nout = 1; BITMAP(verdicts);
+  int k = 0;  // key index, u, R, (R',) m
+  IN(k, key_index, 1); k++;
+  IN(k, sig_u, 8); k++;
+  IN(k, sig_R, pw); k++;
+  if (ks->scheme == 1) { IN(k, sig_R_prime, pw); k++; }
+  IN(k, msg, 8); k++;
+  d.nin = k;
+  OUT(0, rows_out, 8 * SB200_WITNESS_WIDTH(ks->scheme));
+  return run(ctx, n, d);
+}
+int sb200_verify_witness_keyset_bytes(sb200_ctx* ctx, const sb200_keyset* ks, int64_t n, uint32_t flags, const uint32_t* key_index,
+                                      const uint8_t* sig_bytes, const uint8_t* msg32, uint32_t* verdicts, uint32_t* rows_out,
+                                      uint32_t* invalid) {
+  if (!ctx || !ks) return SB200_ERR_ARG;
+  {
+    std::lock_guard<std::mutex> lock(ctx->mu);
+    if (!keyset_of(ctx, ks)) return SB200_ERR_ARG;
+  }
+  Desc d; d.op = OP_VERIFY_WITNESS_KEYSET_BYTES; d.flags = flags; d.aux = ks->scheme; d.ks = ks; d.nin = 3; d.nout = 2;
+  BITMAP(verdicts);
+  IN(0, key_index, 1); IN(1, (const uint32_t*)sig_bytes, ks->scheme == 1 ? 24 : 16); IN(2, (const uint32_t*)msg32, 8);
+  OUT(0, rows_out, 8 * SB200_WITNESS_WIDTH(ks->scheme)); OPT_OUT(1, invalid, -1);
   return run(ctx, n, d);
 }
 int sb200_keyset_create_bytes(sb200_ctx* ctx, int scheme, int64_t n_keys, uint32_t flags, const uint8_t* pk_bytes,

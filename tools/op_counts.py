@@ -89,11 +89,12 @@ nul = np.zeros(24, np.uint32)
 out["verify_witness_single"] = measure(lambda: lib.h_verify_witness(0, H.ptr(H.pt_mont(pk)), H.ptr(nul), H.ptr(H.limbs(u)), H.ptr(H.pt_mont(Rp)), H.ptr(nul), H.ptr(H.mont(m)), 1, 0, H.ptr(tab[0]), H.ptr(tab[1]), H.ptr(rows)))
 out["verify_witness_double"] = measure(lambda: lib.h_verify_witness(1, H.ptr(H.pt_mont(pk)), H.ptr(H.pt_mont(pkp)), H.ptr(H.limbs(ud)), H.ptr(H.pt_mont(Rd)), H.ptr(H.pt_mont(Rdp)), H.ptr(H.mont(m)), 1, 0, H.ptr(tab[0]), H.ptr(tab[1]), H.ptr(rows)))
 out["verify_witness_vargen"] = measure(lambda: lib.h_verify_witness(2, H.ptr(H.pt_mont(pkv)), H.ptr(H.pt_mont(gen)), H.ptr(H.limbs(uvg)), H.ptr(H.pt_mont(Rvg)), H.ptr(nul), H.ptr(H.mont(m)), 1, 0, H.ptr(tab[0]), H.ptr(tab[1]), H.ptr(rows)))
-# verification against a registered key (core.cuh verify_keyset_core, tests/host_keyset.cpp) of valid signatures, affine:
+# verification against a registered key (core.cuh verify_keyset_core, tests/host_keyset.cpp, built here with the keyset
+# witness rows of tests/host_keyset_witness.cpp on top) of valid signatures, affine:
 # the challenge hash, u G by the 16-bit comb (u G' too) or u GEN by the key's 8-bit comb, c PK by the key's 8-bit comb
 sok = os.path.join(ROOT, "build", "host_keyset16.so")
 subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-DSB_COMB_BITS=16", "-include",
-                       os.path.join(ROOT, "tests", "host_shim.h"), "-o", sok, os.path.join(ROOT, "tests", "host_keyset.cpp")])
+                       os.path.join(ROOT, "tests", "host_shim.h"), "-o", sok, os.path.join(ROOT, "tests", "host_keyset_witness.cpp")])
 klib = ctypes.CDLL(sok)
 H.setup_hades(klib)
 klib.h_verify_keyset.argtypes = [ctypes.c_int, ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p, ctypes.c_uint32] + \
@@ -110,6 +111,13 @@ kargs = lambda s, uu, R1, R2: (s, H.ptr(ks[s]), 1, H.ptr(kok), 0, H.ptr(H.limbs(
 out["keyset_verify_single"] = measure(lambda: klib.h_verify_keyset(*kargs(0, u, Rp, nul)), klib)
 out["keyset_verify_double"] = measure(lambda: klib.h_verify_keyset(*kargs(1, ud, Rd, H.pt_mont(Rdp))), klib)
 out["keyset_verify_vargen"] = measure(lambda: klib.h_verify_keyset(*kargs(2, uvg, Rvg, nul)), klib)
+# witness rows against a registered key (core.cuh verify_witness_keyset_core): the keyset verification's combs, the key's
+# coordinates from its comb, and two batched Euclidean inversions (affine outputs; affine R: the first is skipped)
+klib.h_verify_witness_keyset.argtypes = klib.h_verify_keyset.argtypes
+wargs = lambda s, uu, R1, R2: kargs(s, uu, R1, R2)[:-1] + (H.ptr(rows),)
+out["keyset_witness_single"] = measure(lambda: klib.h_verify_witness_keyset(*wargs(0, u, Rp, nul)), klib)
+out["keyset_witness_double"] = measure(lambda: klib.h_verify_witness_keyset(*wargs(1, ud, Rd, H.pt_mont(Rdp))), klib)
+out["keyset_witness_vargen"] = measure(lambda: klib.h_verify_witness_keyset(*wargs(2, uvg, Rvg, nul)), klib)
 st = np.concatenate([H.mont(x) for x in range(5)])
 out["hades_perm_sparse"] = measure(lambda: lib.h_hades(H.ptr(st), 0))  # the production form: small-integer layers for the default MDS
 out["hades_perm_dense"] = measure(lambda: lib.h_hades(H.ptr(st), 1))
